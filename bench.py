@@ -14,6 +14,11 @@ of the 32 MiB counter array per step produces the single global sketch (SURVEY.m
 
 --impl reference times the reference's CPU algorithm (oracle/ C port, all host threads) on a
 bounded sample of the same event stream; the Java itself cannot run here (no JVM in the image).
+
+--dump-outputs DIR writes what the timed steps computed, as float64 DIR/<name>.npy (rank 0, under 64 MB):
+sketch.npy, the [depth, width] sketch after the last step (the all-reduced one at N > 1), and, unless --no-cosine,
+cosine_<precision>_{idx,sim,cnt}.npy of the cosine stage's last step for a fixed sample of rows whose global item
+ids are cosine_rows.npy.  The inputs depend only on the arguments, so two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -29,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree the benchmark runs from may be read-only: no caches next to the sources
 
 SEED = 20240002           # SURVEY.md 8d: 20240001 + config number (config 2 -> ...0003 is 1-based; fixed here)
 SKETCH_SEED = 42
@@ -47,6 +53,8 @@ C3_SEED = 20240003
 C3_CHUNKS = 4              # all-gather chunks per step of the pipelined multi-GPU cosine form
 METRIC = "sketch_updates_per_sec"
 UNIT = "events/s"
+DUMP_ROWS = 4096           # cosine-stage rows written by --dump-outputs (a seeded sample)
+DUMP_MAX_BYTES = 64_000_000
 
 
 def _peaks():
@@ -106,6 +114,17 @@ class ClockSampler(threading.Thread):
         med = float(np.median(self.samples)) if self.samples else None
         return {"sm_mhz": med, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(self.samples)}
+
+
+def _write_dump(path: str, arrays: dict):
+    """--dump-outputs: every array as float64 DIR/<name>.npy"""
+    arrays = {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def _host_threads() -> int:
@@ -400,6 +419,13 @@ def run_ours(args):
                "single_thread": {"value": cpu1_rate, "unit": UNIT, "cores": 1,
                                  "sample": f"first {s1} events, {cpu1_dt:.1f} s"}}
 
+    dump = {} if args.dump_outputs and rank == 0 else None
+    if dump is not None:
+        if world > 1:
+            q = global_sketch.view(DEPTH, WIDTH).to(torch.float64).cpu().numpy()
+            dump["sketch"] = q * 2.0 ** -bank.frac_bits
+        else:
+            dump["sketch"] = bank.read()[0]
     # free the sketch-stage buffers before the cosine stage
     bank.close()
     ebank.close()
@@ -407,7 +433,9 @@ def run_ours(args):
     torch.cuda.empty_cache()
     cosine = None
     if not args.no_cosine:
-        cosine = run_cosine_stage(ctx, stream, world, rank, local, dev, peaks, args.steps, args.warmup)
+        cosine = run_cosine_stage(ctx, stream, world, rank, local, dev, peaks, args.steps, args.warmup, dump)
+    if dump is not None:
+        _write_dump(args.dump_outputs, dump)
     line = None
     if rank == 0:
         kern_s = (k_ms / max(k_n, 1)) * 1e-3
@@ -544,9 +572,10 @@ def _cpu_cosine_rows(bank_host, rows, k, threads):
 
 
 
-def run_cosine_stage(ctx, stream, world, rank, local, dev, peaks, steps, warmup):
+def run_cosine_stage(ctx, stream, world, rank, local, dev, peaks, steps, warmup, dump=None):
     """One step = K2 normalise + all-gather of the 16-bit rows (N > 1) + K3 + K5 for this rank's block
-    row of the N x N similarity matrix.  Returns the `cosine` object of the JSON line (rank 0)."""
+    row of the N x N similarity matrix.  Returns the `cosine` object of the JSON line (rank 0); fills `dump`
+    (rank 0, --dump-outputs) with the last step's top-k of DUMP_ROWS sampled rows per timed precision."""
     import torch
     import torch.distributed as dist
     import mahout_b200 as mb
@@ -885,6 +914,17 @@ def run_cosine_stage(ctx, stream, world, rank, local, dev, peaks, steps, warmup)
                              "sample": f"{rows_chk} rows x all {C3_ITEMS} columns, {cpu_s:.1f} s; oracle/ C port of "
                                        "DoubleCountMinSketch.cosine + top-k"},
         }
+    if dump is not None:
+        local_rows = np.arange(plan.local_count())
+        pick = np.sort(np.random.default_rng(C3_SEED).choice(local_rows, min(DUMP_ROWS, local_rows.size), replace=False))
+        dump["cosine_rows"] = plan.global_row(pick)
+        sel = torch.from_numpy(pick).to(dev)
+        results = {"tensor": (idx, s, cnt), "rescored": (ridx, rs, rcnt)}
+        if cidx is not None:
+            results["certified"] = (cidx, cs, ccnt)
+        for precision, res in results.items():
+            for part, t in zip(("idx", "sim", "cnt"), res):
+                dump[f"cosine_{precision}_{part}"] = t[sel].cpu().numpy()
     if e2e_router is not None:
         e2e_router.close()
     bank.close()
@@ -975,7 +1015,12 @@ def main():
     ap.add_argument("--c5-cos-events", type=float, default=8e9)
     ap.add_argument("--c5-check-rows", type=float, default=512)
     ap.add_argument("--c5-chunk-rows", type=float, default=8192)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed steps' outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times a calibrated prefix of the stream)")
     if args.impl == "reference":
         run_reference(args)
     else:
