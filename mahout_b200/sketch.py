@@ -478,6 +478,8 @@ def cosine_topk_blocks(ctx: Context, a_rows, a_valid, b_rows, b_valid, depth: in
         ldc = blocks * ((b_count + bn - 1) // bn) * bn
         dense = torch.full((a_count, ldc), float("nan"), dtype=torch.float32, device=dev)
         args.dense_out, args.dense_ld = dense.data_ptr(), ldc
+        torch.cuda.synchronize(ctx.device)   # the fill runs on torch's stream, K3 writes on the context's
+
     import os
     import time
     dbg = os.environ.get("MB200_BENCH_DEBUG") is not None
