@@ -94,7 +94,8 @@ int mb200_release_workspace(mb200_ctx* ctx);
 #define MB200_K_PREPARE 5   /* ingest: hash-table preparation + compaction */
 #define MB200_K_GROUP 6     /* K1 bank mode: histogram + scans + the two partition passes in front of K1 */
 #define MB200_K_ROUTE 7     /* sharded ingest: partition by owner GPU + peer scatter */
-#define MB200_K_COUNT 8
+#define MB200_K_RECOMMEND 8 /* user-based recommender: estimates + candidates + top-N */
+#define MB200_K_COUNT 9
 /* when profiling is on every launch of the kernels above is bracketed with CUDA events on the
  * launching stream; mb200_kernel_time syncs and returns the accumulated ms and launch count
  * since the last reset. */
@@ -213,6 +214,40 @@ int mb200_bank_pair_cosine(mb200_bank* bank, const int64_t* ea, const int64_t* e
  * depths differ (Preconditions.checkArgument, DoubleCountMinSketch.java:117-118). */
 int mb200_bank_cross_cosine(mb200_bank* bank_a, const int64_t* ea, mb200_bank* bank_b,
                             const int64_t* eb, int64_t n, double* out, int mem);
+
+/* ---- user-based recommendation over a bank of user sketches ------------------------------------------------ */
+/* GenericUserBasedRecommender (GenericUserBasedRecommender.java:134-184) with CosineCM's point query, over the
+ * neighbourhood lists of mb200_bank_cosine_topk: nb_idx / nb_sim [rows][nb_ld], nb_cnt [rows] exactly as that call
+ * returns them (host or device memory, so a device-resident top-k feeds straight in).  For user row u and item i the
+ * listed neighbours v != u are visited in list order:
+ *   p = (float) DoubleCountMinSketch.get,  s = clamp(sim, -1, 1) (NaN stays NaN)
+ *   p != 0 and s not NaN:  pref += s * (double) p  (product and sum rounded separately),  tot += s,  count++
+ *   estimate = count <= 1 ? NaN : (float) (pref / tot)
+ * Out-of-range user rows, neighbour indexes, counts and item_col entries are found on the device and fail the call
+ * with MB200_ERR_BAD_ARG. */
+/* doEstimatePreference for q (user row, itemID) pairs -> out[q] (NaN = no estimate).  The neighbourhood of query t
+ * is row nb_row[t] of the nb_rows-row lists (nb_row NULL: row user[t], with nb_rows = the bank's entities). */
+int mb200_bank_estimate_prefs(mb200_bank* bank, const int64_t* nb_idx, const double* nb_sim, const int32_t* nb_cnt,
+                              int64_t nb_rows, int32_t nb_ld, const int64_t* user, const int64_t* nb_row,
+                              const int64_t* item_id, int64_t q, float* out, int mem);
+/* recommend(user, how_many) for m user rows.  Neighbourhood lists [entities][nb_ld] indexed by user row.  Data model
+ * = the items each user row rated, CSR: item_ptr [entities + 1] (item_ptr[0] = 0, item_ptr[entities] = nnz),
+ * item_col [nnz] dense item numbers into item_ids [num_items] (strictly ascending itemIDs).  Candidates = items of
+ * the listed neighbours, minus the user's own unless include_known; NaN estimates dropped; ranked by (value desc,
+ * itemID asc).  out_item / out_value [m][how_many] (unused slots -1 / 0), out_cnt [m].  how_many in [1, 1024]. */
+int mb200_bank_recommend(mb200_bank* bank, const int64_t* nb_idx, const double* nb_sim, const int32_t* nb_cnt,
+                         int32_t nb_ld, const int64_t* item_ptr, const int32_t* item_col, int64_t nnz,
+                         const int64_t* item_ids, int64_t num_items, const int64_t* users, int64_t m, int32_t how_many,
+                         int include_known, int64_t* out_item, float* out_value, int32_t* out_cnt, int mem);
+/* what the last mb200_bank_recommend on the context did: users whose candidates were estimated by streaming the
+ * neighbours' sketch rows through shared memory or by gathering single counters (chosen per user by bytes: rows
+ * c*d*W*8 per candidate chunk against C*c*d*32), candidate chunks, candidates (sum, max), sketch rows streamed,
+ * counters gathered, pipeline stages (0: rows too wide to stage) and candidates per chunk */
+typedef struct mb200_recommend_plan {
+  int64_t stream_users, gather_users, chunks, candidates, candidates_max, stream_rows, gather_loads;
+  int32_t stages, chunk_candidates;
+} mb200_recommend_plan;
+int mb200_recommend_last_plan(mb200_ctx* ctx, mb200_recommend_plan* out);
 
 /* ---- sharded ingest: events travel to the GPU that owns their row ------------------------------ */
 /* Item-hash sharding (SURVEY.md 8e): owner(row) = row mod shards, local row = row div shards.  Every GPU

@@ -115,6 +115,23 @@ public final class NativeSketch {
   /** mb200_bank_update_u8: the narrow wire format (uint32 entity / key, one byte of quanta per event). */
   public static native void updateU8(long bank, ByteBuffer entity, ByteBuffer key, ByteBuffer quanta, long n);
 
+  /**
+   * mb200_bank_estimate_prefs: GenericUserBasedRecommender.doEstimatePreference (GenericUserBasedRecommender.java:
+   * 134-184) with the sketch point query for the (user row, itemID) pairs user[t], itemId[t] over the neighbourhood
+   * lists of cosineTopK (nbIdx / nbSim [rows][nbLd], nbCnt [rows]); out[t] is NaN where there is no estimate.
+   */
+  public static native void estimatePrefs(long bank, long[] nbIdx, double[] nbSim, int[] nbCnt, int nbLd, long[] user,
+                                          long[] itemId, float[] out);
+
+  /**
+   * mb200_bank_recommend: GenericUserBasedRecommender.recommend(userID, howMany) for the user rows `users`.  The data
+   * model is CSR over user rows: itemPtr [rows + 1], itemCol = dense item numbers into itemIds (ascending itemIDs).
+   * outItem / outValue are [users][howMany] (unused -1 / 0), outCnt [users].
+   */
+  public static native void recommend(long bank, long[] nbIdx, double[] nbSim, int[] nbCnt, int nbLd, long[] itemPtr,
+                                      int[] itemCol, long[] itemIds, long[] users, int howMany, boolean includeKnown,
+                                      long[] outItem, float[] outValue, int[] outCnt);
+
   /** mb200_host_alloc / mb200_host_free wrapped as a direct ByteBuffer. */
   public static native ByteBuffer allocPinned(long bytes);
   public static native void freePinned(ByteBuffer buffer);

@@ -246,3 +246,64 @@ JNIEXPORT void JNICALL JNI_FN(updateU8)(JNIEnv* env, jclass c, jlong bank, jobje
   CHECK(mb200_bank_update_u8((mb200_bank*)(intptr_t)bank, e, k, q, n, MB200_MEM_HOST), NULL);
 }
 
+
+/* ---- GenericUserBasedRecommender over the user bank (csrc/recommend.cu) --------------------------------------- */
+JNIEXPORT void JNICALL JNI_FN(estimatePrefs)(JNIEnv* env, jclass c, jlong bank, jlongArray nbIdx, jdoubleArray nbSim,
+                                             jintArray nbCnt, jint nbLd, jlongArray user, jlongArray itemId,
+                                             jfloatArray out) {
+  const jsize rows = (*env)->GetArrayLength(env, nbCnt), q = (*env)->GetArrayLength(env, user);
+  jlong* pi = (*env)->GetLongArrayElements(env, nbIdx, NULL);
+  jdouble* ps = (*env)->GetDoubleArrayElements(env, nbSim, NULL);
+  jint* pc = (*env)->GetIntArrayElements(env, nbCnt, NULL);
+  jlong* pu = (*env)->GetLongArrayElements(env, user, NULL);
+  jlong* pt = (*env)->GetLongArrayElements(env, itemId, NULL);
+  jfloat* po = (*env)->GetFloatArrayElements(env, out, NULL);
+  int rc = (*env)->GetArrayLength(env, itemId) != q || (*env)->GetArrayLength(env, out) != q
+               ? MB200_ERR_BAD_ARG
+               : mb200_bank_estimate_prefs((mb200_bank*)(intptr_t)bank, (const int64_t*)pi, ps, (const int32_t*)pc, rows,
+                                           nbLd, (const int64_t*)pu, NULL, (const int64_t*)pt, q, (float*)po,
+                                           MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, nbIdx, pi, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, nbSim, ps, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, nbCnt, pc, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, user, pu, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemId, pt, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, out, po, 0);
+  CHECK(rc, NULL);
+}
+
+JNIEXPORT void JNICALL JNI_FN(recommend)(JNIEnv* env, jclass c, jlong bank, jlongArray nbIdx, jdoubleArray nbSim,
+                                         jintArray nbCnt, jint nbLd, jlongArray itemPtr, jintArray itemCol,
+                                         jlongArray itemIds, jlongArray users, jint howMany, jboolean includeKnown,
+                                         jlongArray outItem, jfloatArray outValue, jintArray outCnt) {
+  jlong* pi = (*env)->GetLongArrayElements(env, nbIdx, NULL);
+  jdouble* ps = (*env)->GetDoubleArrayElements(env, nbSim, NULL);
+  jint* pc = (*env)->GetIntArrayElements(env, nbCnt, NULL);
+  jlong* pp = (*env)->GetLongArrayElements(env, itemPtr, NULL);
+  jint* pl = (*env)->GetIntArrayElements(env, itemCol, NULL);
+  jlong* pd = (*env)->GetLongArrayElements(env, itemIds, NULL);
+  jlong* pu = (*env)->GetLongArrayElements(env, users, NULL);
+  jlong* oi = (*env)->GetLongArrayElements(env, outItem, NULL);
+  jfloat* ov = (*env)->GetFloatArrayElements(env, outValue, NULL);
+  jint* oc = (*env)->GetIntArrayElements(env, outCnt, NULL);
+  const jsize m = (*env)->GetArrayLength(env, users);
+  int rc = (*env)->GetArrayLength(env, outCnt) != m ||
+                   (int64_t)(*env)->GetArrayLength(env, outItem) != (int64_t)m * howMany ||
+                   (*env)->GetArrayLength(env, outValue) != (*env)->GetArrayLength(env, outItem)
+               ? MB200_ERR_BAD_ARG
+               : mb200_bank_recommend((mb200_bank*)(intptr_t)bank, (const int64_t*)pi, ps, (const int32_t*)pc, nbLd,
+                                      (const int64_t*)pp, (const int32_t*)pl, (*env)->GetArrayLength(env, itemCol),
+                                      (const int64_t*)pd, (*env)->GetArrayLength(env, itemIds), (const int64_t*)pu, m,
+                                      howMany, includeKnown, (int64_t*)oi, (float*)ov, (int32_t*)oc, MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, nbIdx, pi, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, nbSim, ps, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, nbCnt, pc, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemPtr, pp, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, itemCol, pl, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemIds, pd, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, users, pu, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outItem, oi, 0);
+  (*env)->ReleaseFloatArrayElements(env, outValue, ov, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
+  CHECK(rc, NULL);
+}

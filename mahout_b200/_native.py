@@ -18,7 +18,7 @@ ERR_NO_DEVICE, ERR_CM_DELTA, ERR_CM_EPSILON, ERR_UNSUPPORTED, ERR_PULL_TIMEOUT =
 MEM_HOST, MEM_DEVICE = 0, 1
 DTYPE_F16, DTYPE_BF16 = 0, 1
 PRECISION_TENSOR, PRECISION_RESCORED, PRECISION_CERTIFIED = 0, 1, 2
-K_UPDATE, K_NORMALIZE, K_COSINE, K_RESCORE, K_PARSE, K_PREPARE, K_GROUP, K_ROUTE = 0, 1, 2, 3, 4, 5, 6, 7
+K_UPDATE, K_NORMALIZE, K_COSINE, K_RESCORE, K_PARSE, K_PREPARE, K_GROUP, K_ROUTE, K_RECOMMEND = 0, 1, 2, 3, 4, 5, 6, 7, 8
 OPT_GROUP_MIN_EVENTS, OPT_GROUP_PREFETCH, OPT_SINGLE_KERNEL, OPT_MAX_FALLBACK_ROWS = 1, 2, 3, 4
 MAX_DEPTH = 32
 
@@ -82,6 +82,13 @@ class JobStats(C.Structure):
                 ("build_s", C.c_double), ("cosine_s", C.c_double)]
 
 
+class RecommendPlan(C.Structure):
+    """struct mb200_recommend_plan (include/mahout_b200.h)."""
+    _fields_ = [("stream_users", C.c_int64), ("gather_users", C.c_int64), ("chunks", C.c_int64),
+                ("candidates", C.c_int64), ("candidates_max", C.c_int64), ("stream_rows", C.c_int64),
+                ("gather_loads", C.c_int64), ("stages", C.c_int32), ("chunk_candidates", C.c_int32)]
+
+
 class CosinePiece(C.Structure):
     """struct mb200_cosine_piece (include/mahout_b200.h)."""
     _fields_ = [
@@ -131,6 +138,10 @@ _PROTOS = {
     "mb200_bank_pair_cosine": (C.c_int, [vp, vp, vp, i64, vp, C.c_int]),
     "mb200_bank_cross_cosine": (C.c_int, [vp, vp, vp, vp, i64, vp, C.c_int]),
     "mb200_bank_cosine_topk": (C.c_int, [vp, i32, f64, C.c_int, C.c_int, C.c_int, vp, vp, vp, C.c_int]),
+    "mb200_bank_estimate_prefs": (C.c_int, [vp, vp, vp, vp, i64, i32, vp, vp, vp, i64, vp, C.c_int]),
+    "mb200_bank_recommend": (C.c_int, [vp, vp, vp, vp, i32, vp, vp, i64, vp, i64, vp, i64, i32, C.c_int, vp, vp, vp,
+                                       C.c_int]),
+    "mb200_recommend_last_plan": (C.c_int, [vp, C.POINTER(RecommendPlan)]),
     "mb200_row_ld": (i64, [i32]),
     "mb200_valid_words": (i64, [i64]),
     "mb200_bank_normalize": (C.c_int, [vp, C.c_int, vp, vp]),

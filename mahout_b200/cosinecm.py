@@ -88,25 +88,18 @@ class CosineCM:
         return r if math.isnan(r) else float(np.clip(r, -1.0, 1.0))
 
     def doEstimatePreference(self, theUserID: int, theNeighborhood, itemID: int) -> float:
-        """GenericUserBasedRecommender.doEstimatePreference with the sketch point query (:134-184): one
-        batched mb200_bank_query over the neighbourhood, one batched pair cosine; NaN unless at least two
-        neighbours contribute."""
+        """GenericUserBasedRecommender.doEstimatePreference with the sketch point query (:134-184): one batched pair
+        cosine for the neighbours' similarities, then one query of mb200_bank_estimate_prefs over the neighbourhood
+        (same accumulation order as the Java loop); NaN unless at least two neighbours contribute."""
         nb = np.asarray([u for u in np.atleast_1d(theNeighborhood) if u != theUserID], np.int64)
         if np.atleast_1d(theNeighborhood).shape[0] == 0 or nb.shape[0] == 0:
             return math.nan
         rows = self._rows(nb)
-        prefs = self.bank.query(rows, np.full(nb.shape[0], itemID, np.int64)).astype(np.float32)   # (float) cm.get
-        sims = self.userSimilarities(np.full(nb.shape[0], theUserID, np.int64), nb)
-        preference = totalSimilarity = 0.0
-        count = 0
-        for p, s in zip(prefs.tolist(), sims.tolist()):             # same accumulation order as the Java loop
-            if p != 0.0 and not math.isnan(s):
-                preference += s * p
-                totalSimilarity += s
-                count += 1
-        if count <= 1:
-            return math.nan
-        return float(np.float32(preference / totalSimilarity))
+        u = self._rows(theUserID)
+        sims = self.bank.pair_cosine(np.full(nb.shape[0], u[0], np.int64), rows)   # clamped on the device
+        out = self.bank.estimate_prefs(rows[None, :], sims[None, :], np.array([nb.shape[0]], np.int32), u,
+                                       np.array([itemID], np.int64), nb_row=np.zeros(1, np.int64))
+        return float(out[0])
 
     def getExportedCMProfile(self, userID: int) -> np.ndarray:
         r = int(self._rows(userID)[0])

@@ -1,0 +1,68 @@
+"""GenericUserBasedRecommender over CosineCM's user sketches, on the GPU.
+
+Mirrors cf/taste/impl/recommender/GenericUserBasedRecommender.java with the fork's sketch point query
+(GenericUserBasedRecommender.java:134-184): NearestNUserNeighborhood(n, minSimilarity) is the bank's re-scored
+cosine top-n (similarities bit-equal to the pair cosine, ties by lower user row), computed once and kept on the
+device; candidate items are the neighbours' items (getAllOtherItems), every candidate is estimated over the
+neighbourhood and the best howMany are kept under (value desc, itemID asc) (TopItems, with this project's tie rule).
+Both run in K_RECOMMEND (csrc/recommend.cu).
+
+Documented deviation: cosine_topk never admits similarities <= 0 (the RowSimilarityJob rule), where
+NearestNUserNeighborhood would when fewer than n users are positively similar.
+"""
+from __future__ import annotations
+
+import numpy as np
+
+from .cosinecm import CosineCM
+
+
+class GenericUserBasedRecommender:
+    def __init__(self, cm: CosineCM, neighborhood_size: int, min_similarity: float | None = None):
+        import torch
+        self.cm = cm
+        self.bank = cm.bank
+        self.neighborhood_size = int(neighborhood_size)
+        dev = f"cuda:{self.bank.ctx.device}"
+        # the data model: the items each user row rated, CSR by user row, items as dense numbers of item_ids
+        rows = np.searchsorted(cm.user_ids, cm._u_sorted)
+        self.item_ids = np.unique(cm._i_sorted)
+        col = np.searchsorted(self.item_ids, cm._i_sorted)
+        pairs = np.unique(rows.astype(np.int64) * self.item_ids.shape[0] + col)   # a user's item set
+        prow, pcol = pairs // self.item_ids.shape[0], pairs % self.item_ids.shape[0]
+        ptr = np.zeros(cm.user_ids.shape[0] + 1, np.int64)
+        np.cumsum(np.bincount(prow, minlength=cm.user_ids.shape[0]), out=ptr[1:])
+        self._csr = tuple(torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+                          for a in (ptr, pcol.astype(np.int32), self.item_ids))
+        self.nb_idx, self.nb_sim, self.nb_cnt = self.bank.cosine_topk(
+            self.neighborhood_size, threshold=min_similarity, exclude_self=True, precision="rescored", device=True)
+
+    def getUserNeighborhood(self, userID: int) -> np.ndarray:
+        r = int(self.cm._rows(userID)[0])
+        n = int(self.nb_cnt[r])
+        return self.cm.user_ids[self.nb_idx[r, :n].cpu().numpy()]
+
+    def recommend_all(self, howMany: int, userIDs=None, includeKnownItems: bool = False):
+        """(user_ids [m], items [m, howMany] itemIDs (-1 unused), values [m, howMany] float32, counts [m])"""
+        import torch
+        user_ids = self.cm.user_ids if userIDs is None else np.atleast_1d(np.asarray(userIDs, np.int64))
+        rows = np.arange(self.cm.user_ids.shape[0], dtype=np.int64) if userIDs is None else self.cm._rows(user_ids)
+        dev = f"cuda:{self.bank.ctx.device}"
+        items, vals, cnt = self.bank.recommend(self.nb_idx, self.nb_sim, self.nb_cnt, *self._csr,
+                                               torch.from_numpy(rows).to(dev), howMany, includeKnownItems)
+        return user_ids, items.cpu().numpy(), vals.cpu().numpy(), cnt.cpu().numpy()
+
+    def recommend(self, userID: int, howMany: int, includeKnownItems: bool = False):
+        """list of (itemID, value), best first"""
+        _, items, vals, cnt = self.recommend_all(howMany, [userID], includeKnownItems)
+        n = int(cnt[0])
+        return [(int(i), float(v)) for i, v in zip(items[0, :n], vals[0, :n])]
+
+    def estimate_preferences(self, userIDs, itemIDs) -> np.ndarray:
+        """doEstimatePreference over the recommender's neighbourhoods for (userID, itemID) pairs -- the held-out
+        pairs of one fold of a K-fold evaluation (RMSRecommenderEvaluatorKFold); float32, NaN = no estimate"""
+        import torch
+        dev = f"cuda:{self.bank.ctx.device}"
+        rows = torch.from_numpy(self.cm._rows(userIDs)).to(dev)
+        items = torch.from_numpy(np.ascontiguousarray(np.atleast_1d(itemIDs), np.int64)).to(dev)
+        return self.bank.estimate_prefs(self.nb_idx, self.nb_sim, self.nb_cnt, rows, items).cpu().numpy()

@@ -408,6 +408,60 @@ class SketchBank:
             _DTYPES[dtype], _PRECISIONS[precision], pi, ps, pc, mem), self.ctx.handle)
         return idx, sim, cnt
 
+    # ---- user-based recommendation over the neighbourhood lists of cosine_topk -------------------------------
+    def estimate_prefs(self, nb_idx, nb_sim, nb_cnt, user, item_id, nb_row=None):
+        """GenericUserBasedRecommender.doEstimatePreference for q (user row, itemID) pairs over the neighbourhood
+        lists (nb_idx [rows, ld], nb_sim [rows, ld], nb_cnt [rows], what cosine_topk returns).  The neighbourhood of
+        query t is row nb_row[t] (None: row user[t]).  Returns float32 [q], NaN where there is no estimate."""
+        ni = _Arg(nb_idx, np.int64, "int64")
+        ns = _Arg(nb_sim, np.float64, "float64")
+        nc = _Arg(nb_cnt, np.int32, "int32")
+        u = _Arg(user, np.int64, "int64")
+        it = _Arg(item_id, np.int64, "int64")
+        nr = _Arg(nb_row, np.int64, "int64", allow_none=True)
+        rows = nc.n
+        ld = ni.n // rows if rows else 1
+        if ni.n != rows * ld or ns.n != ni.n or it.n != u.n or (nr.ptr is not None and nr.n != u.n):
+            raise ValueError("nb_idx / nb_sim must be [rows, ld] with rows = len(nb_cnt); user, item_id (and nb_row) "
+                             "the same length")
+        mem = _same_mem(ni, ns, nc, u, it, nr)
+        out, optr = _out((u.n,), np.float32, "float32", mem, self.ctx.device)
+        N.check(N.lib().mb200_bank_estimate_prefs(self.handle, ni.ptr, ns.ptr, nc.ptr, rows, max(ld, 1), u.ptr, nr.ptr,
+                                                  it.ptr, u.n, optr, mem), self.ctx.handle)
+        return out
+
+    def recommend(self, nb_idx, nb_sim, nb_cnt, item_ptr, item_col, item_ids, users, how_many: int,
+                  include_known: bool = False):
+        """GenericUserBasedRecommender.recommend for the user rows `users`: neighbourhood lists [E, ld] as cosine_topk
+        returns them, data model as CSR over user rows (item_ptr [E+1], item_col = dense item numbers into item_ids,
+        strictly ascending itemIDs).  Returns (items [m, how_many] int64, values [m, how_many] float32, counts [m]
+        int32); unused slots are -1 / 0."""
+        ni = _Arg(nb_idx, np.int64, "int64")
+        ns = _Arg(nb_sim, np.float64, "float64")
+        nc = _Arg(nb_cnt, np.int32, "int32")
+        ip = _Arg(item_ptr, np.int64, "int64")
+        ic = _Arg(item_col, np.int32, "int32")
+        ii = _Arg(item_ids, np.int64, "int64")
+        us = _Arg(users, np.int64, "int64")
+        ld = ni.n // self.E
+        if nc.n != self.E or ni.n != self.E * ld or ns.n != ni.n or ip.n != self.E + 1:
+            raise ValueError("nb_idx / nb_sim must be [E, ld], nb_cnt [E] and item_ptr [E + 1] for the bank's E rows")
+        mem = _same_mem(ni, ns, nc, ip, ic, ii, us)
+        m, n = us.n, int(how_many)
+        items, pi = _out((m, max(n, 0)), np.int64, "int64", mem, self.ctx.device)
+        vals, pv = _out((m, max(n, 0)), np.float32, "float32", mem, self.ctx.device)
+        cnt, pc = _out((m,), np.int32, "int32", mem, self.ctx.device)
+        N.check(N.lib().mb200_bank_recommend(self.handle, ni.ptr, ns.ptr, nc.ptr, max(ld, 1), ip.ptr, ic.ptr, ic.n,
+                                             ii.ptr, ii.n, us.ptr, m, n, int(bool(include_known)), pi, pv, pc, mem),
+                self.ctx.handle)
+        return items, vals, cnt
+
+    def recommend_plan(self) -> dict:
+        """what the last recommend on this bank's context did (mb200_recommend_last_plan)"""
+        pl = N.RecommendPlan()
+        N.check(N.lib().mb200_recommend_last_plan(self.ctx.handle, C.byref(pl)), self.ctx.handle)
+        return {f: getattr(pl, f) for f, _ in N.RecommendPlan._fields_}
+
     def normalize(self, dtype: str = "f16"):
         """K2: unit-norm 16-bit rows [d, E, ld] and validity words [d, valid_words(E)] (torch, device)."""
         import torch
