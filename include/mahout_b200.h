@@ -94,7 +94,7 @@ int mb200_release_workspace(mb200_ctx* ctx);
 #define MB200_K_PREPARE 5   /* ingest: hash-table preparation + compaction */
 #define MB200_K_GROUP 6     /* K1 bank mode: histogram + scans + the two partition passes in front of K1 */
 #define MB200_K_ROUTE 7     /* sharded ingest: partition by owner GPU + peer scatter */
-#define MB200_K_RECOMMEND 8 /* user-based recommender: estimates + candidates + top-N */
+#define MB200_K_RECOMMEND 8 /* recommenders: user-based estimates + candidates + top-N; item-based rank sort + aggregation */
 #define MB200_K_COUNT 9
 /* when profiling is on every launch of the kernels above is bracketed with CUDA events on the
  * launching stream; mb200_kernel_time syncs and returns the accumulated ms and launch count
@@ -248,6 +248,56 @@ typedef struct mb200_recommend_plan {
   int32_t stages, chunk_candidates;
 } mb200_recommend_plan;
 int mb200_recommend_last_plan(mb200_ctx* ctx, mb200_recommend_plan* out);
+
+/* ---- item-based recommendation over the item top-k lists (RecommenderJob's aggregate-and-recommend phase) ---- */
+/* UserVectorSplitterMapper + PartialMultiplyMapper + AggregateAndRecommendReducer of upstream RecommenderJob
+ * (cf/taste/hadoop/item/), restated in DESIGN.md section 3.  For user row u:
+ *   prefs equal to +-0 are not part of the user vector; with more than max_prefs_per_user (P) prefs, T = the P-th
+ *   largest |pref| and only the prefs with |pref| >= T are considered (ties at T all kept);
+ *   the considered prefs are visited in ascending item row j, and for every entry (i, s) of row j's list
+ *     num[i] += s * (double) p_j  (product and sum rounded separately),  den[i] += |s|,  cnt[i]++
+ *   (boolean_data: num[i] += s); the considered items themselves get no prediction (upstream's NaN diagonal);
+ *   prediction = cnt >= 2 ? (float) (num / den) : none   (boolean_data: (float) num)
+ *   predictions that are NaN or <= Float.MIN_VALUE are dropped, then the allowed-items mask; ranked by
+ *   (value desc, itemID asc), the first how_many kept.
+ * Every array is in the memory space `mem`.  Out-of-range list entries or counts, a malformed user_ptr, pref_row
+ * entries out of range or not strictly ascending within a user, and user rows out of range are found on the device
+ * and fail the call with MB200_ERR_BAD_ARG. */
+typedef struct mb200_itembased_args {
+  /* the similarity matrix: row j = item j's top-k list exactly as mb200_bank_cosine_topk writes it */
+  const int64_t* sim_idx;  /* [num_items][sim_ld] item rows */
+  const double* sim_val;   /* [num_items][sim_ld] */
+  const int32_t* sim_cnt;  /* [num_items] */
+  int64_t num_items;
+  int32_t sim_ld;
+  /* the user vectors, CSR over user rows: prefs of row u are [user_ptr[u], user_ptr[u+1]), item rows ascending */
+  const int64_t* user_ptr; /* [num_users + 1] */
+  const int32_t* pref_row; /* [nnz] */
+  const float* pref_val;   /* [nnz] */
+  int64_t num_users, nnz;
+  const int64_t* item_ids; /* [num_items] row -> itemID (output and tie rule; any order) */
+  const uint32_t* allowed; /* optional [ceil(num_items / 32)] bit mask over item rows (--itemsFile); NULL = all */
+  const int64_t* users;    /* [m] user rows to serve */
+  int64_t m;
+  int32_t how_many;            /* [1, 1024] */
+  int32_t max_prefs_per_user;  /* >= 1 */
+  int32_t boolean_data;
+  int64_t* out_item;  /* [m][how_many] itemIDs, -1 unused */
+  float* out_value;   /* [m][how_many], 0 unused */
+  int32_t* out_cnt;   /* [m] */
+  int32_t mem;        /* MB200_MEM_HOST or MB200_MEM_DEVICE, for every array above */
+} mb200_itembased_args;
+int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args);
+/* what the last mb200_recommend_item_based on the context did: users served, users whose accumulators were an
+ * open-addressing table in shared memory (smem) or dense per-CTA slices over num_items (dense) -- chosen per user
+ * from B = the sum of the considered lists' counts --, list entries visited (partial products; sum and max over
+ * users), users with more than max_prefs_per_user prefs (a threshold T was computed), the largest candidate count,
+ * table slots per CTA and dense slices */
+typedef struct mb200_itembased_plan {
+  int64_t users, smem_users, dense_users, entries, entries_max, pruned_users, candidates_max;
+  int32_t table_slots, dense_slices;
+} mb200_itembased_plan;
+int mb200_itembased_last_plan(mb200_ctx* ctx, mb200_itembased_plan* out);
 
 /* ---- sharded ingest: events travel to the GPU that owns their row ------------------------------ */
 /* Item-hash sharding (SURVEY.md 8e): owner(row) = row mod shards, local row = row div shards.  Every GPU

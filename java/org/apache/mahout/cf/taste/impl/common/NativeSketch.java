@@ -132,6 +132,19 @@ public final class NativeSketch {
                                       int[] itemCol, long[] itemIds, long[] users, int howMany, boolean includeKnown,
                                       long[] outItem, float[] outValue, int[] outCnt);
 
+  /**
+   * mb200_recommend_item_based: RecommenderJob's aggregate-and-recommend phase (UserVectorSplitterMapper,
+   * PartialMultiplyMapper, AggregateAndRecommendReducer) for the user rows `users`.  The similarity matrix is the
+   * item top-k lists of cosineTopK (simIdx / simVal [items][simLd], simCnt [items]); the user vectors are CSR over
+   * user rows: userPtr [users + 1], prefRow = item rows ascending within a user, prefVal.  itemIds maps rows to
+   * itemIDs; allowed is an optional bit mask over item rows (null = every item).  outItem / outValue are
+   * [users][howMany] (unused -1 / 0), outCnt [users].
+   */
+  public static native void recommendItemBased(long ctx, long[] simIdx, double[] simVal, int[] simCnt, int simLd,
+                                               long[] userPtr, int[] prefRow, float[] prefVal, long[] itemIds,
+                                               int[] allowed, long[] users, int howMany, int maxPrefsPerUser,
+                                               boolean booleanData, long[] outItem, float[] outValue, int[] outCnt);
+
   /** mb200_host_alloc / mb200_host_free wrapped as a direct ByteBuffer. */
   public static native ByteBuffer allocPinned(long bytes);
   public static native void freePinned(ByteBuffer buffer);

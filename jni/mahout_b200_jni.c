@@ -307,3 +307,56 @@ JNIEXPORT void JNICALL JNI_FN(recommend)(JNIEnv* env, jclass c, jlong bank, jlon
   (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
   CHECK(rc, NULL);
 }
+
+/* ---- RecommenderJob's aggregate-and-recommend phase over the item top-k lists (csrc/recommend.cu) ------------- */
+JNIEXPORT void JNICALL JNI_FN(recommendItemBased)(JNIEnv* env, jclass c, jlong ctx, jlongArray simIdx,
+                                                  jdoubleArray simVal, jintArray simCnt, jint simLd, jlongArray userPtr,
+                                                  jintArray prefRow, jfloatArray prefVal, jlongArray itemIds,
+                                                  jintArray allowed, jlongArray users, jint howMany,
+                                                  jint maxPrefsPerUser, jboolean booleanData, jlongArray outItem,
+                                                  jfloatArray outValue, jintArray outCnt) {
+  mb200_itembased_args a;
+  a.sim_idx = (const int64_t*)(*env)->GetLongArrayElements(env, simIdx, NULL);
+  a.sim_val = (*env)->GetDoubleArrayElements(env, simVal, NULL);
+  a.sim_cnt = (const int32_t*)(*env)->GetIntArrayElements(env, simCnt, NULL);
+  a.num_items = (*env)->GetArrayLength(env, simCnt);
+  a.sim_ld = simLd;
+  a.user_ptr = (const int64_t*)(*env)->GetLongArrayElements(env, userPtr, NULL);
+  a.pref_row = (const int32_t*)(*env)->GetIntArrayElements(env, prefRow, NULL);
+  a.pref_val = (*env)->GetFloatArrayElements(env, prefVal, NULL);
+  a.num_users = (int64_t)(*env)->GetArrayLength(env, userPtr) - 1;
+  a.nnz = (*env)->GetArrayLength(env, prefRow);
+  a.item_ids = (const int64_t*)(*env)->GetLongArrayElements(env, itemIds, NULL);
+  a.allowed = allowed ? (const uint32_t*)(*env)->GetIntArrayElements(env, allowed, NULL) : NULL;
+  a.users = (const int64_t*)(*env)->GetLongArrayElements(env, users, NULL);
+  a.m = (*env)->GetArrayLength(env, users);
+  a.how_many = howMany;
+  a.max_prefs_per_user = maxPrefsPerUser;
+  a.boolean_data = booleanData;
+  a.out_item = (int64_t*)(*env)->GetLongArrayElements(env, outItem, NULL);
+  a.out_value = (*env)->GetFloatArrayElements(env, outValue, NULL);
+  a.out_cnt = (int32_t*)(*env)->GetIntArrayElements(env, outCnt, NULL);
+  a.mem = MB200_MEM_HOST;
+  int rc = (int64_t)(*env)->GetArrayLength(env, simIdx) != a.num_items * simLd ||
+                   (*env)->GetArrayLength(env, simVal) != (*env)->GetArrayLength(env, simIdx) ||
+                   (*env)->GetArrayLength(env, prefVal) != a.nnz || (*env)->GetArrayLength(env, itemIds) != a.num_items ||
+                   (allowed && (*env)->GetArrayLength(env, allowed) != (a.num_items + 31) / 32) ||
+                   (*env)->GetArrayLength(env, outCnt) != a.m ||
+                   (int64_t)(*env)->GetArrayLength(env, outItem) != a.m * howMany ||
+                   (*env)->GetArrayLength(env, outValue) != (*env)->GetArrayLength(env, outItem)
+               ? MB200_ERR_BAD_ARG
+               : mb200_recommend_item_based((mb200_ctx*)(intptr_t)ctx, &a);
+  (*env)->ReleaseLongArrayElements(env, simIdx, (jlong*)a.sim_idx, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, simVal, (jdouble*)a.sim_val, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, simCnt, (jint*)a.sim_cnt, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, userPtr, (jlong*)a.user_ptr, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, prefRow, (jint*)a.pref_row, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, prefVal, (jfloat*)a.pref_val, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemIds, (jlong*)a.item_ids, JNI_ABORT);
+  if (allowed) (*env)->ReleaseIntArrayElements(env, allowed, (jint*)a.allowed, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, users, (jlong*)a.users, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outItem, (jlong*)a.out_item, 0);
+  (*env)->ReleaseFloatArrayElements(env, outValue, a.out_value, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, (jint*)a.out_cnt, 0);
+  CHECK(rc, (mb200_ctx*)(intptr_t)ctx);
+}

@@ -89,6 +89,23 @@ class RecommendPlan(C.Structure):
                 ("gather_loads", C.c_int64), ("stages", C.c_int32), ("chunk_candidates", C.c_int32)]
 
 
+class ItemBasedArgs(C.Structure):
+    """struct mb200_itembased_args (include/mahout_b200.h)."""
+    _fields_ = [("sim_idx", C.c_void_p), ("sim_val", C.c_void_p), ("sim_cnt", C.c_void_p), ("num_items", C.c_int64),
+                ("sim_ld", C.c_int32), ("user_ptr", C.c_void_p), ("pref_row", C.c_void_p), ("pref_val", C.c_void_p),
+                ("num_users", C.c_int64), ("nnz", C.c_int64), ("item_ids", C.c_void_p), ("allowed", C.c_void_p),
+                ("users", C.c_void_p), ("m", C.c_int64), ("how_many", C.c_int32), ("max_prefs_per_user", C.c_int32),
+                ("boolean_data", C.c_int32), ("out_item", C.c_void_p), ("out_value", C.c_void_p),
+                ("out_cnt", C.c_void_p), ("mem", C.c_int32)]
+
+
+class ItemBasedPlan(C.Structure):
+    """struct mb200_itembased_plan (include/mahout_b200.h)."""
+    _fields_ = [("users", C.c_int64), ("smem_users", C.c_int64), ("dense_users", C.c_int64), ("entries", C.c_int64),
+                ("entries_max", C.c_int64), ("pruned_users", C.c_int64), ("candidates_max", C.c_int64),
+                ("table_slots", C.c_int32), ("dense_slices", C.c_int32)]
+
+
 class CosinePiece(C.Structure):
     """struct mb200_cosine_piece (include/mahout_b200.h)."""
     _fields_ = [
@@ -142,6 +159,8 @@ _PROTOS = {
     "mb200_bank_recommend": (C.c_int, [vp, vp, vp, vp, i32, vp, vp, i64, vp, i64, vp, i64, i32, C.c_int, vp, vp, vp,
                                        C.c_int]),
     "mb200_recommend_last_plan": (C.c_int, [vp, C.POINTER(RecommendPlan)]),
+    "mb200_recommend_item_based": (C.c_int, [vp, C.POINTER(ItemBasedArgs)]),
+    "mb200_itembased_last_plan": (C.c_int, [vp, C.POINTER(ItemBasedPlan)]),
     "mb200_row_ld": (i64, [i32]),
     "mb200_valid_words": (i64, [i64]),
     "mb200_bank_normalize": (C.c_int, [vp, C.c_int, vp, vp]),

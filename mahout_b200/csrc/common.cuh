@@ -71,6 +71,8 @@ struct mb200_ctx {
   int64_t stat_events = 0, stat_rows = 0, stat_fallback = 0, stat_h2d = 0, stat_d2h = 0;
   struct mb200_cosine_job* active_job = nullptr;  // the cosine stage's workspaces serve one job at a time
   mb200_recommend_plan last_recommend_plan = {};  // mb200_recommend_last_plan
+  mb200_itembased_plan last_itembased_plan = {};  // mb200_itembased_last_plan
+  int64_t itembased_dense_items = -1, itembased_dense_slices = -1;  // layout of the zeroed dense slices (slot 62)
 };
 
 // borrows workspace slots from the context in request order; nothing is freed on return

@@ -19,6 +19,10 @@
 //      the cheaper by bytes (c*d*W*8 per chunk against C*c*d*32) is taken per user; rows that do not fit twice in
 //      shared memory always gather;
 //   3. top-N by radix select on (value, position) keys + a bitonic sort of the survivors in shared memory.
+//
+// k_itembased: RecommenderJob's aggregate-and-recommend phase over the item top-k lists (DESIGN.md section 3) --
+// per user, the considered prefs' lists are summed into an open-addressing table in shared memory or a dense
+// per-CTA slice (chosen from the entry count), then the same top-N as k_recommend.
 #include <math.h>
 #include <stdlib.h>
 
@@ -163,7 +167,8 @@ __device__ __forceinline__ long long nb_at(const RecArgs& a, long long u, int j)
   return (v == u || v < 0 || v >= a.E) ? -1 : v;
 }
 
-// block-wide exclusive scan of one int per thread (REC_THREADS); returns the total through *total
+// block-wide exclusive scan of one int per thread (NT threads); returns the total through *total
+template <int NT>
 __device__ __forceinline__ int block_exscan(int x, int* sh, int* total) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int inc = x;
@@ -174,16 +179,16 @@ __device__ __forceinline__ int block_exscan(int x, int* sh, int* total) {
   if (lane == 31) sh[warp] = inc;
   __syncthreads();
   if (warp == 0) {
-    int w = lane < REC_THREADS / 32 ? sh[lane] : 0;
+    int w = lane < NT / 32 ? sh[lane] : 0;
     for (int o = 1; o < 32; o <<= 1) {
       const int y = __shfl_up_sync(0xffffffffu, w, o);
       if (lane >= o) w += y;
     }
-    if (lane < REC_THREADS / 32) sh[lane] = w;  // inclusive per warp
+    if (lane < NT / 32) sh[lane] = w;  // inclusive per warp
   }
   __syncthreads();
   const int before = (warp ? sh[warp - 1] : 0) + inc - x;
-  *total = sh[REC_THREADS / 32 - 1];
+  *total = sh[NT / 32 - 1];
   __syncthreads();
   return before;
 }
@@ -194,6 +199,83 @@ __device__ __forceinline__ unsigned long long rank_key(float v, int pos) {
   uint32_t b = __float_as_uint(v == 0.0f ? 0.0f : v);  // -0.0 ranks as 0.0
   b = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
   return ((unsigned long long)b << 32) | (unsigned long long)(0xFFFFFFFFu - (uint32_t)pos);
+}
+
+// top-N of C 64-bit keys (0 = none; the others distinct): the keys >= the how_many-th largest, sorted descending into
+// sortbuf[0, n_out) (REC_MAX_N entries); returns n_out.  A radix select (8 passes of 8 bits) finds the how_many-th
+// key, a bitonic sort in shared memory orders the survivors.  Uses bcast[1..3].
+template <int NT>
+__device__ int topn_keys(const unsigned long long* keys, int C, int how_many, unsigned* hist, int* scan_sh,
+                         long long* bcast, unsigned long long* sortbuf) {
+  const int tid = threadIdx.x;
+  int valid = 0, nvalid = 0;
+  for (int pos = tid; pos < C; pos += NT) valid += keys[pos] != 0ull;
+  block_exscan<NT>(valid, scan_sh, &nvalid);
+  unsigned long long thr = 1ull;  // keys >= thr are kept
+  if (nvalid > how_many) {
+    unsigned long long prefix = 0ull, mask = 0ull;
+    unsigned want = (unsigned)how_many;
+    for (int shift = 56; shift >= 0; shift -= 8) {
+      for (int t = tid; t < 256; t += NT) hist[t] = 0u;
+      __syncthreads();
+      for (int pos = tid; pos < C; pos += NT) {
+        const unsigned long long k = keys[pos];
+        if (k && (k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+      }
+      __syncthreads();
+      if (tid == 0) {
+        unsigned acc = 0;
+        for (int b = 255; b >= 0; b--) {
+          if (acc + hist[b] >= want) {
+            prefix |= (unsigned long long)b << shift;
+            want -= acc;
+            break;
+          }
+          acc += hist[b];
+        }
+        bcast[1] = (long long)prefix;
+        bcast[2] = (long long)want;
+      }
+      __syncthreads();
+      prefix = (unsigned long long)bcast[1];
+      want = (unsigned)bcast[2];
+      mask |= 255ull << shift;
+      __syncthreads();
+    }
+    thr = prefix;  // keys are distinct: exactly how_many keys are >= the how_many-th largest
+  }
+  const int n_out = nvalid < how_many ? nvalid : how_many;
+  int npad = 1;
+  while (npad < n_out) npad <<= 1;
+  for (int t = tid; t < npad; t += NT) sortbuf[t] = 0ull;
+  if (tid == 0) bcast[3] = 0;
+  __syncthreads();
+  for (int pos = tid; pos < C; pos += NT) {
+    const unsigned long long k = keys[pos];
+    if (k && k >= thr) {
+      const unsigned long long at = atomicAdd(reinterpret_cast<unsigned long long*>(&bcast[3]), 1ull);
+      if (at < (unsigned long long)npad) sortbuf[at] = k;
+    }
+  }
+  __syncthreads();
+  // bitonic sort, descending
+  for (int size = 2; size <= npad; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = tid; t < npad; t += NT) {
+        const int partner = t ^ stride;
+        if (partner > t) {
+          const bool desc = (t & size) == 0;
+          const unsigned long long x = sortbuf[t], y = sortbuf[partner];
+          if (desc ? (x < y) : (x > y)) {
+            sortbuf[t] = y;
+            sortbuf[partner] = x;
+          }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  return n_out;
 }
 
 __global__ void __launch_bounds__(REC_THREADS, 1) k_recommend(const RecArgs a) {
@@ -298,7 +380,7 @@ __global__ void __launch_bounds__(REC_THREADS, 1) k_recommend(const RecArgs a) {
     int mine = 0;
     for (int w = w0; w < w1; w++) mine += __popc(bitmap[w]);
     int C = 0;
-    int at = block_exscan(mine, scan_sh, &C);
+    int at = block_exscan<REC_THREADS>(mine, scan_sh, &C);
     for (int w = w0; w < w1; w++) {
       unsigned b = bitmap[w];
       while (b) {
@@ -308,8 +390,8 @@ __global__ void __launch_bounds__(REC_THREADS, 1) k_recommend(const RecArgs a) {
       }
     }
     int tot_bad = 0, tot_c = 0;
-    block_exscan(bad, scan_sh, &tot_bad);
-    block_exscan(c_eff, scan_sh, &tot_c);
+    block_exscan<REC_THREADS>(bad, scan_sh, &tot_bad);
+    block_exscan<REC_THREADS>(c_eff, scan_sh, &tot_c);
     c_eff = tot_c;
     if (tot_bad && tid == 0) atomicAdd(&a.plan[PL_BAD], (unsigned long long)tot_bad);
     // cand[] is written by other threads of the block: ordered by the barriers of the scans above
@@ -420,26 +502,193 @@ __global__ void __launch_bounds__(REC_THREADS, 1) k_recommend(const RecArgs a) {
     }
 
     // ---- 3. top-N ------------------------------------------------------------------------------------------
-    int valid = 0, nvalid = 0;
-    for (int pos = tid; pos < C; pos += REC_THREADS) valid += keys[pos] != 0ull;
-    block_exscan(valid, scan_sh, &nvalid);
-    unsigned long long thr = 1ull;  // keys >= thr are kept
-    if (nvalid > a.how_many) {
-      unsigned long long prefix = 0ull, mask = 0ull;
-      unsigned want = (unsigned)a.how_many;
-      for (int shift = 56; shift >= 0; shift -= 8) {
-        if (tid < 256) hist[tid] = 0u;
+    const int n_out = topn_keys<REC_THREADS>(keys, C, a.how_many, hist, scan_sh, bcast, sortbuf);
+    for (int t = tid; t < n_out; t += REC_THREADS) {
+      const int pos = (int)(0xFFFFFFFFu - (uint32_t)sortbuf[t]);
+      out_item[t] = __ldg(a.item_ids + cand[pos]);
+      out_value[t] = vals[pos];
+    }
+    if (tid == 0) a.out_cnt[i] = n_out;
+    __syncthreads();
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// K_RECOMMEND, item-based: RecommenderJob's aggregate-and-recommend phase over the item top-k lists
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int IB_THREADS = 128;
+constexpr int IB_TABLE_LOG2 = 11;
+constexpr int IB_TABLE = 1 << IB_TABLE_LOG2;  // open-addressing slots per CTA
+constexpr int IB_TABLE_MAX = IB_TABLE / 2;    // users with more list entries than this take a dense slice
+constexpr int IB_SORT_TILE = 2048;            // itemID rank sort: elements per shared-memory tile
+constexpr size_t IB_SMEM = (size_t)IB_TABLE * (8 + 8 + 4 + 4) + REC_MAX_N * 8 + 8 * 8 + 32 * 8 + 256 * 4 + 32 * 4;
+constexpr size_t IB_DENSE_MAX_BYTES = 4ull << 30;  // dense slices of one call, all CTAs together
+
+enum { IP_SMEM = 0, IP_DENSE, IP_ENTRIES, IP_ENTRIES_MAX, IP_PRUNED, IP_CAND_MAX, IP_BAD, IP_NEXT, IP_WORDS };
+
+struct IbArgs {
+  const long long* sim_idx;
+  const double* sim_val;
+  const int* sim_cnt;
+  long long num_items;
+  int ld;
+  const long long* user_ptr;
+  const int* pref_row;
+  const float* pref_val;
+  long long num_users, nnz;
+  const long long* item_ids;
+  const int* rank_of;  // [num_items] row -> rank of its itemID among all itemIDs
+  const int* row_at;   // [num_items] rank -> row
+  const unsigned* allowed;
+  const long long* users;
+  long long m;
+  int how_many, max_prefs, boolean_data;
+  long long* out_item;
+  float* out_value;
+  int* out_cnt;
+  // dense slices [slices][num_items] each; num / den / cnt are all zero between users
+  double* d_num;
+  double* d_den;
+  int* d_cnt;
+  int* d_touched;
+  unsigned long long* d_key;
+  int* d_lock;  // [slices]
+  int slices;
+  unsigned long long* plan;
+};
+
+template <int NT>
+__device__ __forceinline__ long long block_sum(long long x, long long* sh) {
+  for (int o = 16; o; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = x;
+  __syncthreads();
+  long long t = 0;
+  for (int w = 0; w < NT / 32; w++) t += sh[w];
+  __syncthreads();
+  return t;
+}
+
+__device__ __forceinline__ uint32_t ib_hash(int key) { return ((uint32_t)key * 0x9E3779B1u) >> (32 - IB_TABLE_LOG2); }
+
+// slot of `key` in the table, inserted if absent (the table never fills: at most IB_TABLE_MAX keys)
+__device__ __forceinline__ int ib_insert(int* tkey, int key) {
+  uint32_t h = ib_hash(key);
+  for (;;) {
+    const int k = *(volatile int*)&tkey[h];
+    if (k == key) return (int)h;
+    if (k == -1) {
+      const int old = atomicCAS(&tkey[h], -1, key);
+      if (old == -1 || old == key) return (int)h;
+    }
+    h = (h + 1) & (IB_TABLE - 1);
+  }
+}
+
+__device__ __forceinline__ int ib_find(const int* tkey, int key) {
+  uint32_t h = ib_hash(key);
+  for (;;) {
+    const int k = tkey[h];
+    if (k == key) return (int)h;
+    if (k == -1) return -1;
+    h = (h + 1) & (IB_TABLE - 1);
+  }
+}
+
+// AggregateAndRecommendReducer's prediction of item row `row` as a ranking key: order-preserving float bits, then
+// 2^32-1-rank(itemID), so that (value desc, itemID asc) is one descending order; 0 = no recommendation
+__device__ __forceinline__ unsigned long long ib_key(const IbArgs& a, int row, double num, double den, int cnt) {
+  float v;
+  if (a.boolean_data) {
+    v = __double2float_rn(num);
+  } else {
+    if (cnt < 2) return 0ull;  // "preference estimations must be based on at least 2 datapoints"
+    v = __double2float_rn(num / den);
+  }
+  if (!(v > __int_as_float(1))) return 0ull;  // NaN, and TopItemsQueue's sentinel Float.MIN_VALUE
+  if (a.allowed && !((__ldg(a.allowed + (row >> 5)) >> (row & 31)) & 1u)) return 0ull;
+  return ((unsigned long long)(__float_as_uint(v) | 0x80000000u) << 32) |
+         (unsigned long long)(0xFFFFFFFFu - (uint32_t)__ldg(a.rank_of + row));
+}
+
+__global__ void __launch_bounds__(IB_THREADS) k_itembased(const IbArgs a) {
+  extern __shared__ __align__(16) unsigned char ib_smem[];
+  double* tnum = reinterpret_cast<double*>(ib_smem);  // [IB_TABLE]; holds the keys after the accumulation
+  double* tden = tnum + IB_TABLE;
+  int* tkey = reinterpret_cast<int*>(tden + IB_TABLE);  // item row, -1 = empty
+  int* tcnt = tkey + IB_TABLE;
+  unsigned long long* sortbuf = reinterpret_cast<unsigned long long*>(tcnt + IB_TABLE);  // [REC_MAX_N]
+  long long* bcast = reinterpret_cast<long long*>(sortbuf + REC_MAX_N);                   // [8]
+  long long* red = bcast + 8;                                                              // [32]
+  unsigned* hist = reinterpret_cast<unsigned*>(red + 32);                                  // [256]
+  int* scan_sh = reinterpret_cast<int*>(hist + 256);                                       // [32]
+  const int tid = threadIdx.x;
+  for (int s = tid; s < IB_TABLE; s += IB_THREADS) {
+    tkey[s] = -1;
+    tnum[s] = 0.0;
+    tden[s] = 0.0;
+    tcnt[s] = 0;
+  }
+  __syncthreads();
+
+  for (;;) {
+    if (tid == 0) bcast[0] = (long long)atomicAdd(&a.plan[IP_NEXT], 1ull);
+    __syncthreads();
+    const long long i = bcast[0];
+    __syncthreads();
+    if (i >= a.m) break;
+    long long* out_item = a.out_item + i * a.how_many;
+    float* out_value = a.out_value + i * a.how_many;
+    for (int t = tid; t < a.how_many; t += IB_THREADS) {
+      out_item[t] = -1;
+      out_value[t] = 0.0f;
+    }
+
+    // ---- (a) the user vector, checked before anything depends on it ----------------------------------------
+    const long long u = a.users[i];
+    long long lo = 0, hi = 0;
+    bool bad_user = u < 0 || u >= a.num_users;
+    if (!bad_user) {
+      lo = a.user_ptr[u];
+      hi = a.user_ptr[u + 1];
+      bad_user = lo < 0 || hi < lo || hi > a.nnz;
+    }
+    long long bad = 0, nz = 0;
+    if (!bad_user) {
+      for (long long t = lo + tid; t < hi; t += IB_THREADS) {
+        const int r = a.pref_row[t];
+        bad += r < 0 || r >= a.num_items || (t > lo && a.pref_row[t - 1] >= r);
+        nz += a.pref_val[t] != 0.0f;  // RandomAccessSparseVector.set(i, 0) stores nothing
+      }
+    }
+    bad = block_sum<IB_THREADS>(bad, red);
+    nz = block_sum<IB_THREADS>(nz, red);
+    if (bad_user || bad) {
+      if (tid == 0) {
+        atomicAdd(&a.plan[IP_BAD], (unsigned long long)(bad_user ? 1 : bad));
+        a.out_cnt[i] = 0;
+      }
+      continue;
+    }
+    // pruning (UserVectorSplitterMapper.maybePruneUserVector): T = the P-th largest |pref|, as float bits
+    uint32_t T = 0;
+    const bool pruned = nz > a.max_prefs;
+    if (pruned) {
+      uint32_t prefix = 0, mask = 0;
+      unsigned want = (unsigned)a.max_prefs;
+      for (int shift = 24; shift >= 0; shift -= 8) {
+        for (int t = tid; t < 256; t += IB_THREADS) hist[t] = 0u;
         __syncthreads();
-        for (int pos = tid; pos < C; pos += REC_THREADS) {
-          const unsigned long long k = keys[pos];
-          if (k && (k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+        for (long long t = lo + tid; t < hi; t += IB_THREADS) {
+          const float p = a.pref_val[t];
+          const uint32_t b = __float_as_uint(fabsf(p));
+          if (p != 0.0f && (b & mask) == prefix) atomicAdd(&hist[(b >> shift) & 255u], 1u);
         }
         __syncthreads();
         if (tid == 0) {
           unsigned acc = 0;
           for (int b = 255; b >= 0; b--) {
             if (acc + hist[b] >= want) {
-              prefix |= (unsigned long long)b << shift;
+              prefix |= (uint32_t)b << shift;
               want -= acc;
               break;
             }
@@ -449,49 +698,237 @@ __global__ void __launch_bounds__(REC_THREADS, 1) k_recommend(const RecArgs a) {
           bcast[2] = (long long)want;
         }
         __syncthreads();
-        prefix = (unsigned long long)bcast[1];
+        prefix = (uint32_t)bcast[1];
         want = (unsigned)bcast[2];
-        mask |= 255ull << shift;
+        mask |= 255u << shift;
         __syncthreads();
       }
-      thr = prefix;  // keys are distinct: exactly how_many keys are >= the how_many-th largest
+      T = prefix;
     }
-    const int n_out = nvalid < a.how_many ? nvalid : a.how_many;
-    int npad = 1;
-    while (npad < n_out) npad <<= 1;
-    for (int t = tid; t < npad; t += REC_THREADS) sortbuf[t] = 0ull;
-    if (tid == 0) bcast[3] = 0;
-    __syncthreads();
-    for (int pos = tid; pos < C; pos += REC_THREADS) {
-      const unsigned long long k = keys[pos];
-      if (k && k >= thr) sortbuf[atomicAdd(reinterpret_cast<unsigned long long*>(&bcast[3]), 1ull)] = k;
+    // considered: non-zero, and |pref| >= T (ties at T all kept; below it upstream sets the pref to NaN)
+    auto considered = [&](float p) { return p != 0.0f && __float_as_uint(fabsf(p)) >= T; };
+
+    // ---- (b) B = entries of the considered lists --------------------------------------------------------------
+    long long B = 0;
+    for (long long t = lo + tid; t < hi; t += IB_THREADS) {
+      if (!considered(a.pref_val[t])) continue;
+      const int c = a.sim_cnt[a.pref_row[t]];
+      if (c < 0 || c > a.ld) bad++;
+      else B += c;
     }
-    __syncthreads();
-    // bitonic sort, descending
-    for (int size = 2; size <= npad; size <<= 1) {
-      for (int stride = size >> 1; stride > 0; stride >>= 1) {
-        for (int t = tid; t < npad; t += REC_THREADS) {
-          const int partner = t ^ stride;
-          if (partner > t) {
-            const bool desc = (t & size) == 0;
-            const unsigned long long x = sortbuf[t], y = sortbuf[partner];
-            if (desc ? (x < y) : (x > y)) {
-              sortbuf[t] = y;
-              sortbuf[partner] = x;
-            }
+    bad = block_sum<IB_THREADS>(bad, red);
+    B = block_sum<IB_THREADS>(B, red);
+    if (bad) {
+      if (tid == 0) {
+        atomicAdd(&a.plan[IP_BAD], (unsigned long long)bad);
+        a.out_cnt[i] = 0;
+      }
+      continue;
+    }
+    const bool dense = B > IB_TABLE_MAX;
+    double *num = tnum, *den = tden;
+    int* cnt = tcnt;
+    int* touched = nullptr;
+    unsigned long long* dkeys = nullptr;
+    int slice = -1;
+    if (dense) {
+      if (tid == 0) {
+        for (int s = 0;; s = s + 1 == a.slices ? 0 : s + 1)
+          if (atomicCAS(&a.d_lock[s], 0, 1) == 0) {
+            bcast[3] = s;
+            break;
           }
+        __threadfence();
+        bcast[4] = 0;  // touched items
+      }
+      __syncthreads();
+      slice = (int)bcast[3];
+      const size_t off = (size_t)slice * a.num_items;
+      num = a.d_num + off;
+      den = a.d_den + off;
+      cnt = a.d_cnt + off;
+      touched = a.d_touched + off;
+      dkeys = a.d_key + off;
+    }
+
+    // ---- (c) partial products: one pass per considered list in ascending item row, lanes split its entries ----
+    for (long long t = lo; t < hi; t++) {
+      const float p = a.pref_val[t];
+      if (!considered(p)) continue;  // the same t on every thread: uniform
+      const long long j = a.pref_row[t];
+      const int c = a.sim_cnt[j];
+      const double pd = (double)p;
+      for (int e = tid; e < c; e += IB_THREADS) {
+        const long long it = __ldg(a.sim_idx + j * a.ld + e);
+        const double s = __ldg(a.sim_val + j * a.ld + e);
+        if (it < 0 || it >= a.num_items) {
+          bad++;
+          continue;
         }
-        __syncthreads();
+        int at;
+        double n0, d0;
+        if (dense) {
+          // the counts are updated at L2 (atomics): dense slices are read past L1
+          at = (int)it;
+          if (atomicAdd(&cnt[at], 1) == 0) touched[atomicAdd(reinterpret_cast<unsigned long long*>(&bcast[4]), 1ull)] = at;
+          n0 = __ldcg(num + at);
+          d0 = __ldcg(den + at);
+        } else {
+          at = ib_insert(tkey, (int)it);
+          cnt[at]++;
+          n0 = num[at];
+          d0 = den[at];
+        }
+        num[at] = a.boolean_data ? __dadd_rn(n0, s) : __dadd_rn(n0, __dmul_rn(s, pd));
+        den[at] = __dadd_rn(d0, fabs(s));
+      }
+      __syncthreads();
+    }
+    // known items: upstream's NaN diagonal gives every considered item a NaN prediction
+    for (long long t = lo + tid; t < hi; t += IB_THREADS) {
+      if (!considered(a.pref_val[t])) continue;
+      const int j = a.pref_row[t];
+      const int at = dense ? (__ldcg(cnt + j) ? j : -1) : ib_find(tkey, j);
+      if (at >= 0) num[at] = __longlong_as_double(0x7ff8000000000000ll);
+    }
+    __syncthreads();
+
+    // ---- (d) ranking keys, top-N ------------------------------------------------------------------------------
+    int C;
+    unsigned long long* keys;
+    long long cand = 0;
+    if (dense) {
+      C = (int)bcast[4];
+      keys = dkeys;
+      for (int t = tid; t < C; t += IB_THREADS) {
+        const int it = touched[t];
+        keys[t] = ib_key(a, it, __ldcg(num + it), __ldcg(den + it), __ldcg(cnt + it));
+      }
+      cand = C;
+    } else {
+      C = IB_TABLE;
+      keys = reinterpret_cast<unsigned long long*>(tnum);  // in place: each slot read, then written, by one thread
+      for (int s = tid; s < IB_TABLE; s += IB_THREADS) {
+        const int it = tkey[s];
+        keys[s] = it >= 0 ? ib_key(a, it, tnum[s], tden[s], tcnt[s]) : 0ull;
+        cand += it >= 0;
+      }
+      cand = block_sum<IB_THREADS>(cand, red);
+    }
+    __syncthreads();
+    const int n_out = topn_keys<IB_THREADS>(keys, C, a.how_many, hist, scan_sh, bcast, sortbuf);
+    for (int t = tid; t < n_out; t += IB_THREADS) {
+      const unsigned long long k = sortbuf[t];
+      const int row = __ldg(a.row_at + (0xFFFFFFFFu - (uint32_t)k));
+      out_item[t] = __ldg(a.item_ids + row);
+      out_value[t] = __uint_as_float((uint32_t)(k >> 32) & 0x7FFFFFFFu);
+    }
+    bad = block_sum<IB_THREADS>(bad, red);
+    if (tid == 0) {
+      a.out_cnt[i] = n_out;
+      if (bad) atomicAdd(&a.plan[IP_BAD], (unsigned long long)bad);
+      atomicAdd(&a.plan[dense ? IP_DENSE : IP_SMEM], 1ull);
+      atomicAdd(&a.plan[IP_ENTRIES], (unsigned long long)B);
+      atomicMax(&a.plan[IP_ENTRIES_MAX], (unsigned long long)B);
+      if (pruned) atomicAdd(&a.plan[IP_PRUNED], 1ull);
+      atomicMax(&a.plan[IP_CAND_MAX], (unsigned long long)cand);
+    }
+
+    // ---- reset the accumulators for the next user -------------------------------------------------------------
+    if (dense) {
+      for (int t = tid; t < C; t += IB_THREADS) {
+        const int it = touched[t];
+        num[it] = 0.0;
+        den[it] = 0.0;
+        cnt[it] = 0;
+      }
+      __syncthreads();
+      if (tid == 0) {
+        __threadfence();
+        atomicExch(&a.d_lock[slice], 0);
+      }
+    } else {
+      for (int s = tid; s < IB_TABLE; s += IB_THREADS) {
+        tkey[s] = -1;
+        tnum[s] = 0.0;
+        tden[s] = 0.0;
+        tcnt[s] = 0;
       }
     }
-    for (int t = tid; t < n_out; t += REC_THREADS) {
-      const int pos = (int)(0xFFFFFFFFu - (uint32_t)sortbuf[t]);
-      out_item[t] = __ldg(a.item_ids + cand[pos]);
-      out_value[t] = vals[pos];
-    }
-    if (tid == 0) a.out_cnt[i] = n_out;
     __syncthreads();
   }
+}
+
+// itemID rank table: (itemID, row) pairs sorted ascending by a bitonic sort; keys are itemID ^ 2^63 (signed order
+// as unsigned), padding keys ~0.  One tile of IB_SORT_TILE elements per CTA: every size up to the tile (k_fixed = 0)
+// or the strides below the tile of one size k_fixed.
+__device__ __forceinline__ void rank_cmp(unsigned long long* key, int* row, long long t, long long j, long long k) {
+  const long long p = t + j;
+  const bool asc = (t & k) == 0;
+  const unsigned long long x = key[t], y = key[p];
+  if (asc ? x > y : x < y) {
+    key[t] = y;
+    key[p] = x;
+    const int r = row[t];
+    row[t] = row[p];
+    row[p] = r;
+  }
+}
+
+__global__ void __launch_bounds__(IB_SORT_TILE / 2) k_rank_tile(unsigned long long* key, int* row, long long npad,
+                                                                 long long k_fixed) {
+  __shared__ unsigned long long sk[IB_SORT_TILE];
+  __shared__ int sr[IB_SORT_TILE];
+  const long long tile = npad < IB_SORT_TILE ? npad : IB_SORT_TILE;
+  const long long base = (long long)blockIdx.x * tile;
+  for (long long t = threadIdx.x; t < tile; t += blockDim.x) {
+    sk[t] = key[base + t];
+    sr[t] = row[base + t];
+  }
+  __syncthreads();
+  const long long k0 = k_fixed ? k_fixed : 2, k1 = k_fixed ? k_fixed : tile;
+  for (long long k = k0; k <= k1; k <<= 1) {
+    for (long long j = (k >> 1) < tile ? (k >> 1) : (tile >> 1); j > 0; j >>= 1) {
+      for (long long c = threadIdx.x; c < tile / 2; c += blockDim.x) {
+        const long long t = (c / j) * 2 * j + (c % j);
+        // direction from the global position
+        const long long p = t + j;
+        const bool asc = ((base + t) & k) == 0;
+        const unsigned long long x = sk[t], y = sk[p];
+        if (asc ? x > y : x < y) {
+          sk[t] = y;
+          sk[p] = x;
+          const int r = sr[t];
+          sr[t] = sr[p];
+          sr[p] = r;
+        }
+      }
+      __syncthreads();
+    }
+  }
+  for (long long t = threadIdx.x; t < tile; t += blockDim.x) {
+    key[base + t] = sk[t];
+    row[base + t] = sr[t];
+  }
+}
+
+__global__ void k_rank_global(unsigned long long* key, int* row, long long npad, long long j, long long k) {
+  const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= npad / 2) return;
+  rank_cmp(key, row, (c / j) * 2 * j + (c % j), j, k);
+}
+
+__global__ void k_rank_init(const long long* __restrict__ item_ids, long long n, long long npad,
+                            unsigned long long* key, int* row) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= npad) return;
+  key[t] = t < n ? ((unsigned long long)item_ids[t] ^ 0x8000000000000000ull) : ~0ull;
+  row[t] = t < n ? (int)t : -1;
+}
+
+__global__ void k_rank_scatter(const int* __restrict__ row_at, long long n, int* rank_of) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n) rank_of[row_at[t]] = (int)t;
 }
 
 }  // namespace
@@ -733,6 +1170,159 @@ int mb200_recommend_last_plan(mb200_ctx* ctx, mb200_recommend_plan* out) {
   if (!ctx || !out) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_last_plan: NULL argument");
   std::lock_guard<std::mutex> g(ctx->mu);
   *out = ctx->last_recommend_plan;
+  return MB200_OK;
+}
+
+int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args) {
+  if (!ctx || !args) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_item_based: NULL argument");
+  std::lock_guard<std::mutex> g(ctx->mu);
+  const mb200_itembased_args& x = *args;
+  if (x.how_many < 1 || x.how_many > REC_MAX_N)
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_item_based: how_many must be in [1, %d] (got %d)",
+                      REC_MAX_N, x.how_many);
+  if (x.max_prefs_per_user < 1)
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_item_based: max_prefs_per_user must be >= 1 (got %d)",
+                      x.max_prefs_per_user);
+  if (x.m < 0 || x.sim_ld < 1 || x.num_items < 0 || x.num_items >= (1LL << 31) || x.num_users < 0 || x.nnz < 0 ||
+      (x.mem != MB200_MEM_HOST && x.mem != MB200_MEM_DEVICE))
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG,
+                      "mb200_recommend_item_based: bad shape (m=%lld sim_ld=%d num_items=%lld num_users=%lld nnz=%lld)",
+                      (long long)x.m, x.sim_ld, (long long)x.num_items, (long long)x.num_users, (long long)x.nnz);
+  if (x.m == 0) return MB200_OK;
+  if (!x.user_ptr || !x.users || !x.out_item || !x.out_value || !x.out_cnt ||
+      (x.num_items > 0 && (!x.sim_idx || !x.sim_val || !x.sim_cnt || !x.item_ids)) ||
+      (x.nnz > 0 && (!x.pref_row || !x.pref_val)))
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_item_based: NULL array argument");
+  MB_CUDA(ctx, cudaSetDevice(ctx->device));
+  const long long n = x.num_items;
+  const long long words = (n + 31) / 32;
+
+  Staged st(ctx, x.mem);
+  IbArgs a;
+  a.num_items = n;
+  a.ld = x.sim_ld;
+  a.num_users = x.num_users;
+  a.nnz = x.nnz;
+  a.m = x.m;
+  a.how_many = x.how_many;
+  a.max_prefs = x.max_prefs_per_user;
+  a.boolean_data = x.boolean_data != 0;
+  const size_t lists = (size_t)n * x.sim_ld;
+  MB_CHECK(st.in((const long long*)x.sim_idx, lists, &a.sim_idx));
+  MB_CHECK(st.in(x.sim_val, lists, &a.sim_val));
+  MB_CHECK(st.in((const int*)x.sim_cnt, (size_t)n, &a.sim_cnt));
+  MB_CHECK(st.in((const long long*)x.user_ptr, (size_t)x.num_users + 1, &a.user_ptr));
+  MB_CHECK(st.in((const int*)x.pref_row, (size_t)x.nnz, &a.pref_row));
+  MB_CHECK(st.in(x.pref_val, (size_t)x.nnz, &a.pref_val));
+  MB_CHECK(st.in((const long long*)x.item_ids, (size_t)n, &a.item_ids));
+  MB_CHECK(st.in((const unsigned*)x.allowed, x.allowed ? (size_t)words : 0, &a.allowed));
+  MB_CHECK(st.in((const long long*)x.users, (size_t)x.m, &a.users));
+  MB_CHECK(st.out((long long*)x.out_item, (size_t)x.m * x.how_many, &a.out_item));
+  MB_CHECK(st.out(x.out_value, (size_t)x.m * x.how_many, &a.out_value));
+  MB_CHECK(st.out((int*)x.out_cnt, (size_t)x.m, &a.out_cnt));
+
+  // the itemID rank table: (itemID, row) sorted on the device, rank -> row and row -> rank
+  long long npad = 1;
+  while (npad < n) npad <<= 1;
+  void *wk = nullptr, *wr = nullptr, *wo = nullptr, *wp = nullptr;
+  MB_CHECK(mb200_group_ws(ctx, 60, (size_t)npad * 8, &wk));
+  MB_CHECK(mb200_group_ws(ctx, 61, (size_t)npad * 4, &wr));
+  MB_CHECK(mb200_group_ws(ctx, 63, (size_t)(n > 0 ? n : 1) * 4, &wo));
+  MB_CHECK(mb200_group_ws(ctx, 64, IP_WORDS * sizeof(unsigned long long), &wp));
+  a.row_at = (const int*)wr;
+  a.rank_of = (const int*)wo;
+  a.plan = (unsigned long long*)wp;
+  MB_CUDA(ctx, cudaMemsetAsync(wp, 0, IP_WORDS * sizeof(unsigned long long), ctx->stream));
+  if (n > 0) {
+    ProfScope prof(ctx, MB200_K_RECOMMEND);
+    unsigned long long* key = (unsigned long long*)wk;
+    int* row = (int*)wr;
+    k_rank_init<<<(unsigned)ceil_div64(npad, 256), 256, 0, ctx->stream>>>(a.item_ids, n, npad, key, row);
+    const long long tile = npad < IB_SORT_TILE ? npad : IB_SORT_TILE;
+    k_rank_tile<<<(unsigned)(npad / tile), IB_SORT_TILE / 2, 0, ctx->stream>>>(key, row, npad, 0);
+    ctx->launches += 2;
+    for (long long k = 2 * IB_SORT_TILE; k <= npad; k <<= 1) {
+      for (long long j = k >> 1; j >= IB_SORT_TILE; j >>= 1) {
+        k_rank_global<<<(unsigned)ceil_div64(npad / 2, 256), 256, 0, ctx->stream>>>(key, row, npad, j, k);
+        ctx->launches++;
+      }
+      k_rank_tile<<<(unsigned)(npad / IB_SORT_TILE), IB_SORT_TILE / 2, 0, ctx->stream>>>(key, row, npad, k);
+      ctx->launches++;
+    }
+    k_rank_scatter<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(row, n, (int*)wo);
+    ctx->launches++;
+    MB_CUDA(ctx, cudaGetLastError());
+  }
+
+  // persistent CTAs, as many as fit; dense slices for as many of them as 4 GiB allow
+  MB_CUDA(ctx, cudaFuncSetAttribute(k_itembased, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)IB_SMEM));
+  int per_sm = 0;
+  MB_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_itembased, IB_THREADS, IB_SMEM));
+  per_sm = per_sm < 1 ? 1 : per_sm;
+  const long long grid = x.m < (long long)ctx->num_sms * per_sm ? x.m : (long long)ctx->num_sms * per_sm;
+  const size_t slice_bytes = (size_t)(n > 0 ? n : 1) * (8 + 8 + 4 + 4 + 8);
+  long long slices = (long long)(IB_DENSE_MAX_BYTES / slice_bytes);
+  slices = slices < 1 ? 1 : (slices > grid ? grid : slices);
+  // slot 62 holds the slices; num / den / cnt are kept zero by the kernel, so they are cleared only when the slot or
+  // its layout changes
+  const size_t dense_bytes = (size_t)slices * slice_bytes;
+  const size_t had = ctx->ws_group.size() > 62 ? ctx->ws_group[62].second : 0;
+  void *wd = nullptr, *wl = nullptr;
+  MB_CHECK(mb200_group_ws(ctx, 62, dense_bytes, &wd));
+  if (ctx->ws_group[62].second != had || ctx->itembased_dense_items != n || ctx->itembased_dense_slices != slices) {
+    MB_CUDA(ctx, cudaMemsetAsync(wd, 0, dense_bytes, ctx->stream));
+    ctx->itembased_dense_items = n;
+    ctx->itembased_dense_slices = slices;
+  }
+  MB_CHECK(mb200_group_ws(ctx, 65, (size_t)slices * 4, &wl));
+  MB_CUDA(ctx, cudaMemsetAsync(wl, 0, (size_t)slices * 4, ctx->stream));
+  const size_t per = (size_t)slices * (n > 0 ? n : 1);
+  a.d_num = (double*)wd;
+  a.d_den = a.d_num + per;
+  a.d_key = (unsigned long long*)(a.d_den + per);
+  a.d_cnt = (int*)(a.d_key + per);
+  a.d_touched = a.d_cnt + per;
+  a.d_lock = (int*)wl;
+  a.slices = (int)slices;
+  {
+    ProfScope prof(ctx, MB200_K_RECOMMEND);
+    k_itembased<<<(unsigned)grid, IB_THREADS, IB_SMEM, ctx->stream>>>(a);
+  }
+  ctx->launches++;
+  MB_CUDA(ctx, cudaGetLastError());
+  MB_CHECK(st.finish());
+  unsigned long long h[IP_WORDS];
+  MB_CUDA(ctx, cudaMemcpyAsync(h, a.plan, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  mb200_itembased_plan& pl = ctx->last_itembased_plan;
+  pl.users = x.m;
+  pl.smem_users = (int64_t)h[IP_SMEM];
+  pl.dense_users = (int64_t)h[IP_DENSE];
+  pl.entries = (int64_t)h[IP_ENTRIES];
+  pl.entries_max = (int64_t)h[IP_ENTRIES_MAX];
+  pl.pruned_users = (int64_t)h[IP_PRUNED];
+  pl.candidates_max = (int64_t)h[IP_CAND_MAX];
+  pl.table_slots = IB_TABLE;
+  pl.dense_slices = (int32_t)slices;
+  if (getenv("MB200_TRACE"))
+    fprintf(stderr,
+            "[mb200 trace] itembased plan: users=%lld smem=%lld dense=%lld entries=%lld entries_max=%lld pruned=%lld "
+            "candidates_max=%lld table=%d slices=%lld grid=%lld\n",
+            (long long)pl.users, (long long)pl.smem_users, (long long)pl.dense_users, (long long)pl.entries,
+            (long long)pl.entries_max, (long long)pl.pruned_users, (long long)pl.candidates_max, IB_TABLE, slices, grid);
+  if (h[IP_BAD])
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG,
+                      "mb200_recommend_item_based: %llu user row(s), user_ptr range(s), pref_row entr(ies) (out of range "
+                      "or not ascending), list count(s) or list entr(ies) out of range (num_users %lld, num_items %lld, "
+                      "nnz %lld, sim_ld %d)",
+                      h[IP_BAD], (long long)x.num_users, (long long)n, (long long)x.nnz, x.sim_ld);
+  return MB200_OK;
+}
+
+int mb200_itembased_last_plan(mb200_ctx* ctx, mb200_itembased_plan* out) {
+  if (!ctx || !out) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_itembased_last_plan: NULL argument");
+  std::lock_guard<std::mutex> g(ctx->mu);
+  *out = ctx->last_itembased_plan;
   return MB200_OK;
 }
 

@@ -46,7 +46,27 @@ def java_double_to_string(v: float) -> str:
     if v == 0.0:
         return "-0.0" if math.copysign(1.0, v) < 0 else "0.0"
     sign, digits, exp = decimal.Decimal(repr(float(v))).as_tuple()
-    digits = "".join(map(str, digits))
+    return _java_notation(sign, "".join(map(str, digits)), exp)
+
+
+def java_float_to_string(v: float) -> str:
+    """Float.toString: the shortest digits that round-trip through float32, with Double.toString's notation rules
+    (`0.70710677`, `1.0E-4`, `9999999.0`, `1.0E7`); what RecommenderJob's text output writes for a value."""
+    import math
+    v = float(np.float32(v))
+    if math.isnan(v) or math.isinf(v) or v == 0.0:
+        return java_double_to_string(v)
+    mant, e = np.format_float_scientific(np.float32(v), unique=True, trim="-").split("e")
+    if len(mant.lstrip("-")) == 1 and abs(v) < 1.1754943508222875e-38:
+        # a subnormal whose shortest form has one digit: Java prints d.d, the closest two digits (1.4E-45)
+        mant, e = np.format_float_scientific(np.float32(v), precision=1, unique=False).split("e")
+    sign = mant.startswith("-")
+    digits = mant.lstrip("-").replace(".", "")
+    return _java_notation(sign, digits, int(e) - len(digits) + 1)
+
+
+def _java_notation(sign, digits: str, exp: int) -> str:
+    """digits x 10^exp in Java's notation: decimal for 1e-3 <= |v| < 1e7, else computerised scientific"""
     stripped = digits.rstrip("0") or "0"
     exp += len(digits) - len(stripped)
     digits = stripped
@@ -82,27 +102,31 @@ def most_similar_item_pairs(idx, sim, cnt, item_id=None):
 # ------------------------------------------------------------------------------------------------
 def item_similarity(row, user, pref, num_items: int, k: int = DEFAULT_MAX_SIMILAR_ITEMS_PER_ITEM,
                     threshold: float | None = None, width: int = 4096, depth: int = 4, seed: int = 42,
-                    frac_bits: int = 1, dtype: str = "f16", precision: str = "rescored", ctx=None):
+                    frac_bits: int = 1, dtype: str = "f16", precision: str = "rescored", ctx=None,
+                    device: bool = False):
     """Sketch build + all-pairs cosine + per-item top-k on one GPU.
-    entity = item row, key = userID, increment = pref (SURVEY.md 8a5, item-similarity mode)."""
+    entity = item row, key = userID, increment = pref (SURVEY.md 8a5, item-similarity mode).
+    device=True returns the lists as torch CUDA tensors (they stay in HBM for the item-based recommender)."""
     ctx = ctx or sk.default_context()
     bank = sk.SketchBank(num_items, width, depth, seed, frac_bits, ctx)
     try:
         bank.update(row, user, pref)
         bank.check()
-        return bank.cosine_topk(k, threshold, True, dtype, precision)
+        return bank.cosine_topk(k, threshold, True, dtype, precision, device=device)
     finally:
         bank.close()
 
 
 def exact_item_similarity(row, user, pref, num_items: int, k: int = DEFAULT_MAX_SIMILAR_ITEMS_PER_ITEM,
                           threshold: float | None = None, frac_bits: int = 1, dtype: str = "f16",
-                          precision: str = "rescored", ctx=None, ucol=None, num_users: int | None = None):
+                          precision: str = "rescored", ctx=None, ucol=None, num_users: int | None = None,
+                          device: bool = False):
     """RowSimilarityJob with CosineSimilarity, exactly (RowSimilarityJob.java:478-559; no sketch, no
     --maxPrefs down-sampling): the users are renumbered 0..U-1 and every user owns one counter column
     (depth 1, width U, identity hash), so K1 writes the item x user matrix, K3 computes all pairs on the
     tensor cores and K5 re-scores the kept candidates in exact integer / FP64 arithmetic.
-    The events must be de-duplicated (one pref per (user, item): `Events.prepare`)."""
+    The events must be de-duplicated (one pref per (user, item): `Events.prepare`).  device=True: as in
+    item_similarity."""
     import torch
     ctx = ctx or sk.default_context()
     dev = f"cuda:{ctx.device}"
@@ -115,7 +139,7 @@ def exact_item_similarity(row, user, pref, num_items: int, k: int = DEFAULT_MAX_
     try:
         bank.update(torch.as_tensor(row).to(dev), col, torch.as_tensor(pref).to(dev))
         bank.check()
-        return bank.cosine_topk(k, threshold, True, dtype, precision)
+        return bank.cosine_topk(k, threshold, True, dtype, precision, device=device)
     finally:
         bank.close()
 
