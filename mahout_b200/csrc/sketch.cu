@@ -20,19 +20,27 @@ struct Quad {
   T inc[4];
 };
 
-template <typename T, bool HAS_ENTITY, bool VEC, typename K>
+// vector load of the event columns; STREAM marks the lines evict-first (ld.global.cs), so that a stream of
+// events does not push an L2-resident working set out
+template <bool STREAM, typename V>
+__device__ __forceinline__ V ld_ev(const V* ptr) {
+  if constexpr (STREAM) return __ldcs(ptr);
+  else return __ldg(ptr);
+}
+
+template <typename T, bool HAS_ENTITY, bool VEC, typename K, bool STREAM = false>
 __device__ __forceinline__ void load_quad(const UpdateArgs<T, K>& p, long long base, Quad<T>& q) {
   if constexpr (sizeof(K) == 4) {
     // narrow wire format: four u32 keys in one 16-byte load, four u8 quanta in one 4-byte load
     if (VEC) {
-      const uint4 k = __ldg(reinterpret_cast<const uint4*>(p.key + base));
+      const uint4 k = ld_ev<STREAM>(reinterpret_cast<const uint4*>(p.key + base));
       q.key[0] = k.x; q.key[1] = k.y; q.key[2] = k.z; q.key[3] = k.w;
       if (HAS_ENTITY) {
         const uint4 e = __ldg(reinterpret_cast<const uint4*>(p.entity + base));
         q.ent[0] = e.x; q.ent[1] = e.y; q.ent[2] = e.z; q.ent[3] = e.w;
       }
       if constexpr (sizeof(T) == 1) {
-        const uchar4 c = __ldg(reinterpret_cast<const uchar4*>(p.inc + base));
+        const uchar4 c = ld_ev<STREAM>(reinterpret_cast<const uchar4*>(p.inc + base));
         q.inc[0] = c.x; q.inc[1] = c.y; q.inc[2] = c.z; q.inc[3] = c.w;
       } else {
 #pragma unroll
@@ -48,7 +56,7 @@ __device__ __forceinline__ void load_quad(const UpdateArgs<T, K>& p, long long b
     }
   } else if (VEC) {
     const longlong2* k2 = reinterpret_cast<const longlong2*>(p.key + base);
-    longlong2 k01 = __ldg(k2), k23 = __ldg(k2 + 1);
+    longlong2 k01 = ld_ev<STREAM>(k2), k23 = ld_ev<STREAM>(k2 + 1);
     q.key[0] = k01.x; q.key[1] = k01.y; q.key[2] = k23.x; q.key[3] = k23.y;
     if (HAS_ENTITY) {
       const longlong2* e2 = reinterpret_cast<const longlong2*>(p.entity + base);
@@ -56,11 +64,11 @@ __device__ __forceinline__ void load_quad(const UpdateArgs<T, K>& p, long long b
       q.ent[0] = e01.x; q.ent[1] = e01.y; q.ent[2] = e23.x; q.ent[3] = e23.y;
     }
     if constexpr (sizeof(T) == 4) {
-      float4 v = __ldg(reinterpret_cast<const float4*>(p.inc + base));
+      float4 v = ld_ev<STREAM>(reinterpret_cast<const float4*>(p.inc + base));
       q.inc[0] = (T)v.x; q.inc[1] = (T)v.y; q.inc[2] = (T)v.z; q.inc[3] = (T)v.w;
     } else if constexpr (sizeof(T) == 8) {
       const double2* d2 = reinterpret_cast<const double2*>(p.inc + base);
-      double2 a = __ldg(d2), b = __ldg(d2 + 1);
+      double2 a = ld_ev<STREAM>(d2), b = ld_ev<STREAM>(d2 + 1);
       q.inc[0] = (T)a.x; q.inc[1] = (T)a.y; q.inc[2] = (T)b.x; q.inc[3] = (T)b.y;
     } else {
 #pragma unroll
@@ -293,8 +301,41 @@ __device__ __forceinline__ long long quanta_of(unsigned char v, double qscale, f
   return inc_to_quanta(v, qscale, bad, maxabs);
 }
 
-template <typename T, bool VEC, int D, typename K, bool AGG>
-__global__ void __launch_bounds__(V2_THREADS, 1) k_update_single_v2(const UpdateArgs<T, K> p) {
+// Key table (large calls).  The keys the cache does not hold are the Zipf tail: unique inside any window a CTA sees,
+// so nothing on the chip can merge them, but they do repeat over a call of 10^8+ events.  With KT a queued miss whose
+// key is in [0, KT_ROWS) is drained with ONE reduction into ktab[key] (its per-call total, int64 quanta) instead of d
+// hashes and d reductions; k_keytab_flush then scatters every nonzero total once and zeroes it.  The decision is taken
+// at drain time, with every lane busy, so the per-event loop is the direct path's (measured: 4.53 ms per 10^9 Zipf 1.1
+// events against 4.90 with a predicated reduction in the lane that met the miss).  Integer adds commute: the
+// counters are the direct path's bit for bit, and an entry is a partial sum of the counters it ends up in, so the
+// exactness bound is untouched.  The table's lines are reduced with an L2 evict_last policy and the events are
+// loaded evict-first, so that the touched part of the table stays in L2 while the event stream passes.
+static constexpr int KT_LOG2 = 24;
+static constexpr long long KT_ROWS = 1LL << KT_LOG2;  // 128 MiB of int64 totals
+// trace counters (MB200_TRACE): misses into the table, events scattered directly, cache slots flushed, table keys
+// flushed
+enum { KS_TABLE = 0, KS_DIRECT = 1, KS_CACHE = 2, KS_FLUSHED = 3, KS_WORDS = 4 };
+
+__device__ __forceinline__ unsigned long long l2_evict_last_policy() {
+  unsigned long long pol;
+  asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+  return pol;
+}
+
+__device__ __forceinline__ void red_add_hinted(long long* addr, long long v, unsigned long long pol) {
+  asm volatile("red.global.add.L2::cache_hint.u64 [%0], %1, %2;" ::"l"(addr), "l"(v), "l"(pol) : "memory");
+}
+
+// one count per lane, one atomic per warp (whole warps only)
+__device__ __forceinline__ void publish_count(unsigned long long* stats, int word, unsigned v) {
+  v = __reduce_add_sync(0xffffffffu, v);
+  if ((threadIdx.x & 31) == 0 && v) atomicAdd(&stats[word], (unsigned long long)v);
+}
+
+// COUNT: keep the trace counters (MB200_TRACE only: the counting costs issue slots)
+template <typename T, bool VEC, int D, typename K, bool AGG, bool KT, bool COUNT>
+__global__ void __launch_bounds__(V2_THREADS, 1)
+    k_update_single_v2(const UpdateArgs<T, K> p, long long* __restrict__ ktab, unsigned long long* __restrict__ stats) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   CacheV2 c;
   c.tags = reinterpret_cast<uint2*>(smem_raw);
@@ -312,6 +353,9 @@ __global__ void __launch_bounds__(V2_THREADS, 1) k_update_single_v2(const Update
   int qn = 0;
   unsigned int bad = 0;
   unsigned long long maxabs = 0;
+  unsigned n_table = 0, n_direct = 0;  // this lane's table reductions / direct scatters (trace counters)
+  unsigned long long pol = 0;
+  if (KT) pol = l2_evict_last_policy();
   const float qscale_f = (float)p.qscale;
   const long long n4 = p.n & ~3LL;
   const long long stride = (long long)gridDim.x * blockDim.x * 4;
@@ -320,7 +364,7 @@ __global__ void __launch_bounds__(V2_THREADS, 1) k_update_single_v2(const Update
     const long long base = wbase + (long long)lane * 4;
     const bool live = base < n4;
     Quad<T> ev;
-    if (live) load_quad<T, false, VEC, K>(p, base, ev);
+    if (live) load_quad<T, false, VEC, K, KT>(p, base, ev);
 #pragma unroll
     for (int j = 0; j < 4; j++) {
       long long q = 0;
@@ -354,25 +398,79 @@ __global__ void __launch_bounds__(V2_THREADS, 1) k_update_single_v2(const Update
       __syncwarp();
       if (qn >= 32) {
         qn -= 32;
-        scatter_event<D>(p.counters, p.hf, mq_key[qn + lane], mq_val[qn + lane]);
+        {
+          const long long k = mq_key[qn + lane], v = mq_val[qn + lane];
+          if (KT && (unsigned long long)k < (unsigned long long)KT_ROWS) {
+            red_add_hinted(ktab + k, v, pol);
+            if (COUNT) n_table++;
+          } else {
+            scatter_event<D>(p.counters, p.hf, k, v);
+            if (COUNT) n_direct++;
+          }
+        }
         __syncwarp();
       }
     }
   }
-  if (lane < qn) scatter_event<D>(p.counters, p.hf, mq_key[lane], mq_val[lane]);
+  if (lane < qn) {
+    const long long k = mq_key[lane], v = mq_val[lane];
+    if (KT && (unsigned long long)k < (unsigned long long)KT_ROWS) {
+      red_add_hinted(ktab + k, v, pol);
+      if (COUNT) n_table++;
+    } else {
+      scatter_event<D>(p.counters, p.hf, k, v);
+      if (COUNT) n_direct++;
+    }
+  }
   if (blockIdx.x == 0 && threadIdx.x < (unsigned)(p.n - n4)) {
     long long t = n4 + threadIdx.x;
     long long q = inc_to_quanta(p.inc[t], p.qscale, bad, maxabs);
-    if (q != 0) scatter_event<D>(p.counters, p.hf, (long long)p.key[t], q);
+    if (q != 0) {
+      scatter_event<D>(p.counters, p.hf, (long long)p.key[t], q);
+      if (COUNT) n_direct++;
+    }
   }
   __syncthreads();
+  unsigned n_cache = 0;
   for (int s = threadIdx.x; s < 2 * V2_SETS; s += blockDim.x) {
     const unsigned t = reinterpret_cast<const unsigned*>(c.tags)[s];
     if (t == V2_EMPTY) continue;
     const long long sum = (long long)(((unsigned long long)(unsigned int)c.hi[s] << 32) | c.lo[s]);
-    if (sum != 0) scatter_event<D>(p.counters, p.hf, (long long)t, sum);
+    if (sum != 0) {
+      scatter_event<D>(p.counters, p.hf, (long long)t, sum);
+      if (COUNT) n_cache++;
+    }
   }
   publish_flags(p.flags, bad, 0u, maxabs);
+  if (COUNT) {
+    publish_count(stats, KS_TABLE, n_table);
+    publish_count(stats, KS_DIRECT, n_direct);
+    publish_count(stats, KS_CACHE, n_cache);
+  }
+}
+
+// the key table's second half: every nonzero total -> d reductions, and the entry back to 0 (untouched entries are
+// only read).  One pass: each thread owns KT_FLUSH_PER entries, loaded up front (two 16-byte loads in flight per
+// thread, the whole table in flight across the grid -- a grid-stride loop left the scan latency-bound).
+static constexpr int KT_FLUSH_THREADS = 256, KT_FLUSH_PER = 4;
+
+template <int D>
+__global__ void __launch_bounds__(KT_FLUSH_THREADS) k_keytab_flush(long long* __restrict__ ktab, long long* __restrict__ counters,
+                                                                   const HashFamily hf, unsigned long long* __restrict__ stats) {
+  unsigned n_keys = 0;
+  const long long i0 = ((long long)blockIdx.x * KT_FLUSH_THREADS + threadIdx.x) * KT_FLUSH_PER;
+  const longlong2 a = __ldcs(reinterpret_cast<const longlong2*>(ktab + i0));
+  const longlong2 b = __ldcs(reinterpret_cast<const longlong2*>(ktab + i0 + 2));
+  const long long v[KT_FLUSH_PER] = {a.x, a.y, b.x, b.y};
+#pragma unroll
+  for (int j = 0; j < KT_FLUSH_PER; j++) {
+    if (v[j] != 0) {
+      ktab[i0 + j] = 0;
+      scatter_event<D>(counters, hf, i0 + j, v[j]);
+      n_keys++;
+    }
+  }
+  if (stats) publish_count(stats, KS_FLUSHED, n_keys);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -533,6 +631,28 @@ __global__ void __launch_bounds__(256) k_widen_events(const uint32_t* __restrict
   }
 }
 
+// Single-sketch calls of at least this many events take the key table (k_update_single_v2<KT> + k_keytab_flush).
+// The flush costs a scan of the table plus d reductions per distinct key, so the table pays off on large calls only;
+// the host-memory path stages 2^23-event chunks, which stay on the direct path.  DESIGN.md §3 has the crossover.
+static constexpr int64_t KT_MIN_EVENTS = 1LL << 26;
+static constexpr size_t KT_SLOT = 20, KT_STATS_SLOT = 21;  // ws_group slots
+
+static int64_t keytab_min_events() {
+  if (const char* ev = getenv("MB200_K1_KEYTABLE_MIN_EVENTS"))  // tuning / test override: 0 = always, huge = never
+    return strtoll(ev, nullptr, 10);
+  return KT_MIN_EVENTS;
+}
+
+// the table is zeroed when it is allocated and every call leaves it zeroed (k_keytab_flush)
+static int keytab(mb200_ctx* ctx, long long** out) {
+  const size_t had = ctx->ws_group.size() > KT_SLOT ? ctx->ws_group[KT_SLOT].second : 0;
+  void* p = nullptr;
+  MB_CHECK(mb200_group_ws(ctx, KT_SLOT, (size_t)KT_ROWS * sizeof(long long), &p));
+  if (ctx->ws_group[KT_SLOT].second != had) MB_CUDA(ctx, cudaMemsetAsync(p, 0, (size_t)KT_ROWS * sizeof(long long), ctx->stream));
+  *out = (long long*)p;
+  return MB200_OK;
+}
+
 template <typename T, typename K = long long>
 static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T* inc, int64_t n) {
   mb200_ctx* ctx = bk->ctx;
@@ -573,29 +693,71 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
   }
   ProfScope prof(ctx, MB200_K_UPDATE);
   if (bk->E == 1 && ctx->single_kernel != 0) {
-    // single-sketch mode, second form: one 1024-thread CTA per SM, 2-way cache, optional warp aggregation
+    // single-sketch mode, second form: one 1024-thread CTA per SM, 2-way cache, optional warp aggregation; the
+    // default form (1) sends the cache's misses of a large call through the key table
     const size_t smem = (size_t)V2_SETS * 24 + (size_t)(V2_THREADS / 32) * 2 * MISS_Q * sizeof(long long);
     long long want = ceil_div64(n, (int64_t)V2_THREADS * 4);
     int grid = (int)(want < (long long)ctx->num_sms ? want : (long long)ctx->num_sms);
-#define LAUNCH_V2(VEC, D, AGG)                                                                               \
-  do {                                                                                                       \
-    MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single_v2<T, VEC, D, K, AGG>,                                 \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));              \
-    k_update_single_v2<T, VEC, D, K, AGG><<<grid, V2_THREADS, smem, ctx->stream>>>(p);                       \
-  } while (0)
     const bool agg = ctx->single_kernel == 2;
+    const bool table = !agg && n >= keytab_min_events();
+    const bool trace = getenv("MB200_TRACE") != nullptr;
+    long long* ktab = nullptr;
+    unsigned long long* stats = nullptr;
+    if (table) MB_CHECK(keytab(ctx, &ktab));
+    if (trace) {
+      void* s = nullptr;
+      MB_CHECK(mb200_group_ws(ctx, KT_STATS_SLOT, KS_WORDS * sizeof(unsigned long long), &s));
+      MB_CUDA(ctx, cudaMemsetAsync(s, 0, KS_WORDS * sizeof(unsigned long long), ctx->stream));
+      stats = (unsigned long long*)s;
+    }
+#define LAUNCH_V2_C(VEC, D, AGG, KT, COUNT)                                                                  \
+  do {                                                                                                       \
+    MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single_v2<T, VEC, D, K, AGG, KT, COUNT>,                      \
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));              \
+    k_update_single_v2<T, VEC, D, K, AGG, KT, COUNT><<<grid, V2_THREADS, smem, ctx->stream>>>(p, ktab, stats); \
+  } while (0)
+#define LAUNCH_V2(VEC, D, AGG, KT)                \
+  do {                                            \
+    if (trace) LAUNCH_V2_C(VEC, D, AGG, KT, true); \
+    else LAUNCH_V2_C(VEC, D, AGG, KT, false);      \
+  } while (0)
     if (d4) {
-      if (vec && agg) LAUNCH_V2(true, 4, true);
-      else if (vec) LAUNCH_V2(true, 4, false);
-      else if (agg) LAUNCH_V2(false, 4, true);
-      else LAUNCH_V2(false, 4, false);
+      if (table && vec) LAUNCH_V2(true, 4, false, true);
+      else if (table) LAUNCH_V2(false, 4, false, true);
+      else if (vec && agg) LAUNCH_V2(true, 4, true, false);
+      else if (vec) LAUNCH_V2(true, 4, false, false);
+      else if (agg) LAUNCH_V2(false, 4, true, false);
+      else LAUNCH_V2(false, 4, false, false);
     } else {
-      if (vec && agg) LAUNCH_V2(true, 0, true);
-      else if (vec) LAUNCH_V2(true, 0, false);
-      else if (agg) LAUNCH_V2(false, 0, true);
-      else LAUNCH_V2(false, 0, false);
+      if (table && vec) LAUNCH_V2(true, 0, false, true);
+      else if (table) LAUNCH_V2(false, 0, false, true);
+      else if (vec && agg) LAUNCH_V2(true, 0, true, false);
+      else if (vec) LAUNCH_V2(true, 0, false, false);
+      else if (agg) LAUNCH_V2(false, 0, true, false);
+      else LAUNCH_V2(false, 0, false, false);
     }
 #undef LAUNCH_V2
+#undef LAUNCH_V2_C
+    if (table) {
+      ctx->launches++;
+      MB_CUDA(ctx, cudaGetLastError());
+      const unsigned fgrid = (unsigned)(KT_ROWS / (KT_FLUSH_THREADS * KT_FLUSH_PER));
+      if (d4) k_keytab_flush<4><<<fgrid, KT_FLUSH_THREADS, 0, ctx->stream>>>(ktab, p.counters, p.hf, stats);
+      else k_keytab_flush<0><<<fgrid, KT_FLUSH_THREADS, 0, ctx->stream>>>(ktab, p.counters, p.hf, stats);
+    }
+    if (trace) {
+      MB_CUDA(ctx, cudaGetLastError());
+      unsigned long long h[KS_WORDS];
+      MB_CUDA(ctx, cudaMemcpyAsync(h, stats, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+      MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      // L2 reductions of the call: one per table miss, d per direct event, cached key and flushed table key
+      const double reds = (double)h[KS_TABLE] + (double)bk->d * (double)(h[KS_DIRECT] + h[KS_CACHE] + h[KS_FLUSHED]);
+      fprintf(stderr,
+              "[mb200 trace] k1: path=%s n=%lld misses_table=%llu misses_direct=%llu cache_keys=%llu flushed_keys=%llu "
+              "reds_per_event=%.4f\n",
+              table ? "table" : "direct", (long long)n, h[KS_TABLE], h[KS_DIRECT], h[KS_CACHE], h[KS_FLUSHED],
+              reds / (double)n);
+    }
   } else if (bk->E == 1) {
     // single-sketch mode: the entity column (if any) is not needed
     const int threads = 512;
