@@ -252,6 +252,50 @@ typedef struct mb200_recommend_plan {
 } mb200_recommend_plan;
 int mb200_recommend_last_plan(mb200_ctx* ctx, mb200_recommend_plan* out);
 
+/* ---- CosineCM with a CountMinSketchConfig: every user's sketch at its own (width, depth) ---------------------- */
+/* The sized bank holds user u's sketch at (width[u], depth[u]) -- mb200_cm_dims(getDelta(u), getEpsilon(u)), as
+ * `new DoubleCountMinSketch(delta, epsilon, hfb)` sizes it -- all users sharing one hash family a[], b[] (HOST arrays of
+ * at least max(depth) entries).  The data model is CSR by user row: the prefs of row u are [user_ptr[u], user_ptr[u+1]),
+ * user_ptr[0] = 0; every (item, pref) given is added (CosineCM.exportProfile).  Counters are int64 fixed point with
+ * quantum 2^-frac_bits; MB200_ERR_INEXACT / _RANGE as for banks (a sketch row whose sum of squared quanta reaches
+ * 2^53 is out of range too).  depth in [1, 32], width >= 1; malformed widths, depths or user_ptr fail with
+ * MB200_ERR_BAD_ARG.  The bank keeps the prefs on the device: queries re-sketch users from them.  width, depth, user_ptr,
+ * item and pref are in `mem`. */
+typedef struct mb200_sized_bank mb200_sized_bank;
+int mb200_sized_bank_create(mb200_ctx* ctx, int64_t users, const int32_t* width, const int32_t* depth, const int64_t* a,
+                            const int64_t* b, int32_t frac_bits, const int64_t* user_ptr, const int64_t* item,
+                            const float* pref, int mem, mb200_sized_bank** out);
+int mb200_sized_bank_destroy(mb200_sized_bank* bank);
+/* user row u's own sketch as the reference's doubles, HOST out[depth[u]][width[u]] */
+int mb200_sized_bank_read(mb200_sized_bank* bank, int64_t user, double* out);
+/* CosineCM.userSimilarity(u1[t], u2[t]) exactly as written (CosineCM.java:84-96): u1's prefs sketched at u2's
+ * shape, DoubleCountMinSketch.cosine against u2's own sketch (min over rows of AB/(sqrt(AA)*sqrt(BB)), rows with a
+ * zero denominator skipped, NaN if none), clamped to [-1, 1] with NaN kept.  Bit-equal to
+ * mb200_bank_cross_cosine on two banks of u2's shape.  MB200_ERR_RANGE if a re-sketched row's sum of squared quanta
+ * reaches 2^53 (the FP64 sums would no longer be exact). */
+int mb200_sized_pair_cosine(mb200_sized_bank* bank, const int64_t* u1, const int64_t* u2, int64_t n, double* out,
+                            int mem);
+/* NearestNUserNeighborhood(n, min_similarity) over that similarity for the q query rows: every other user v is
+ * scored as userSimilarity(query, v); NaN is never admitted, sim >= min_similarity is (negatives too: pass -INFINITY
+ * for no threshold); the best n under (sim desc, user row asc) are kept.  n in [1, 1024].  out_idx / out_sim
+ * [q][n] (unused slots -1 / 0), out_cnt [q] -- mb200_bank_cosine_topk's list format. */
+int mb200_sized_neighborhood(mb200_sized_bank* bank, const int64_t* query_rows, int64_t q, int32_t n,
+                             double min_similarity, int64_t* out_idx, double* out_sim, int32_t* out_cnt, int mem);
+/* mb200_bank_estimate_prefs's contract, except that neighbour v's point query is min over v's own depth[v] rows of
+ * C_v[i][h_i(item) mod width[v]] (the sketch CosineCM.getExportedCMProfile(v) caches). */
+int mb200_sized_estimate_prefs(mb200_sized_bank* bank, const int64_t* nb_idx, const double* nb_sim,
+                               const int32_t* nb_cnt, int64_t nb_rows, int32_t nb_ld, const int64_t* user,
+                               const int64_t* nb_row, const int64_t* item_id, int64_t q, float* out, int mem);
+/* what the last mb200_sized_neighborhood on the context did: queries, distinct candidate shapes (classes), classes
+ * whose query sketches were built in shared memory or in a per-CTA global slice, pair FMAs of the shape model
+ * (sum over classes of queries * members * depth * width), query batches, work items, the largest query tile and
+ * the shared-memory budget for query sketches */
+typedef struct mb200_sized_plan {
+  int64_t queries, classes, smem_classes, global_classes, pair_fmas, batches, items;
+  int32_t query_tile_max, smem_bytes;
+} mb200_sized_plan;
+int mb200_sized_last_plan(mb200_ctx* ctx, mb200_sized_plan* out);
+
 /* ---- item-based recommendation over the item top-k lists (RecommenderJob's aggregate-and-recommend phase) ---- */
 /* UserVectorSplitterMapper + PartialMultiplyMapper + AggregateAndRecommendReducer of upstream RecommenderJob
  * (cf/taste/hadoop/item/), restated in DESIGN.md section 3.  For user row u:

@@ -145,6 +145,34 @@ public final class NativeSketch {
                                                int[] allowed, long[] users, int howMany, int maxPrefsPerUser,
                                                boolean booleanData, long[] outItem, float[] outValue, int[] outCnt);
 
+  /**
+   * mb200_sized_bank_create: CosineCM with a CountMinSketchConfig -- user row u's sketch at (width[u], depth[u]) =
+   * the (w, d) of new DoubleCountMinSketch(getDelta(u), getEpsilon(u), hfb), all users sharing the hash parameters
+   * a / b (hashParams for the largest depth).  The data model is CSR by user row: userPtr [users + 1], item / pref.
+   */
+  public static native long createSizedBank(long ctx, int[] width, int[] depth, long[] a, long[] b, int fracBits,
+                                            long[] userPtr, long[] item, float[] pref);
+  public static native void destroySizedBank(long sizedBank);
+
+  /** mb200_sized_pair_cosine: CosineCM.userSimilarity(u1[t], u2[t]) (u1 re-sketched at u2's size), clamped. */
+  public static native void sizedPairCosine(long sizedBank, long[] u1, long[] u2, double[] out);
+
+  /**
+   * mb200_sized_neighborhood: NearestNUserNeighborhood(n, minSimilarity) over that similarity for the user rows
+   * queryRows (Double.NEGATIVE_INFINITY = no threshold).  outIdx / outSim are [queries][n] (unused -1 / 0), outCnt
+   * [queries].
+   */
+  public static native void sizedNeighborhood(long sizedBank, long[] queryRows, int n, double minSimilarity,
+                                              long[] outIdx, double[] outSim, int[] outCnt);
+
+  /**
+   * mb200_sized_estimate_prefs: doEstimatePreference for the (user row, itemID) pairs user[t], itemId[t] over the
+   * lists of sizedNeighborhood (row nbRow[t] of them; nbRow null = row user[t]), each neighbour point-queried in its
+   * own sketch; out[t] is NaN where there is no estimate.
+   */
+  public static native void sizedEstimatePrefs(long sizedBank, long[] nbIdx, double[] nbSim, int[] nbCnt, int nbLd,
+                                               long[] user, long[] nbRow, long[] itemId, float[] out);
+
   /** mb200_host_alloc / mb200_host_free wrapped as a direct ByteBuffer. */
   public static native ByteBuffer allocPinned(long bytes);
   public static native void freePinned(ByteBuffer buffer);

@@ -360,3 +360,101 @@ JNIEXPORT void JNICALL JNI_FN(recommendItemBased)(JNIEnv* env, jclass c, jlong c
   (*env)->ReleaseIntArrayElements(env, outCnt, (jint*)a.out_cnt, 0);
   CHECK(rc, (mb200_ctx*)(intptr_t)ctx);
 }
+
+/* ---- CosineCM with a CountMinSketchConfig: per-user sketch sizes (csrc/cmsized.cu) ------------------------------ */
+JNIEXPORT jlong JNICALL JNI_FN(createSizedBank)(JNIEnv* env, jclass c, jlong ctx, jintArray width, jintArray depth,
+                                                jlongArray a, jlongArray b, jint fracBits, jlongArray userPtr,
+                                                jlongArray item, jfloatArray pref) {
+  mb200_sized_bank* bank = NULL;
+  const jsize users = (*env)->GetArrayLength(env, width);
+  jint* pw = (*env)->GetIntArrayElements(env, width, NULL);
+  jint* pd = (*env)->GetIntArrayElements(env, depth, NULL);
+  jlong* pa = (*env)->GetLongArrayElements(env, a, NULL);
+  jlong* pb = (*env)->GetLongArrayElements(env, b, NULL);
+  jlong* pp = (*env)->GetLongArrayElements(env, userPtr, NULL);
+  jlong* pi = (*env)->GetLongArrayElements(env, item, NULL);
+  jfloat* pv = (*env)->GetFloatArrayElements(env, pref, NULL);
+  int rc = (*env)->GetArrayLength(env, depth) != users || (*env)->GetArrayLength(env, userPtr) != users + 1 ||
+                   (*env)->GetArrayLength(env, pref) != (*env)->GetArrayLength(env, item) ||
+                   (users > 0 && pp[users] != (*env)->GetArrayLength(env, item))
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_bank_create((mb200_ctx*)(intptr_t)ctx, users, (const int32_t*)pw, (const int32_t*)pd,
+                                         (const int64_t*)pa, (const int64_t*)pb, fracBits, (const int64_t*)pp,
+                                         (const int64_t*)pi, (const float*)pv, MB200_MEM_HOST, &bank);
+  (*env)->ReleaseIntArrayElements(env, width, pw, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, depth, pd, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, a, pa, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, b, pb, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, userPtr, pp, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, item, pi, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, pref, pv, JNI_ABORT);
+  CHECK(rc, (mb200_ctx*)(intptr_t)ctx);
+  return (jlong)(intptr_t)bank;
+}
+
+JNIEXPORT void JNICALL JNI_FN(destroySizedBank)(JNIEnv* env, jclass c, jlong bank) {
+  mb200_sized_bank_destroy((mb200_sized_bank*)(intptr_t)bank);
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedPairCosine)(JNIEnv* env, jclass c, jlong bank, jlongArray u1, jlongArray u2,
+                                               jdoubleArray out) {
+  const jsize n = (*env)->GetArrayLength(env, u1);
+  jlong* p1 = (*env)->GetLongArrayElements(env, u1, NULL);
+  jlong* p2 = (*env)->GetLongArrayElements(env, u2, NULL);
+  jdouble* po = (*env)->GetDoubleArrayElements(env, out, NULL);
+  int rc = (*env)->GetArrayLength(env, u2) != n || (*env)->GetArrayLength(env, out) != n
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_pair_cosine((mb200_sized_bank*)(intptr_t)bank, (const int64_t*)p1, (const int64_t*)p2, n,
+                                         po, MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, u1, p1, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, u2, p2, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, out, po, 0);
+  CHECK(rc, NULL);
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedNeighborhood)(JNIEnv* env, jclass c, jlong bank, jlongArray queryRows, jint n,
+                                                 jdouble minSimilarity, jlongArray outIdx, jdoubleArray outSim,
+                                                 jintArray outCnt) {
+  const jsize q = (*env)->GetArrayLength(env, queryRows);
+  jlong* pq = (*env)->GetLongArrayElements(env, queryRows, NULL);
+  jlong* oi = (*env)->GetLongArrayElements(env, outIdx, NULL);
+  jdouble* os = (*env)->GetDoubleArrayElements(env, outSim, NULL);
+  jint* oc = (*env)->GetIntArrayElements(env, outCnt, NULL);
+  int rc = (*env)->GetArrayLength(env, outCnt) != q || (int64_t)(*env)->GetArrayLength(env, outIdx) != (int64_t)q * n ||
+                   (*env)->GetArrayLength(env, outSim) != (*env)->GetArrayLength(env, outIdx)
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_neighborhood((mb200_sized_bank*)(intptr_t)bank, (const int64_t*)pq, q, n, minSimilarity,
+                                          (int64_t*)oi, os, (int32_t*)oc, MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, queryRows, pq, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outIdx, oi, 0);
+  (*env)->ReleaseDoubleArrayElements(env, outSim, os, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
+  CHECK(rc, NULL);
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedEstimatePrefs)(JNIEnv* env, jclass c, jlong bank, jlongArray nbIdx,
+                                                  jdoubleArray nbSim, jintArray nbCnt, jint nbLd, jlongArray user,
+                                                  jlongArray nbRow, jlongArray itemId, jfloatArray out) {
+  const jsize rows = (*env)->GetArrayLength(env, nbCnt), q = (*env)->GetArrayLength(env, user);
+  jlong* pi = (*env)->GetLongArrayElements(env, nbIdx, NULL);
+  jdouble* ps = (*env)->GetDoubleArrayElements(env, nbSim, NULL);
+  jint* pc = (*env)->GetIntArrayElements(env, nbCnt, NULL);
+  jlong* pu = (*env)->GetLongArrayElements(env, user, NULL);
+  jlong* pr = nbRow ? (*env)->GetLongArrayElements(env, nbRow, NULL) : NULL;
+  jlong* pt = (*env)->GetLongArrayElements(env, itemId, NULL);
+  jfloat* po = (*env)->GetFloatArrayElements(env, out, NULL);
+  int rc = (*env)->GetArrayLength(env, itemId) != q || (*env)->GetArrayLength(env, out) != q ||
+                   (nbRow && (*env)->GetArrayLength(env, nbRow) != q)
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_estimate_prefs((mb200_sized_bank*)(intptr_t)bank, (const int64_t*)pi, ps,
+                                            (const int32_t*)pc, rows, nbLd, (const int64_t*)pu, (const int64_t*)pr,
+                                            (const int64_t*)pt, q, (float*)po, MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, nbIdx, pi, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, nbSim, ps, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, nbCnt, pc, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, user, pu, JNI_ABORT);
+  if (pr) (*env)->ReleaseLongArrayElements(env, nbRow, pr, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemId, pt, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, out, po, 0);
+  CHECK(rc, NULL);
+}

@@ -5,7 +5,7 @@ host-side mirror of the reference's operator API over that ABI.  No CPU fallback
 """
 from ._native import (CMException, InexactError, NativeError, LIB_PATH)  # noqa: F401
 from .sketch import (Context, DoubleCountMinSketch, HashFunction, HashFunctionBuilder,  # noqa: F401
-                     SketchBank, cm_dims, default_context)
+                     SizedBank, SketchBank, cm_dims, default_context)
 
-__all__ = ["Context", "DoubleCountMinSketch", "HashFunction", "HashFunctionBuilder", "SketchBank",
+__all__ = ["Context", "DoubleCountMinSketch", "HashFunction", "HashFunctionBuilder", "SizedBank", "SketchBank",
            "cm_dims", "default_context", "CMException", "InexactError", "NativeError", "LIB_PATH"]

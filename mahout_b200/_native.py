@@ -106,6 +106,13 @@ class ItemBasedPlan(C.Structure):
                 ("table_slots", C.c_int32), ("dense_slices", C.c_int32)]
 
 
+class SizedPlan(C.Structure):
+    """struct mb200_sized_plan (include/mahout_b200.h)."""
+    _fields_ = [("queries", C.c_int64), ("classes", C.c_int64), ("smem_classes", C.c_int64),
+                ("global_classes", C.c_int64), ("pair_fmas", C.c_int64), ("batches", C.c_int64), ("items", C.c_int64),
+                ("query_tile_max", C.c_int32), ("smem_bytes", C.c_int32)]
+
+
 class CosinePiece(C.Structure):
     """struct mb200_cosine_piece (include/mahout_b200.h)."""
     _fields_ = [
@@ -161,6 +168,13 @@ _PROTOS = {
     "mb200_recommend_last_plan": (C.c_int, [vp, C.POINTER(RecommendPlan)]),
     "mb200_recommend_item_based": (C.c_int, [vp, C.POINTER(ItemBasedArgs)]),
     "mb200_itembased_last_plan": (C.c_int, [vp, C.POINTER(ItemBasedPlan)]),
+    "mb200_sized_bank_create": (C.c_int, [vp, i64, vp, vp, vp, vp, i32, vp, vp, vp, C.c_int, C.POINTER(vp)]),
+    "mb200_sized_bank_destroy": (C.c_int, [vp]),
+    "mb200_sized_bank_read": (C.c_int, [vp, i64, vp]),
+    "mb200_sized_pair_cosine": (C.c_int, [vp, vp, vp, i64, vp, C.c_int]),
+    "mb200_sized_neighborhood": (C.c_int, [vp, vp, i64, i32, f64, vp, vp, vp, C.c_int]),
+    "mb200_sized_estimate_prefs": (C.c_int, [vp, vp, vp, vp, i64, i32, vp, vp, vp, i64, vp, C.c_int]),
+    "mb200_sized_last_plan": (C.c_int, [vp, C.POINTER(SizedPlan)]),
     "mb200_row_ld": (i64, [i32]),
     "mb200_valid_words": (i64, [i64]),
     "mb200_bank_normalize": (C.c_int, [vp, C.c_int, vp, vp]),

@@ -6,9 +6,11 @@ user's preferences (key = itemID, increment = preference value, CosineCM.java:41
 AbstractSimilarity.normalizeWeightResult, AbstractSimilarity.java:313-330, unweighted), plus the
 point-query consumer of GenericUserBasedRecommender.doEstimatePreference (:139-159).
 
-The reference sizes u1's sketch by u2's (delta, epsilon) on every call and rebuilds it each time;
-here all users share one (width, depth) -- what BASELINE.json's configurations fix -- and every
-profile is built once, in one K1 launch.  Per-user sizing (CountMinSketchConfig) is SURVEY.md 8f-4.
+The reference sizes u1's sketch by u2's (delta, epsilon) on every call and rebuilds it each time.
+`userSimilarity` lets all users share one (width, depth) -- what BASELINE.json's configurations fix -- and
+builds every profile once, in one K1 launch.  With a CountMinSketchConfig (SURVEY.md 8f-4),
+`userSimilaritiesPerUserConfig` follows the reference's per-pair sizing on a SizedBank: every user's sketch
+at its own cm_dims(getDelta(u), getEpsilon(u)), u1 re-sketched on the device at u2's shape.
 """
 from __future__ import annotations
 
@@ -26,6 +28,7 @@ class CosineCM:
         per-pair sizing (u1's sketch rebuilt with u2's (delta, epsilon), CosineCM.java:84-96)."""
         user = np.asarray(user, np.int64)
         self.config = config
+        self._sized = None
         self._hfb = hfBuilder if isinstance(hfBuilder, sk.HashFunctionBuilder) else sk.HashFunctionBuilder(int(hfBuilder))
         self._frac_bits, self._ctx = frac_bits, ctx
         order = np.argsort(user, kind="stable")
@@ -78,14 +81,38 @@ class CosineCM:
         cm.update(items, prefs)
         return cm
 
+    def sized_bank(self) -> sk.SizedBank:
+        """every user's sketch at its own (delta, epsilon) from `config`, shaped as `new DoubleCountMinSketch(delta,
+        epsilon, hfb)` shapes it (cm_dims of the stored parameters, never best_dims); built on first use"""
+        if self._sized is None:
+            if self.config is None:
+                raise ValueError("no CountMinSketchConfig was given")
+            dims = {}
+            w = np.empty(self.user_ids.shape[0], np.int32)
+            d = np.empty(self.user_ids.shape[0], np.int32)
+            for r, u in enumerate(self.user_ids.tolist()):
+                key = (self.config.getDelta(u), self.config.getEpsilon(u))
+                if key not in dims:
+                    try:
+                        dims[key] = sk.cm_dims(*key)
+                    except sk.N.CMException as e:    # CosineCM.java:45-47 wraps it in a TasteException
+                        raise RuntimeError(f"CountMinSketch error:{e}") from e
+                w[r], d[r] = dims[key]
+            ptr = np.zeros(self.user_ids.shape[0] + 1, np.int64)
+            np.cumsum(np.bincount(np.searchsorted(self.user_ids, self._u_sorted), minlength=self.user_ids.shape[0]),
+                      out=ptr[1:])
+            self._sized = sk.SizedBank(w, d, self._hfb, ptr, self._i_sorted, self._p_sorted.astype(np.float32),
+                                       self._frac_bits, self.bank.ctx)
+        return self._sized
+
+    def userSimilaritiesPerUserConfig(self, ids1, ids2) -> np.ndarray:
+        """CosineCM.userSimilarity exactly as written (:84-96) for the pairs (ids1[t], ids2[t]): user 1's prefs
+        sketched at user 2's size, compared with user 2's own sketch, clamped to [-1, 1] (NaN kept)."""
+        return self.sized_bank().pair_cosine(self._rows(ids1), self._rows(ids2))
+
     def userSimilarityPerUserConfig(self, userID1: int, userID2: int) -> float:
-        """CosineCM.userSimilarity exactly as written (:84-96): both sketches sized by user 2's parameters."""
-        if self.config is None:
-            raise ValueError("no CountMinSketchConfig was given")
-        d2, e2 = self.config.getDelta(userID2), self.config.getEpsilon(userID2)
-        cm1, cm2 = self.exportProfile(userID1, d2, e2), self.exportProfile(userID2, d2, e2)
-        r = sk.DoubleCountMinSketch.cosine(cm1, cm2)
-        return r if math.isnan(r) else float(np.clip(r, -1.0, 1.0))
+        """one pair of userSimilaritiesPerUserConfig"""
+        return float(self.userSimilaritiesPerUserConfig([userID1], [userID2])[0])
 
     def doEstimatePreference(self, theUserID: int, theNeighborhood, itemID: int) -> float:
         """GenericUserBasedRecommender.doEstimatePreference with the sketch point query (:134-184): one batched pair
@@ -118,4 +145,6 @@ class CosineCM:
         return self.user_ids[idx[r, :cnt[r]]], sim[r, :cnt[r]]
 
     def close(self):
+        if self._sized is not None:
+            self._sized.close()
         self.bank.close()

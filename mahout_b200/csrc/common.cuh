@@ -72,6 +72,7 @@ struct mb200_ctx {
   struct mb200_cosine_job* active_job = nullptr;  // the cosine stage's workspaces serve one job at a time
   mb200_recommend_plan last_recommend_plan = {};  // mb200_recommend_last_plan
   mb200_itembased_plan last_itembased_plan = {};  // mb200_itembased_last_plan
+  mb200_sized_plan last_sized_plan = {};          // mb200_sized_last_plan
   int64_t itembased_dense_items = -1, itembased_dense_slices = -1;  // layout of the zeroed dense slices (slot 62)
 };
 

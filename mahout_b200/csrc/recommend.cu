@@ -27,6 +27,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "nb_terms.cuh"
 #include "tc05.cuh"
 
 namespace {
@@ -71,26 +72,6 @@ struct RecArgs {
   int ch;                // candidates per chunk (multiple of REC_THREADS, <= REC_KMAX * REC_THREADS)
   unsigned long long* plan;
 };
-
-__device__ __forceinline__ double clamp_sim(double s) {
-  // AbstractSimilarity.normalizeWeightResult: clamp to [-1, 1], NaN stays NaN
-  return s != s ? s : (s < -1.0 ? -1.0 : (s > 1.0 ? 1.0 : s));
-}
-
-// one neighbour's term of doEstimatePreference, FP64 with the product and the sum rounded separately (Java does not
-// fuse them)
-__device__ __forceinline__ void nb_term(long long mn, double inv_q, double s, double& pref, double& tot, int& count) {
-  const float p = __double2float_rn((double)mn * inv_q);
-  if (p != 0.0f && s == s) {
-    pref = __dadd_rn(pref, __dmul_rn(s, (double)p));
-    tot = __dadd_rn(tot, s);
-    count++;
-  }
-}
-
-__device__ __forceinline__ float nb_result(double pref, double tot, int count) {
-  return count <= 1 ? __int_as_float(0x7fc00000) : __double2float_rn(pref / tot);
-}
 
 // min over the d rows of sketch `sk` at the columns cols[r * stride] -- DoubleCountMinSketch.get on int64 quanta
 // (the conversion to double is exact and monotone, so the min commutes with it)

@@ -66,3 +66,42 @@ class GenericUserBasedRecommender:
         rows = torch.from_numpy(self.cm._rows(userIDs)).to(dev)
         items = torch.from_numpy(np.ascontiguousarray(np.atleast_1d(itemIDs), np.int64)).to(dev)
         return self.bank.estimate_prefs(self.nb_idx, self.nb_sim, self.nb_cnt, rows, items).cpu().numpy()
+
+
+class PerUserConfigUserBasedRecommender:
+    """GenericUserBasedRecommender's neighbourhoods and estimates over CosineCM with a CountMinSketchConfig: every
+    user's sketch at its own size (CosineCM.sized_bank), similarities as CosineCM.userSimilarity computes them (user 1
+    re-sketched at user 2's size), NearestNUserNeighborhood(n, min_similarity) exactly -- NaN never admitted,
+    negative similarities admitted when they pass min_similarity, ties by lower user row -- and doEstimatePreference
+    point-querying each neighbour's own sketch.  All in K_RECOMMEND (csrc/cmsized.cu)."""
+
+    def __init__(self, cm: CosineCM, n: int, min_similarity: float = float("-inf")):
+        self.cm = cm
+        self.bank = cm.sized_bank()
+        self.n = int(n)
+        self.min_similarity = float(min_similarity)
+
+    def _dev(self):
+        return f"cuda:{self.bank.ctx.device}"
+
+    def neighborhoods(self, userIDs=None):
+        """(idx [m, n], sim [m, n], cnt [m]) as device tensors, rows = user rows (unused slots -1 / 0), for userIDs
+        (every user when None)"""
+        import torch
+        rows = np.arange(self.cm.user_ids.shape[0], dtype=np.int64) if userIDs is None else self.cm._rows(userIDs)
+        return self.bank.neighborhood(torch.from_numpy(rows).to(self._dev()), self.n, self.min_similarity)
+
+    def getUserNeighborhood(self, userID: int) -> np.ndarray:
+        idx, _, cnt = self.bank.neighborhood(self.cm._rows(userID), self.n, self.min_similarity)
+        return self.cm.user_ids[idx[0, :int(cnt[0])]]
+
+    def estimate_preferences(self, userIDs, itemIDs) -> np.ndarray:
+        """doEstimatePreference for (userID, itemID) pairs over each user's neighbourhood; float32, NaN = none"""
+        import torch
+        rows = self.cm._rows(userIDs)
+        uniq, inv = np.unique(rows, return_inverse=True)
+        dev = self._dev()
+        idx, sim, cnt = self.bank.neighborhood(torch.from_numpy(uniq).to(dev), self.n, self.min_similarity)
+        items = torch.from_numpy(np.ascontiguousarray(np.atleast_1d(itemIDs), np.int64)).to(dev)
+        return self.bank.estimate_prefs(idx, sim, cnt, torch.from_numpy(rows).to(dev), items,
+                                        nb_row=torch.from_numpy(inv.astype(np.int64)).to(dev)).cpu().numpy()

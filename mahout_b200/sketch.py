@@ -495,6 +495,120 @@ class SketchBank:
         return p.value, n.value
 
 
+class SizedBank:
+    """One count-min sketch per user at the user's own (width[u], depth[u]) -- what a CountMinSketchConfig gives --
+    all sharing one HashFunctionBuilder, built from the data model as CSR by user row (user_ptr [U+1], item / pref
+    [nnz]).  The prefs stay on the device: similarities re-sketch a user at another user's shape
+    (CosineCM.userSimilarity, CosineCM.java:84-96)."""
+
+    def __init__(self, width, depth, hfBuilder: HashFunctionBuilder | int, user_ptr, item, pref, frac_bits: int = 1,
+                 ctx: Context | None = None):
+        self.ctx = ctx or default_context()
+        if not isinstance(hfBuilder, (HashFunctionBuilder, IdentityHashBuilder)):
+            hfBuilder = HashFunctionBuilder(int(hfBuilder))
+        self.width = np.ascontiguousarray(width, np.int32)
+        self.depth = np.ascontiguousarray(depth, np.int32)
+        if self.width.shape != self.depth.shape or self.width.ndim != 1:
+            raise ValueError("width and depth must be 1-d arrays of one entry per user")
+        dmax = int(self.depth.max()) if self.depth.size else 1
+        if not (0 < dmax <= N.MAX_DEPTH):
+            raise ValueError(f"depth must be in (0, {N.MAX_DEPTH}] (got {dmax})")
+        self.a, self.b = hfBuilder.params(dmax)
+        p = _Arg(user_ptr, np.int64, "int64")
+        it = _Arg(item, np.int64, "int64")
+        pr = _Arg(pref, np.float32, "float32")
+        wa = _Arg(self.width, np.int32, "int32")
+        da = _Arg(self.depth, np.int32, "int32")
+        if p.n != self.width.shape[0] + 1 or it.n != pr.n:
+            raise ValueError("user_ptr must have users + 1 entries; item and pref the same length")
+        mem = _same_mem(p, it, pr)
+        if mem == N.MEM_DEVICE:   # the shapes are small host arrays; the device path wants all arrays alike
+            import torch
+            dev = f"cuda:{self.ctx.device}"
+            wa = _Arg(torch.from_numpy(self.width).to(dev), np.int32, "int32")
+            da = _Arg(torch.from_numpy(self.depth).to(dev), np.int32, "int32")
+        h = C.c_void_p()
+        self._h = None
+        N.check(N.lib().mb200_sized_bank_create(
+            self.ctx.handle, self.width.shape[0], wa.ptr, da.ptr, self.a.ctypes.data_as(C.c_void_p),
+            self.b.ctypes.data_as(C.c_void_p), int(frac_bits), p.ptr, it.ptr, pr.ptr, mem, C.byref(h)), self.ctx.handle)
+        self._h = h
+        self.U, self.frac_bits = int(self.width.shape[0]), int(frac_bits)
+
+    @property
+    def handle(self):
+        if self._h is None:
+            raise ValueError("bank is closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and self.ctx._h is not None:
+            try:
+                N.lib().mb200_sized_bank_destroy(self._h)
+            except Exception:   # interpreter shutdown
+                pass
+        self._h = None
+
+    __del__ = close
+
+    def read(self, user: int) -> np.ndarray:
+        """user row `user`'s own sketch as the reference's doubles, [depth[user], width[user]]"""
+        if not (0 <= int(user) < self.U):
+            raise ValueError(f"user row {user} outside [0, {self.U})")
+        out = np.empty((int(self.depth[user]), int(self.width[user])), np.float64)
+        N.check(N.lib().mb200_sized_bank_read(self.handle, int(user), out.ctypes.data_as(C.c_void_p)), self.ctx.handle)
+        return out
+
+    def pair_cosine(self, u1, u2):
+        """CosineCM.userSimilarity(u1[t], u2[t]) (u1 re-sketched at u2's shape), clamped, NaN kept; float64"""
+        a = _Arg(u1, np.int64, "int64")
+        b = _Arg(u2, np.int64, "int64")
+        if a.n != b.n:
+            raise ValueError("u1 and u2 must have the same length")
+        mem = _same_mem(a, b)
+        out, optr = _out((a.n,), np.float64, "float64", mem, self.ctx.device)
+        N.check(N.lib().mb200_sized_pair_cosine(self.handle, a.ptr, b.ptr, a.n, optr, mem), self.ctx.handle)
+        return out
+
+    def neighborhood(self, query_rows, n: int, min_similarity: float = -np.inf):
+        """NearestNUserNeighborhood(n, min_similarity) of each query row over that similarity: (idx [q, n] int64,
+        sim [q, n] float64, cnt [q] int32), unused slots -1 / 0; host or device like query_rows."""
+        qa = _Arg(query_rows, np.int64, "int64")
+        mem = _same_mem(qa)
+        idx, pi = _out((qa.n, int(n)), np.int64, "int64", mem, self.ctx.device)
+        sim, ps = _out((qa.n, int(n)), np.float64, "float64", mem, self.ctx.device)
+        cnt, pc = _out((qa.n,), np.int32, "int32", mem, self.ctx.device)
+        N.check(N.lib().mb200_sized_neighborhood(self.handle, qa.ptr, qa.n, int(n), float(min_similarity), pi, ps, pc,
+                                                 mem), self.ctx.handle)
+        return idx, sim, cnt
+
+    def estimate_prefs(self, nb_idx, nb_sim, nb_cnt, user, item_id, nb_row=None):
+        """doEstimatePreference for q (user row, itemID) pairs, each neighbour point-queried in its own sketch;
+        the lists as neighborhood() returns them.  float32 [q], NaN where there is no estimate."""
+        ni = _Arg(nb_idx, np.int64, "int64")
+        ns = _Arg(nb_sim, np.float64, "float64")
+        nc = _Arg(nb_cnt, np.int32, "int32")
+        u = _Arg(user, np.int64, "int64")
+        it = _Arg(item_id, np.int64, "int64")
+        nr = _Arg(nb_row, np.int64, "int64", allow_none=True)
+        rows = nc.n
+        ld = ni.n // rows if rows else 1
+        if ni.n != rows * ld or ns.n != ni.n or it.n != u.n or (nr.ptr is not None and nr.n != u.n):
+            raise ValueError("nb_idx / nb_sim must be [rows, ld] with rows = len(nb_cnt); user, item_id (and nb_row) "
+                             "the same length")
+        mem = _same_mem(ni, ns, nc, u, it, nr)
+        out, optr = _out((u.n,), np.float32, "float32", mem, self.ctx.device)
+        N.check(N.lib().mb200_sized_estimate_prefs(self.handle, ni.ptr, ns.ptr, nc.ptr, rows, max(ld, 1), u.ptr,
+                                                   nr.ptr, it.ptr, u.n, optr, mem), self.ctx.handle)
+        return out
+
+    def plan(self) -> dict:
+        """what the last neighborhood() on this bank's context did (mb200_sized_last_plan)"""
+        pl = N.SizedPlan()
+        N.check(N.lib().mb200_sized_last_plan(self.ctx.handle, C.byref(pl)), self.ctx.handle)
+        return {f: getattr(pl, f) for f, _ in N.SizedPlan._fields_}
+
+
 _DTYPES = {"f16": N.DTYPE_F16, "bf16": N.DTYPE_BF16}
 _PRECISIONS = {"tensor": N.PRECISION_TENSOR, "rescored": N.PRECISION_RESCORED, "certified": N.PRECISION_CERTIFIED}
 
