@@ -295,6 +295,30 @@ typedef struct mb200_sized_plan {
   int32_t query_tile_max, smem_bytes;
 } mb200_sized_plan;
 int mb200_sized_last_plan(mb200_ctx* ctx, mb200_sized_plan* out);
+/* recommend(user, how_many) for m user rows over per-user sketch shapes: mb200_bank_recommend's contract (the data
+ * model as CSR over the bank's user rows, item_ptr [users + 1]; candidates, NaN dropped, (value desc, itemID asc)),
+ * except that the neighbourhood of users[t] is row t of the lists (nb_idx / nb_sim [m][nb_ld], nb_cnt [m], as
+ * mb200_sized_neighborhood returns them for users) and every estimate is mb200_sized_estimate_prefs's, bit for bit.
+ * Negative similarities can make an estimate negative or infinite; it ranks by value like any other.  Out-of-range
+ * user rows, counts, neighbour indexes, item_ptr ranges and item_col entries fail with MB200_ERR_BAD_ARG. */
+int mb200_sized_recommend(mb200_sized_bank* bank, const int64_t* nb_idx, const double* nb_sim, const int32_t* nb_cnt,
+                          int32_t nb_ld, const int64_t* item_ptr, const int32_t* item_col, int64_t nnz,
+                          const int64_t* item_ids, int64_t num_items, const int64_t* users, int64_t m,
+                          int32_t how_many, int include_known, int64_t* out_item, float* out_value, int32_t* out_cnt,
+                          int mem);
+/* what the last mb200_sized_recommend on the context did.  Per candidate chunk each listed neighbour is either
+ * streamed (its whole sketch, or row by row when the sketch does not fit a stage, through a shared-memory ring) or
+ * gathered (one counter per candidate and row), whichever moves fewer bytes (8*d*w against chunk*d*32); rows wider
+ * than a stage are always gathered.  users, chunks, candidates (sum, max), neighbour visits streamed (row_visits:
+ * those streamed row by row) / gathered (gathered includes too_wide: visits that would have streamed but did not fit
+ * a stage), bytes streamed, counters gathered, neighbour terms (sum over users of candidates * listed neighbours other than the user), pipeline
+ * stages, bytes per stage and candidates per chunk. */
+typedef struct mb200_sized_recommend_plan {
+  int64_t users, chunks, candidates, candidates_max, stream_visits, row_visits, gather_visits, too_wide_visits,
+      stream_bytes, gather_loads, terms;
+  int32_t stages, stage_bytes, chunk_candidates;
+} mb200_sized_recommend_plan;
+int mb200_sized_recommend_last_plan(mb200_ctx* ctx, mb200_sized_recommend_plan* out);
 
 /* ---- item-based recommendation over the item top-k lists (RecommenderJob's aggregate-and-recommend phase) ---- */
 /* UserVectorSplitterMapper + PartialMultiplyMapper + AggregateAndRecommendReducer of upstream RecommenderJob

@@ -173,6 +173,17 @@ public final class NativeSketch {
   public static native void sizedEstimatePrefs(long sizedBank, long[] nbIdx, double[] nbSim, int[] nbCnt, int nbLd,
                                                long[] user, long[] nbRow, long[] itemId, float[] out);
 
+  /**
+   * mb200_sized_recommend: GenericUserBasedRecommender.recommend(userID, howMany) over the per-user sketch sizes for
+   * the user rows `users`.  Row t of the lists (nbIdx / nbSim [users][nbLd], nbCnt [users], as sizedNeighborhood
+   * returns them for `users`) is users[t]'s neighbourhood, and every estimate is sizedEstimatePrefs's.  The data
+   * model is CSR over user rows: itemPtr [rows + 1], itemCol = dense item numbers into itemIds (ascending itemIDs).
+   * outItem / outValue are [users][howMany] (unused -1 / 0), outCnt [users].
+   */
+  public static native void sizedRecommend(long sizedBank, long[] nbIdx, double[] nbSim, int[] nbCnt, int nbLd,
+                                           long[] itemPtr, int[] itemCol, long[] itemIds, long[] users, int howMany,
+                                           boolean includeKnown, long[] outItem, float[] outValue, int[] outCnt);
+
   /** mb200_host_alloc / mb200_host_free wrapped as a direct ByteBuffer. */
   public static native ByteBuffer allocPinned(long bytes);
   public static native void freePinned(ByteBuffer buffer);

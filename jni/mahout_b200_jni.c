@@ -458,3 +458,44 @@ JNIEXPORT void JNICALL JNI_FN(sizedEstimatePrefs)(JNIEnv* env, jclass c, jlong b
   (*env)->ReleaseFloatArrayElements(env, out, po, 0);
   CHECK(rc, NULL);
 }
+
+JNIEXPORT void JNICALL JNI_FN(sizedRecommend)(JNIEnv* env, jclass c, jlong bank, jlongArray nbIdx, jdoubleArray nbSim,
+                                              jintArray nbCnt, jint nbLd, jlongArray itemPtr, jintArray itemCol,
+                                              jlongArray itemIds, jlongArray users, jint howMany,
+                                              jboolean includeKnown, jlongArray outItem, jfloatArray outValue,
+                                              jintArray outCnt) {
+  jlong* pi = (*env)->GetLongArrayElements(env, nbIdx, NULL);
+  jdouble* ps = (*env)->GetDoubleArrayElements(env, nbSim, NULL);
+  jint* pc = (*env)->GetIntArrayElements(env, nbCnt, NULL);
+  jlong* pp = (*env)->GetLongArrayElements(env, itemPtr, NULL);
+  jint* pl = (*env)->GetIntArrayElements(env, itemCol, NULL);
+  jlong* pd = (*env)->GetLongArrayElements(env, itemIds, NULL);
+  jlong* pu = (*env)->GetLongArrayElements(env, users, NULL);
+  jlong* oi = (*env)->GetLongArrayElements(env, outItem, NULL);
+  jfloat* ov = (*env)->GetFloatArrayElements(env, outValue, NULL);
+  jint* oc = (*env)->GetIntArrayElements(env, outCnt, NULL);
+  const jsize m = (*env)->GetArrayLength(env, users);
+  /* row t of the lists is users[t]'s neighbourhood */
+  int rc = (*env)->GetArrayLength(env, nbCnt) != m || (*env)->GetArrayLength(env, outCnt) != m ||
+                   nbLd < 1 || (int64_t)(*env)->GetArrayLength(env, nbIdx) != (int64_t)m * nbLd ||
+                   (*env)->GetArrayLength(env, nbSim) != (*env)->GetArrayLength(env, nbIdx) ||
+                   (int64_t)(*env)->GetArrayLength(env, outItem) != (int64_t)m * howMany ||
+                   (*env)->GetArrayLength(env, outValue) != (*env)->GetArrayLength(env, outItem)
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_recommend((mb200_sized_bank*)(intptr_t)bank, (const int64_t*)pi, ps, (const int32_t*)pc,
+                                       nbLd, (const int64_t*)pp, (const int32_t*)pl,
+                                       (*env)->GetArrayLength(env, itemCol), (const int64_t*)pd,
+                                       (*env)->GetArrayLength(env, itemIds), (const int64_t*)pu, m, howMany,
+                                       includeKnown, (int64_t*)oi, (float*)ov, (int32_t*)oc, MB200_MEM_HOST);
+  (*env)->ReleaseLongArrayElements(env, nbIdx, pi, JNI_ABORT);
+  (*env)->ReleaseDoubleArrayElements(env, nbSim, ps, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, nbCnt, pc, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemPtr, pp, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, itemCol, pl, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemIds, pd, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, users, pu, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outItem, oi, 0);
+  (*env)->ReleaseFloatArrayElements(env, outValue, ov, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
+  CHECK(rc, NULL);
+}

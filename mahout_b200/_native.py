@@ -113,6 +113,16 @@ class SizedPlan(C.Structure):
                 ("query_tile_max", C.c_int32), ("smem_bytes", C.c_int32)]
 
 
+class SizedRecommendPlan(C.Structure):
+    """struct mb200_sized_recommend_plan (include/mahout_b200.h)."""
+    _fields_ = [("users", C.c_int64), ("chunks", C.c_int64), ("candidates", C.c_int64),
+                ("candidates_max", C.c_int64), ("stream_visits", C.c_int64), ("row_visits", C.c_int64),
+                ("gather_visits", C.c_int64),
+                ("too_wide_visits", C.c_int64), ("stream_bytes", C.c_int64), ("gather_loads", C.c_int64),
+                ("terms", C.c_int64), ("stages", C.c_int32), ("stage_bytes", C.c_int32),
+                ("chunk_candidates", C.c_int32)]
+
+
 class CosinePiece(C.Structure):
     """struct mb200_cosine_piece (include/mahout_b200.h)."""
     _fields_ = [
@@ -175,6 +185,9 @@ _PROTOS = {
     "mb200_sized_neighborhood": (C.c_int, [vp, vp, i64, i32, f64, vp, vp, vp, C.c_int]),
     "mb200_sized_estimate_prefs": (C.c_int, [vp, vp, vp, vp, i64, i32, vp, vp, vp, i64, vp, C.c_int]),
     "mb200_sized_last_plan": (C.c_int, [vp, C.POINTER(SizedPlan)]),
+    "mb200_sized_recommend": (C.c_int, [vp, vp, vp, vp, i32, vp, vp, i64, vp, i64, vp, i64, i32, C.c_int, vp, vp, vp,
+                                        C.c_int]),
+    "mb200_sized_recommend_last_plan": (C.c_int, [vp, C.POINTER(SizedRecommendPlan)]),
     "mb200_row_ld": (i64, [i32]),
     "mb200_valid_words": (i64, [i64]),
     "mb200_bank_normalize": (C.c_int, [vp, C.c_int, vp, vp]),

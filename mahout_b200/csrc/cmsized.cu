@@ -22,6 +22,10 @@
 //   k_sized_select    one CTA per query: radix select + bitonic sort of the admitted similarities of one batch row
 //   k_sized_pair      one CTA per pair (pair cosine of the batched Python call)
 //   k_sized_estimate  one thread per query, as k_estimate_prefs
+//   k_sized_recommend one persistent CTA per SM, one list row at a time, k_recommend's phases: candidate bitmap and
+//                     compaction; estimates per chunk of candidates, each neighbour either streamed (its whole
+//                     sketch or row by row, cp.async.bulk into an mbarrier ring) or gathered, whichever moves fewer
+//                     bytes; top-N
 #include <math.h>
 #include <stdlib.h>
 
@@ -33,6 +37,8 @@
 #include "common.cuh"
 #include "k1_dev.cuh"
 #include "nb_terms.cuh"
+#include "rec_topn.cuh"
+#include "tc05.cuh"
 
 struct mb200_sized_bank {
   mb200_ctx* ctx = nullptr;
@@ -356,30 +362,6 @@ __device__ __forceinline__ unsigned long long sim_key(double s, double min_sim) 
   return bits < 0 ? ~(unsigned long long)bits : ((unsigned long long)bits | 0x8000000000000000ull);
 }
 
-__device__ __forceinline__ int block_exscan(int x, int* sh, int* total) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  int inc = x;
-  for (int o = 1; o < 32; o <<= 1) {
-    const int y = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += y;
-  }
-  if (lane == 31) sh[warp] = inc;
-  __syncthreads();
-  if (warp == 0) {
-    int s = lane < nw ? sh[lane] : 0;
-    for (int o = 1; o < 32; o <<= 1) {
-      const int y = __shfl_up_sync(0xffffffffu, s, o);
-      if (lane >= o) s += y;
-    }
-    if (lane < nw) sh[lane] = s;
-  }
-  __syncthreads();
-  const int before = (warp ? sh[warp - 1] : 0) + inc - x;
-  *total = sh[nw - 1];
-  __syncthreads();
-  return before;
-}
-
 __global__ void __launch_bounds__(SEL_THREADS) k_sized_select(const double* __restrict__ sims, long long U, int n,
                                                               double min_sim, long long* __restrict__ out_idx,
                                                               double* __restrict__ out_sim, int* __restrict__ out_cnt) {
@@ -395,7 +377,7 @@ __global__ void __launch_bounds__(SEL_THREADS) k_sized_select(const double* __re
   double* os = out_sim + (size_t)blockIdx.x * n;
   int valid = 0, nvalid = 0;
   for (long long v = tid; v < U; v += SEL_THREADS) valid += sim_key(row[v], min_sim) != 0ull;
-  block_exscan(valid, scan_sh, &nvalid);
+  block_exscan<SEL_THREADS>(valid, scan_sh, &nvalid);
   // keys > kstar are all taken; of the keys == kstar the first `need_eq` in row order
   unsigned long long kstar = 0ull;
   unsigned need_eq = 0;
@@ -440,9 +422,9 @@ __global__ void __launch_bounds__(SEL_THREADS) k_sized_select(const double* __re
     const unsigned long long k = v < U ? sim_key(row[v], min_sim) : 0ull;
     const int eq = k != 0ull && k == kstar;
     int eq_total = 0, tk_total = 0;
-    const int eq_before = block_exscan(eq, scan_sh, &eq_total);
+    const int eq_before = block_exscan<SEL_THREADS>(eq, scan_sh, &eq_total);
     const int take = (k != 0ull && k > kstar) || (eq && (unsigned)(eq_taken + eq_before) < need_eq);
-    const int at = block_exscan(take, scan_sh, &tk_total);
+    const int at = block_exscan<SEL_THREADS>(take, scan_sh, &tk_total);
     if (take) {
       sel_key[taken + at] = k;
       sel_row[taken + at] = (int)v;
@@ -601,6 +583,340 @@ __global__ void __launch_bounds__(EST_THREADS) k_sized_estimate(
     nb_term(mn, inv_q, clamp_sim(nb_sim[row * ld + j]), pref, tot, count);
   }
   out[t] = nb_result(pref, tot, count);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// recommend(user, how_many): one persistent CTA per SM, one list row at a time (k_recommend's three phases)
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int SR_THREADS = 512;
+constexpr int SR_KMAX = 8;                  // candidates per thread and chunk
+constexpr int SR_BITMAP_SMEM_WORDS = 4096;  // 131072 items: larger catalogues use a per-CTA global bitmap
+constexpr int SR_RES_BYTES = 64 * 1024;     // the chunk's hash residues (more when d_max leaves < 512 candidates)
+constexpr int SR_STAGES = 4;
+
+enum { SR_GATHER = 0, SR_WHOLE, SR_ROWS, SR_TOO_WIDE };
+enum { RP_CHUNKS = 0, RP_CAND_SUM, RP_CAND_MAX, RP_STREAM, RP_ROWS, RP_GATHER, RP_TOO_WIDE, RP_STREAM_BYTES, RP_GATHER_LOADS,
+       RP_TERMS, RP_BAD, RP_NEXT, RP_WORDS };
+
+struct SrArgs {
+  const int* W;
+  const int* D;
+  const long long* off;
+  const long long* counters;
+  SizedHash hf;
+  int dmax;
+  long long U;
+  double inv_q;
+  const long long* nb_idx;  // [m][ld]: row t belongs to users[t]
+  const double* nb_sim;
+  const int* nb_cnt;
+  int ld;
+  const long long* item_ptr;
+  const int* item_col;
+  long long nnz;
+  const long long* item_ids;
+  long long num_items;
+  const long long* users;
+  long long m;
+  int how_many, include_known;
+  long long* out_item;
+  float* out_value;
+  int* out_cnt;
+  unsigned* ws_bitmap;         // [grid][words] when the bitmap does not fit shared memory
+  int* ws_cand;                // [grid][num_items]
+  unsigned long long* ws_key;  // [grid][num_items]
+  float* ws_val;               // [grid][num_items]
+  int words, bitmap_smem;
+  int stages;
+  long long stage_bytes;  // multiple of 16; 0 when there are no stages
+  int ch;                 // candidates per chunk (multiple of SR_THREADS, <= SR_KMAX * SR_THREADS)
+  unsigned long long* plan;
+};
+
+// how neighbour (w, d) is read for a chunk of cn candidates: streamed when its sketch moves fewer bytes than the
+// single counters (8*d*w < cn*d*32) -- whole when the sketch's enclosing 16-byte span fits a stage, else row by row
+// -- and gathered otherwise, or when even a row does not fit (the span of n cells is at most 8*n + 8 bytes)
+__device__ __forceinline__ int sr_mode(const SrArgs& a, int w, int d, int cn) {
+  if ((long long)w >= 4ll * cn) return SR_GATHER;
+  if ((long long)d * w * 8 + 8 <= a.stage_bytes) return SR_WHOLE;
+  if ((long long)w * 8 + 8 <= a.stage_bytes) return SR_ROWS;
+  return SR_TOO_WIDE;
+}
+
+// cp.async.bulk wants 16-byte-aligned addresses and sizes: the enclosing span of [src, src + n) is copied, and the
+// stage is read at the 8-byte skew of src
+__device__ __forceinline__ uint32_t span_bytes(const long long* src, long long n) {
+  return (uint32_t)((((uintptr_t)src & 15) + (uintptr_t)n * 8 + 15) & ~(uintptr_t)15);
+}
+__device__ __forceinline__ int span_skew(const long long* src) { return (int)(((uintptr_t)src & 15) >> 3); }
+
+__global__ void __launch_bounds__(SR_THREADS, 1) k_sized_recommend(const SrArgs a) {
+  extern __shared__ __align__(16) unsigned char sr_smem[];
+  // layout: [stages][stage_bytes] | full barriers [4] | scratch [8] | sort keys [REC_MAX_N] | residues [dmax][ch] |
+  // histogram [256] | scan [32] | bitmap [words] (when it fits)
+  unsigned char* p = sr_smem;
+  unsigned char* stage_base = p;
+  p += (size_t)a.stages * a.stage_bytes;
+  unsigned long long* full = reinterpret_cast<unsigned long long*>(p);
+  p += 8 * 4;
+  long long* bcast = reinterpret_cast<long long*>(p);
+  p += 8 * 8;
+  unsigned long long* sortbuf = reinterpret_cast<unsigned long long*>(p);
+  p += REC_MAX_N * 8;
+  unsigned long long* res = reinterpret_cast<unsigned long long*>(p);
+  p += (size_t)a.dmax * a.ch * 8;
+  unsigned* hist = reinterpret_cast<unsigned*>(p);
+  p += 256 * 4;
+  int* scan_sh = reinterpret_cast<int*>(p);
+  p += 32 * 4;
+  unsigned* bitmap_sh = reinterpret_cast<unsigned*>(p);
+
+  unsigned* bitmap = a.bitmap_smem ? bitmap_sh : a.ws_bitmap + (size_t)blockIdx.x * a.words;
+  int* cand = a.ws_cand + (size_t)blockIdx.x * a.num_items;
+  unsigned long long* keys = a.ws_key + (size_t)blockIdx.x * a.num_items;
+  float* vals = a.ws_val + (size_t)blockIdx.x * a.num_items;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+
+  if (tid == 0 && a.stages) {
+    for (int s = 0; s < a.stages; s++) tc05::mbar_init(tc05::smem_u32(&full[s]), 1);
+    tc05::mbar_fence_init();
+  }
+  __syncthreads();
+  uint32_t seq = 0;  // stage loads consumed by this CTA so far: stage = seq % stages, parity = (seq / stages) & 1
+
+  for (;;) {
+    if (tid == 0) bcast[0] = (long long)atomicAdd(&a.plan[RP_NEXT], 1ull);
+    __syncthreads();
+    const long long i = bcast[0];
+    __syncthreads();
+    if (i >= a.m) break;
+    long long* out_item = a.out_item + i * a.how_many;
+    float* out_value = a.out_value + i * a.how_many;
+    for (int t = tid; t < a.how_many; t += SR_THREADS) {
+      out_item[t] = -1;
+      out_value[t] = 0.0f;
+    }
+    const long long u = a.users[i];
+    const int cnt = a.nb_cnt[i];
+    if (u < 0 || u >= a.U || cnt < 0 || cnt > a.ld) {
+      if (tid == 0) {
+        atomicAdd(&a.plan[RP_BAD], 1ull);
+        a.out_cnt[i] = 0;
+      }
+      continue;
+    }
+    const long long* nbi = a.nb_idx + i * a.ld;
+    const double* nbs = a.nb_sim + i * a.ld;
+
+    // ---- 1. candidates: every index and range is checked before the load it guards --------------------------
+    for (int w = tid; w < a.words; w += SR_THREADS) bitmap[w] = 0u;
+    __syncthreads();
+    int bad = 0, c_eff = 0;
+    for (int j = warp; j < cnt; j += SR_THREADS / 32) {
+      const long long v = __ldg(nbi + j);
+      if (v < 0 || v >= a.U) {
+        bad += lane == 0;
+        continue;
+      }
+      const long long lo = __ldg(a.item_ptr + v), hi = __ldg(a.item_ptr + v + 1);
+      if (lo < 0 || hi < lo || hi > a.nnz) {
+        bad += lane == 0;
+        continue;
+      }
+      for (long long t = lo + lane; t < hi; t += 32) {
+        const int it = __ldg(a.item_col + t);
+        if (it < 0 || it >= a.num_items) bad++;
+        else atomicOr(&bitmap[it >> 5], 1u << (it & 31));
+      }
+    }
+    for (int j = tid; j < cnt; j += SR_THREADS) c_eff += __ldg(nbi + j) != u;
+    __syncthreads();
+    if (!a.include_known) {
+      const long long lo = a.item_ptr[u], hi = a.item_ptr[u + 1];
+      if (lo >= 0 && hi >= lo && hi <= a.nnz) {
+        for (long long t = lo + tid; t < hi; t += SR_THREADS) {
+          const int it = __ldg(a.item_col + t);
+          if (it < 0 || it >= a.num_items) bad++;
+          else atomicAnd(&bitmap[it >> 5], ~(1u << (it & 31)));
+        }
+      } else {
+        bad += tid == 0;
+      }
+    }
+    int tot_bad = 0, tot_c = 0;
+    block_exscan<SR_THREADS>(bad, scan_sh, &tot_bad);
+    block_exscan<SR_THREADS>(c_eff, scan_sh, &tot_c);
+    c_eff = tot_c;
+    if (tot_bad) {  // the neighbour lists or the data model are malformed: no estimates read through them
+      if (tid == 0) {
+        atomicAdd(&a.plan[RP_BAD], (unsigned long long)tot_bad);
+        a.out_cnt[i] = 0;
+      }
+      continue;
+    }
+    // compaction: thread tid owns a contiguous run of words (ascending dense order = ascending itemID)
+    const int per = (a.words + SR_THREADS - 1) / SR_THREADS;
+    const int w0 = tid * per, w1 = min(a.words, w0 + per);
+    int mine = 0;
+    for (int w = w0; w < w1; w++) mine += __popc(bitmap[w]);
+    int C = 0;
+    int at = block_exscan<SR_THREADS>(mine, scan_sh, &C);
+    for (int w = w0; w < w1; w++) {
+      unsigned b = bitmap[w];
+      while (b) {
+        const int k = __ffs(b) - 1;
+        b &= b - 1;
+        cand[at++] = w * 32 + k;
+      }
+    }
+    __syncthreads();  // cand[] is read by other threads below
+
+    // ---- 2. estimates, in chunks of candidates; each neighbour streamed or gathered by bytes ----------------
+    long long n_stream = 0, n_rows = 0, n_gather = 0, n_wide = 0, s_bytes = 0, g_loads = 0;  // thread 0's plan tallies
+    for (int c0 = 0; c0 < C; c0 += a.ch) {
+      const int cn = min(a.ch, C - c0);
+      const int kk = (cn + SR_THREADS - 1) / SR_THREADS;
+      for (int pos = tid; pos < cn; pos += SR_THREADS) {
+        const unsigned long long kr = cmh_residue(__ldg(a.item_ids + cand[c0 + pos]));
+        for (int r = 0; r < a.dmax; r++) res[(size_t)r * a.ch + pos] = mod_p(a.hf.a[r], a.hf.b[r], kr);
+      }
+      double pref[SR_KMAX], tot[SR_KMAX];
+      int count[SR_KMAX];
+      long long mn[SR_KMAX];
+#pragma unroll
+      for (int k = 0; k < SR_KMAX; k++) {
+        pref[k] = 0.0;
+        tot[k] = 0.0;
+        count[k] = 0;
+        mn[k] = 0;
+      }
+      __syncthreads();
+      // producer (thread 0): the next stage load of this chunk, in list order; nothing once the list is done
+      const int S = a.stages;
+      int pj = 0, pr = 0;
+      auto issue = [&](uint32_t slot_seq) {
+        for (; pj < cnt; pj++) {
+          const long long v = __ldg(nbi + pj);
+          if (v == u) continue;
+          const int mode = sr_mode(a, __ldg(a.W + v), __ldg(a.D + v), cn);
+          if (mode == SR_WHOLE || mode == SR_ROWS) break;
+        }
+        if (pj >= cnt) return;
+        const long long v = __ldg(nbi + pj);
+        const int w = __ldg(a.W + v), d = __ldg(a.D + v);
+        const bool whole = sr_mode(a, w, d, cn) == SR_WHOLE;
+        const long long* src = a.counters + __ldg(a.off + v) + (whole ? 0 : (size_t)pr * w);
+        const uint32_t bytes = span_bytes(src, whole ? (long long)d * w : w);
+        const int s = slot_seq % S;
+        const uint32_t bar = tc05::smem_u32(&full[s]);
+        tc05::mbar_expect_tx(bar, bytes);
+        bulk_row(tc05::smem_u32(stage_base + (size_t)s * a.stage_bytes),
+                 reinterpret_cast<const void*>((uintptr_t)src & ~(uintptr_t)15), bytes, bar);
+        s_bytes += bytes;
+        if (whole || ++pr == d) {
+          pr = 0;
+          pj++;
+        }
+      };
+      if (tid == 0)
+        for (int t = 0; t < S; t++) issue(seq + t);
+      for (int j = 0; j < cnt; j++) {
+        const long long v = __ldg(nbi + j);
+        if (v == u) continue;
+        const int w = __ldg(a.W + v), d = __ldg(a.D + v);
+        const unsigned uw = (unsigned)w;
+        const long long* sk = a.counters + __ldg(a.off + v);
+        const double sim = clamp_sim(__ldg(nbs + j));
+        const int mode = sr_mode(a, w, d, cn);
+        if (mode == SR_GATHER || mode == SR_TOO_WIDE) {
+#pragma unroll
+          for (int k = 0; k < SR_KMAX; k++) {
+            const int pos = tid + k * SR_THREADS;
+            if (k < kk && pos < cn) {
+              long long x = __ldg(sk + res[pos] % uw);
+              for (int r = 1; r < d; r++) {
+                const long long y = __ldg(sk + (size_t)r * w + res[(size_t)r * a.ch + pos] % uw);
+                x = y < x ? y : x;
+              }
+              nb_term(x, a.inv_q, sim, pref[k], tot[k], count[k]);
+            }
+          }
+          if (tid == 0) {
+            n_gather++;
+            n_wide += mode == SR_TOO_WIDE;
+            g_loads += (long long)cn * d;
+          }
+          continue;
+        }
+        const bool whole = mode == SR_WHOLE;
+        const int loads = whole ? 1 : d;
+        for (int r0 = 0; r0 < loads; r0++) {
+          const int s = seq % S;
+          tc05::mbar_wait(tc05::smem_u32(&full[s]), (seq / S) & 1u);
+          const long long* src = sk + (whole ? 0 : (size_t)r0 * w);
+          const long long* st = reinterpret_cast<const long long*>(stage_base + (size_t)s * a.stage_bytes) + span_skew(src);
+#pragma unroll
+          for (int k = 0; k < SR_KMAX; k++) {
+            const int pos = tid + k * SR_THREADS;
+            if (k < kk && pos < cn) {
+              if (whole) {
+                long long x = st[res[pos] % uw];
+                for (int r = 1; r < d; r++) {
+                  const long long y = st[(size_t)r * w + res[(size_t)r * a.ch + pos] % uw];
+                  x = y < x ? y : x;
+                }
+                mn[k] = x;
+              } else {
+                const long long x = st[res[(size_t)r0 * a.ch + pos] % uw];
+                mn[k] = (r0 == 0 || x < mn[k]) ? x : mn[k];
+              }
+            }
+          }
+          __syncthreads();  // every thread is done with stage s
+          if (tid == 0) issue(seq + S);
+          seq++;
+        }
+#pragma unroll
+        for (int k = 0; k < SR_KMAX; k++)
+          if (k < kk && tid + k * SR_THREADS < cn) nb_term(mn[k], a.inv_q, sim, pref[k], tot[k], count[k]);
+        n_stream += tid == 0;
+        n_rows += tid == 0 && !whole;
+      }
+#pragma unroll
+      for (int k = 0; k < SR_KMAX; k++) {
+        const int pos = tid + k * SR_THREADS;
+        if (k < kk && pos < cn) {
+          const float e = nb_result(pref[k], tot[k], count[k]);
+          vals[c0 + pos] = e;
+          keys[c0 + pos] = rank_key(e, c0 + pos);
+        }
+      }
+      __syncthreads();  // the residues are rewritten by the next chunk
+    }
+    if (tid == 0) {
+      const int nchunks = (C + a.ch - 1) / a.ch;
+      atomicAdd(&a.plan[RP_CHUNKS], (unsigned long long)nchunks);
+      atomicAdd(&a.plan[RP_CAND_SUM], (unsigned long long)C);
+      atomicMax(&a.plan[RP_CAND_MAX], (unsigned long long)C);
+      atomicAdd(&a.plan[RP_STREAM], (unsigned long long)n_stream);
+      atomicAdd(&a.plan[RP_ROWS], (unsigned long long)n_rows);
+      atomicAdd(&a.plan[RP_GATHER], (unsigned long long)n_gather);
+      atomicAdd(&a.plan[RP_TOO_WIDE], (unsigned long long)n_wide);
+      atomicAdd(&a.plan[RP_STREAM_BYTES], (unsigned long long)s_bytes);
+      atomicAdd(&a.plan[RP_GATHER_LOADS], (unsigned long long)g_loads);
+      atomicAdd(&a.plan[RP_TERMS], (unsigned long long)C * (unsigned long long)c_eff);
+    }
+
+    // ---- 3. top-N ------------------------------------------------------------------------------------------
+    const int n_out = topn_keys<SR_THREADS>(keys, C, a.how_many, hist, scan_sh, bcast, sortbuf);
+    for (int t = tid; t < n_out; t += SR_THREADS) {
+      const int pos = (int)(0xFFFFFFFFu - (uint32_t)sortbuf[t]);
+      out_item[t] = __ldg(a.item_ids + cand[pos]);
+      out_value[t] = vals[pos];
+    }
+    if (tid == 0) a.out_cnt[i] = n_out;
+    __syncthreads();
+  }
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -782,7 +1098,8 @@ int create_impl(mb200_ctx* ctx, int64_t U, const int32_t* width, const int32_t* 
   const int64_t nnz = bk->nnz;
   MB_CHECK(dev_alloc(ctx, &bk->off, (size_t)U + 1));
   MB_CHECK(dev_alloc(ctx, &bk->rowoff, (size_t)U + 1));
-  MB_CHECK(dev_alloc(ctx, &bk->counters, (size_t)bk->cells));
+  // two cells of padding: k_sized_recommend copies the enclosing 16-byte span of the last sketch
+  MB_CHECK(dev_alloc(ctx, &bk->counters, (size_t)bk->cells + 2));
   MB_CHECK(dev_alloc(ctx, &bk->sumsq, (size_t)bk->rows));
   MB_CHECK(dev_alloc(ctx, &bk->quanta, (size_t)nnz));
   MB_CHECK(dev_alloc(ctx, &bk->hres, (size_t)nnz * bk->dmax));
@@ -1118,6 +1435,149 @@ int mb200_sized_estimate_prefs(mb200_sized_bank* bk, const int64_t* nb_idx, cons
                       "mb200_sized_estimate_prefs: %llu user row(s), neighbourhood row(s), counts or neighbour "
                       "index(es) out of range (users %lld, neighbourhood rows %lld, nb_ld %d)",
                       h[SW_BAD], (long long)bk->U, (long long)nb_rows, nb_ld);
+  return MB200_OK;
+}
+
+int mb200_sized_recommend(mb200_sized_bank* bk, const int64_t* nb_idx, const double* nb_sim, const int32_t* nb_cnt,
+                          int32_t nb_ld, const int64_t* item_ptr, const int32_t* item_col, int64_t nnz,
+                          const int64_t* item_ids, int64_t num_items, const int64_t* users, int64_t m,
+                          int32_t how_many, int include_known, int64_t* out_item, float* out_value, int32_t* out_cnt,
+                          int mem) {
+  if (!bk) return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_sized_recommend: bank is NULL");
+  mb200_ctx* ctx = bk->ctx;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (how_many < 1 || how_many > REC_MAX_N)
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_recommend: how_many must be in [1, %d] (got %d)", REC_MAX_N,
+                      how_many);
+  if (m < 0 || nb_ld < 1 || nnz < 0 || num_items < 0 || num_items >= (1LL << 31) ||
+      (mem != MB200_MEM_HOST && mem != MB200_MEM_DEVICE))
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG,
+                      "mb200_sized_recommend: bad shape (m=%lld nb_ld=%d nnz=%lld num_items=%lld)", (long long)m, nb_ld,
+                      (long long)nnz, (long long)num_items);
+  if (m == 0) return MB200_OK;
+  if (!nb_idx || !nb_sim || !nb_cnt || !item_ptr || (nnz > 0 && !item_col) || (num_items > 0 && !item_ids) || !users ||
+      !out_item || !out_value || !out_cnt)
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_recommend: NULL array argument");
+  const int64_t U = bk->U;
+  if (mem == MB200_MEM_HOST) {
+    // the data model is host memory: its shape can be checked here
+    if (item_ptr[0] != 0 || item_ptr[U] != nnz)
+      return mb200_fail(ctx, MB200_ERR_BAD_ARG,
+                        "mb200_sized_recommend: item_ptr[0] must be 0 and item_ptr[users] = nnz (%lld)", (long long)nnz);
+    for (int64_t t = 1; t < num_items; t++)
+      if (item_ids[t] <= item_ids[t - 1])
+        return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_recommend: item_ids must be strictly ascending");
+  }
+  MB_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int dmax = bk->dmax > 0 ? bk->dmax : 1;
+  const long long words = (num_items + 31) / 32;
+  const bool bitmap_smem = words <= SR_BITMAP_SMEM_WORDS;
+  int ch = SR_RES_BYTES / (8 * dmax) / SR_THREADS * SR_THREADS;
+  ch = std::max(SR_THREADS, std::min(ch, SR_KMAX * SR_THREADS));
+  const size_t fixed = 8 * 4 + 8 * 8 + REC_MAX_N * 8 + (size_t)dmax * ch * 8 + 256 * 4 + 32 * 4 +
+                       (bitmap_smem ? (size_t)words * 4 : 0);
+  // the ring takes what shared memory is left, in SR_STAGES equal stages (MB200_SIZED_REC_STAGE_BYTES caps a stage:
+  // tests and A/B runs)
+  long long stage_bytes = ctx->smem_optin > fixed ? (long long)((ctx->smem_optin - fixed) / SR_STAGES) & ~15ll : 0;
+  if (const char* e = getenv("MB200_SIZED_REC_STAGE_BYTES"))
+    stage_bytes = std::min<long long>(stage_bytes, strtoll(e, nullptr, 10) & ~15ll);
+  const int stages = stage_bytes >= 32 ? SR_STAGES : 0;
+  if (!stages) stage_bytes = 0;
+  const size_t smem = fixed + (size_t)stages * stage_bytes;
+  const int grid = (int)std::min<int64_t>(m, ctx->num_sms);
+
+  SzStage st(ctx, mem);
+  SrArgs a;
+  a.W = bk->w;
+  a.D = bk->d;
+  a.off = bk->off;
+  a.counters = bk->counters;
+  a.hf = hash_of(bk);
+  a.dmax = dmax;
+  a.U = U;
+  a.inv_q = ldexp(1.0, -bk->frac_bits);
+  a.ld = nb_ld;
+  a.nnz = nnz;
+  a.num_items = num_items;
+  a.m = m;
+  a.how_many = how_many;
+  a.include_known = include_known != 0;
+  a.words = (int)words;
+  a.bitmap_smem = bitmap_smem;
+  a.stages = stages;
+  a.stage_bytes = stage_bytes;
+  a.ch = ch;
+  const size_t nbc = (size_t)m * nb_ld;
+  MB_CHECK(st.in((const long long*)nb_idx, nbc, &a.nb_idx));
+  MB_CHECK(st.in(nb_sim, nbc, &a.nb_sim));
+  MB_CHECK(st.in((const int*)nb_cnt, (size_t)m, &a.nb_cnt));
+  MB_CHECK(st.in((const long long*)item_ptr, (size_t)U + 1, &a.item_ptr));
+  MB_CHECK(st.in((const int*)item_col, (size_t)nnz, &a.item_col));
+  MB_CHECK(st.in((const long long*)item_ids, (size_t)num_items, &a.item_ids));
+  MB_CHECK(st.in((const long long*)users, (size_t)m, &a.users));
+  MB_CHECK(st.out((long long*)out_item, (size_t)m * how_many, &a.out_item));
+  MB_CHECK(st.out(out_value, (size_t)m * how_many, &a.out_value));
+  MB_CHECK(st.out((int*)out_cnt, (size_t)m, &a.out_cnt));
+  void *wb = nullptr, *wc = nullptr, *wk = nullptr, *wv = nullptr, *wp = nullptr;
+  const size_t per = (size_t)(num_items > 0 ? num_items : 1);
+  MB_CHECK(st.scratch(bitmap_smem ? 4 : (size_t)grid * words * 4, &wb));
+  MB_CHECK(st.scratch((size_t)grid * per * 4, &wc));
+  MB_CHECK(st.scratch((size_t)grid * per * 8, &wk));
+  MB_CHECK(st.scratch((size_t)grid * per * 4, &wv));
+  MB_CHECK(st.scratch(RP_WORDS * sizeof(unsigned long long), &wp));
+  MB_CUDA(ctx, cudaMemsetAsync(wp, 0, RP_WORDS * sizeof(unsigned long long), ctx->stream));
+  a.ws_bitmap = (unsigned*)wb;
+  a.ws_cand = (int*)wc;
+  a.ws_key = (unsigned long long*)wk;
+  a.ws_val = (float*)wv;
+  a.plan = (unsigned long long*)wp;
+  MB_CUDA(ctx, cudaFuncSetAttribute(k_sized_recommend, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  {
+    ProfScope prof(ctx, MB200_K_RECOMMEND);
+    k_sized_recommend<<<grid, SR_THREADS, smem, ctx->stream>>>(a);
+  }
+  ctx->launches++;
+  MB_CUDA(ctx, cudaGetLastError());
+  MB_CHECK(st.finish());
+  unsigned long long h[RP_WORDS];
+  MB_CUDA(ctx, cudaMemcpyAsync(h, wp, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  mb200_sized_recommend_plan& pl = ctx->last_sized_recommend_plan;
+  pl.users = m;
+  pl.chunks = (int64_t)h[RP_CHUNKS];
+  pl.candidates = (int64_t)h[RP_CAND_SUM];
+  pl.candidates_max = (int64_t)h[RP_CAND_MAX];
+  pl.stream_visits = (int64_t)h[RP_STREAM];
+  pl.row_visits = (int64_t)h[RP_ROWS];
+  pl.gather_visits = (int64_t)h[RP_GATHER];
+  pl.too_wide_visits = (int64_t)h[RP_TOO_WIDE];
+  pl.stream_bytes = (int64_t)h[RP_STREAM_BYTES];
+  pl.gather_loads = (int64_t)h[RP_GATHER_LOADS];
+  pl.terms = (int64_t)h[RP_TERMS];
+  pl.stages = stages;
+  pl.stage_bytes = (int32_t)stage_bytes;
+  pl.chunk_candidates = ch;
+  if (getenv("MB200_TRACE"))
+    fprintf(stderr,
+            "[mb200 trace] sized recommend plan: users=%lld chunks=%lld candidates=%lld max=%lld stream=%lld "
+            "rows=%lld gather=%lld too_wide=%lld stream_bytes=%lld gather_loads=%lld terms=%lld stages=%d stage_bytes=%lld "
+            "chunk=%d bitmap=%s\n",
+            (long long)m, (long long)pl.chunks, (long long)pl.candidates, (long long)pl.candidates_max,
+            (long long)pl.stream_visits, (long long)pl.row_visits, (long long)pl.gather_visits, (long long)pl.too_wide_visits,
+            (long long)pl.stream_bytes, (long long)pl.gather_loads, (long long)pl.terms, stages, stage_bytes, ch,
+            bitmap_smem ? "smem" : "global");
+  if (h[RP_BAD])
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG,
+                      "mb200_sized_recommend: %llu user row(s), neighbour count(s) or index(es), item_ptr range(s) or "
+                      "item_col entr(ies) out of range (users %lld, num_items %lld, nnz %lld, nb_ld %d)",
+                      h[RP_BAD], (long long)U, (long long)num_items, (long long)nnz, nb_ld);
+  return MB200_OK;
+}
+
+int mb200_sized_recommend_last_plan(mb200_ctx* ctx, mb200_sized_recommend_plan* out) {
+  if (!ctx || !out) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_recommend_last_plan: NULL argument");
+  std::lock_guard<std::mutex> g(ctx->mu);
+  *out = ctx->last_sized_recommend_plan;
   return MB200_OK;
 }
 

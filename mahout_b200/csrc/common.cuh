@@ -73,6 +73,7 @@ struct mb200_ctx {
   mb200_recommend_plan last_recommend_plan = {};  // mb200_recommend_last_plan
   mb200_itembased_plan last_itembased_plan = {};  // mb200_itembased_last_plan
   mb200_sized_plan last_sized_plan = {};          // mb200_sized_last_plan
+  mb200_sized_recommend_plan last_sized_recommend_plan = {};  // mb200_sized_recommend_last_plan
   int64_t itembased_dense_items = -1, itembased_dense_slices = -1;  // layout of the zeroed dense slices (slot 62)
 };
 

@@ -17,23 +17,28 @@ import numpy as np
 from .cosinecm import CosineCM
 
 
+def _item_csr(cm: CosineCM, device: int):
+    """the data model as K_RECOMMEND takes it, on the device: the items each user row rated, CSR by user row
+    (item_ptr [U+1], item_col int32), items as dense numbers of item_ids (ascending itemIDs)"""
+    import torch
+    rows = np.searchsorted(cm.user_ids, cm._u_sorted)
+    item_ids = np.unique(cm._i_sorted)
+    col = np.searchsorted(item_ids, cm._i_sorted)
+    pairs = np.unique(rows.astype(np.int64) * item_ids.shape[0] + col)   # a user's item set
+    prow, pcol = pairs // item_ids.shape[0], pairs % item_ids.shape[0]
+    ptr = np.zeros(cm.user_ids.shape[0] + 1, np.int64)
+    np.cumsum(np.bincount(prow, minlength=cm.user_ids.shape[0]), out=ptr[1:])
+    return tuple(torch.from_numpy(np.ascontiguousarray(a)).to(f"cuda:{device}")
+                 for a in (ptr, pcol.astype(np.int32), item_ids))
+
+
 class GenericUserBasedRecommender:
     def __init__(self, cm: CosineCM, neighborhood_size: int, min_similarity: float | None = None):
-        import torch
         self.cm = cm
         self.bank = cm.bank
         self.neighborhood_size = int(neighborhood_size)
-        dev = f"cuda:{self.bank.ctx.device}"
-        # the data model: the items each user row rated, CSR by user row, items as dense numbers of item_ids
-        rows = np.searchsorted(cm.user_ids, cm._u_sorted)
-        self.item_ids = np.unique(cm._i_sorted)
-        col = np.searchsorted(self.item_ids, cm._i_sorted)
-        pairs = np.unique(rows.astype(np.int64) * self.item_ids.shape[0] + col)   # a user's item set
-        prow, pcol = pairs // self.item_ids.shape[0], pairs % self.item_ids.shape[0]
-        ptr = np.zeros(cm.user_ids.shape[0] + 1, np.int64)
-        np.cumsum(np.bincount(prow, minlength=cm.user_ids.shape[0]), out=ptr[1:])
-        self._csr = tuple(torch.from_numpy(np.ascontiguousarray(a)).to(dev)
-                          for a in (ptr, pcol.astype(np.int32), self.item_ids))
+        self._csr = _item_csr(cm, self.bank.ctx.device)
+        self.item_ids = self._csr[2].cpu().numpy()
         self.nb_idx, self.nb_sim, self.nb_cnt = self.bank.cosine_topk(
             self.neighborhood_size, threshold=min_similarity, exclude_self=True, precision="rescored", device=True)
 
@@ -73,13 +78,15 @@ class PerUserConfigUserBasedRecommender:
     user's sketch at its own size (CosineCM.sized_bank), similarities as CosineCM.userSimilarity computes them (user 1
     re-sketched at user 2's size), NearestNUserNeighborhood(n, min_similarity) exactly -- NaN never admitted,
     negative similarities admitted when they pass min_similarity, ties by lower user row -- and doEstimatePreference
-    point-querying each neighbour's own sketch.  All in K_RECOMMEND (csrc/cmsized.cu)."""
+    point-querying each neighbour's own sketch; recommend() ranks the neighbours' items by those estimates.  All in
+    K_RECOMMEND (csrc/cmsized.cu)."""
 
     def __init__(self, cm: CosineCM, n: int, min_similarity: float = float("-inf")):
         self.cm = cm
         self.bank = cm.sized_bank()
         self.n = int(n)
         self.min_similarity = float(min_similarity)
+        self._csr = None   # the data model for recommend(), built on first use
 
     def _dev(self):
         return f"cuda:{self.bank.ctx.device}"
@@ -105,3 +112,23 @@ class PerUserConfigUserBasedRecommender:
         items = torch.from_numpy(np.ascontiguousarray(np.atleast_1d(itemIDs), np.int64)).to(dev)
         return self.bank.estimate_prefs(idx, sim, cnt, torch.from_numpy(rows).to(dev), items,
                                         nb_row=torch.from_numpy(inv.astype(np.int64)).to(dev)).cpu().numpy()
+
+    def recommend_all(self, howMany: int, userIDs=None, includeKnownItems: bool = False):
+        """(user_ids [m], items [m, howMany] itemIDs (-1 unused), values [m, howMany] float32, counts [m]): each
+        user's neighbourhood, then GenericUserBasedRecommender.recommend over it -- NaN estimates dropped, ranked by
+        (value desc, itemID asc); negative and infinite estimates (negative similarities) rank by value"""
+        import torch
+        user_ids = self.cm.user_ids if userIDs is None else np.atleast_1d(np.asarray(userIDs, np.int64))
+        rows = np.arange(self.cm.user_ids.shape[0], dtype=np.int64) if userIDs is None else self.cm._rows(user_ids)
+        if self._csr is None:
+            self._csr = _item_csr(self.cm, self.bank.ctx.device)
+        rows_d = torch.from_numpy(rows).to(self._dev())
+        idx, sim, cnt = self.bank.neighborhood(rows_d, self.n, self.min_similarity)
+        items, vals, c = self.bank.recommend(idx, sim, cnt, *self._csr, rows_d, howMany, includeKnownItems)
+        return user_ids, items.cpu().numpy(), vals.cpu().numpy(), c.cpu().numpy()
+
+    def recommend(self, userID: int, howMany: int, includeKnownItems: bool = False):
+        """list of (itemID, value), best first"""
+        _, items, vals, cnt = self.recommend_all(howMany, [userID], includeKnownItems)
+        n = int(cnt[0])
+        return [(int(i), float(v)) for i, v in zip(items[0, :n], vals[0, :n])]

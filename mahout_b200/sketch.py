@@ -602,6 +602,40 @@ class SizedBank:
                                                    nr.ptr, it.ptr, u.n, optr, mem), self.ctx.handle)
         return out
 
+    def recommend(self, nb_idx, nb_sim, nb_cnt, item_ptr, item_col, item_ids, users, how_many: int,
+                  include_known: bool = False):
+        """GenericUserBasedRecommender.recommend for the user rows `users`, row t of the lists (nb_idx / nb_sim
+        [m, ld], nb_cnt [m], as neighborhood(users) returns them) being users[t]'s neighbourhood; every estimate is
+        estimate_prefs()'s.  Data model as CSR over user rows (item_ptr [U+1], item_col = dense item numbers into
+        item_ids, strictly ascending itemIDs).  Returns (items [m, how_many] int64, values [m, how_many] float32,
+        counts [m] int32); unused slots are -1 / 0."""
+        ni = _Arg(nb_idx, np.int64, "int64")
+        ns = _Arg(nb_sim, np.float64, "float64")
+        nc = _Arg(nb_cnt, np.int32, "int32")
+        ip = _Arg(item_ptr, np.int64, "int64")
+        ic = _Arg(item_col, np.int32, "int32")
+        ii = _Arg(item_ids, np.int64, "int64")
+        us = _Arg(users, np.int64, "int64")
+        m, n = us.n, int(how_many)
+        ld = ni.n // m if m else 1
+        if nc.n != m or ni.n != m * ld or ns.n != ni.n or ip.n != self.U + 1:
+            raise ValueError("nb_idx / nb_sim must be [m, ld] and nb_cnt [m] for the m users; item_ptr [U + 1] for "
+                             "the bank's U rows")
+        mem = _same_mem(ni, ns, nc, ip, ic, ii, us)
+        items, pi = _out((m, max(n, 0)), np.int64, "int64", mem, self.ctx.device)
+        vals, pv = _out((m, max(n, 0)), np.float32, "float32", mem, self.ctx.device)
+        cnt, pc = _out((m,), np.int32, "int32", mem, self.ctx.device)
+        N.check(N.lib().mb200_sized_recommend(self.handle, ni.ptr, ns.ptr, nc.ptr, max(ld, 1), ip.ptr, ic.ptr, ic.n,
+                                              ii.ptr, ii.n, us.ptr, m, n, int(bool(include_known)), pi, pv, pc, mem),
+                self.ctx.handle)
+        return items, vals, cnt
+
+    def recommend_plan(self) -> dict:
+        """what the last recommend() on this bank's context did (mb200_sized_recommend_last_plan)"""
+        pl = N.SizedRecommendPlan()
+        N.check(N.lib().mb200_sized_recommend_last_plan(self.ctx.handle, C.byref(pl)), self.ctx.handle)
+        return {f: getattr(pl, f) for f, _ in N.SizedRecommendPlan._fields_}
+
     def plan(self) -> dict:
         """what the last neighborhood() on this bank's context did (mb200_sized_last_plan)"""
         pl = N.SizedPlan()

@@ -13,6 +13,13 @@ Per call: time (best of --repeats, device-synchronised, after one warm-up call),
 over candidate users v != query of d_v * w_v), FMA/s, the plan (mb200_sized_last_plan) and bit parity of the lists
 with orc_sized_neighborhood on --parity sampled queries.  Prints one JSON line with the GPU's name and power limit.
 --dry prints the shape model only (no GPU).
+
+Recommend leg (config3, --recommend-populations): recommend(user, 10) over the users' n = 100 neighbourhoods
+(mb200_sized_recommend) for the 4096 sampled users, then all users.  Per call: time (best of --repeats after a
+warm-up, device-synchronised), users/s, neighbour terms/s (sum over users of candidates x listed neighbours other than
+the user), the plan (mb200_sized_recommend_last_plan), the bytes model (streamed bytes + 32 B per gathered counter)
+over the time as a share of 7.7 TB/s of HBM, the neighbourhood time of the same users beside it, and bit parity with
+oracle.sized_recommend on --parity sampled users.
 """
 from __future__ import annotations
 
@@ -100,6 +107,8 @@ def main():
     ap.add_argument("--repeats", type=int, default=3)
     ap.add_argument("--all-zipf", action="store_true", help="also time all users on the zipf population")
     ap.add_argument("--dry", action="store_true", help="shape model only, no GPU")
+    ap.add_argument("--recommend-populations", default="config3", help="populations of the recommend leg ('' = none)")
+    ap.add_argument("--how-many", type=int, default=10)
     args = ap.parse_args()
     out = {"tool": "cmsized_perf", "n": N_NB, "q": 1.0}
     if not args.dry:
@@ -120,6 +129,8 @@ def main():
             rec["calls"][label] = {"queries": int(qrows.shape[0]), "pair_fmas": fmas}
         if not args.dry:
             run(rec, name, w, d, ptr, item, pref, calls, args)
+            if name in args.recommend_populations.split(","):
+                run_recommend(rec, w, d, ptr, item, pref, calls, args)
         out[name] = rec
         print(json.dumps({name: rec}), file=sys.stderr, flush=True)
     print(json.dumps(out))
@@ -158,6 +169,59 @@ def run(rec, name, w, d, ptr, item, pref, calls, args):
         gi, gs, gc = (x.cpu().numpy()[pick] for x in res)
         c["parity_queries"] = int(pick.shape[0])
         c["parity"] = bool((gc == oc).all() and (gi == oi).all() and gs.tobytes() == osim.tobytes())
+    bank.close()
+    ctx.close()
+
+
+HBM_BYTES_PER_S = 7.7e12   # HGX B200 data sheet, one GPU
+
+
+def run_recommend(rec, w, d, ptr, item, pref, calls, args):
+    import torch
+    import mahout_b200 as mb
+    from oracle import recommend as orec
+    from oracle.sized_recommend import sized_recommend
+    ctx = mb.Context(0)
+    dev = f"cuda:{ctx.device}"
+    U = w.shape[0]
+    bank = mb.SizedBank(w, d, mb.HashFunctionBuilder(SEED), ptr, item, pref, 1, ctx)
+    data = orec.item_csr(np.repeat(np.arange(U), np.diff(ptr)), item, U)
+    data_d = [torch.from_numpy(np.ascontiguousarray(x)).to(dev) for x in data]
+    rec["recommend"] = {}
+    for label, qrows in calls:
+        c = {"users": int(qrows.shape[0]), "how_many": args.how_many}
+        q = torch.from_numpy(qrows).to(dev)
+        t = time.perf_counter()
+        lists = bank.neighborhood(q, N_NB)
+        torch.cuda.synchronize(ctx.device)
+        c["neighborhood_s"] = time.perf_counter() - t
+        res = bank.recommend(*lists, *data_d, q, args.how_many)        # warm-up
+        torch.cuda.synchronize(ctx.device)
+        best = float("inf")
+        for _ in range(args.repeats):
+            t = time.perf_counter()
+            res = bank.recommend(*lists, *data_d, q, args.how_many)
+            torch.cuda.synchronize(ctx.device)
+            best = min(best, time.perf_counter() - t)
+        pl = bank.recommend_plan()
+        c["time_s"] = best
+        c["users_per_s"] = qrows.shape[0] / best
+        c["terms_per_s"] = pl["terms"] / best
+        c["plan"] = pl
+        c["model_bytes"] = pl["stream_bytes"] + 32 * pl["gather_loads"]
+        c["hbm_share"] = c["model_bytes"] / best / HBM_BYTES_PER_S
+        pick = np.sort(np.random.Generator(np.random.PCG64(SEED + 9)).choice(qrows.shape[0], min(args.parity,
+                                                                                                qrows.shape[0]),
+                                                                             replace=False))
+        idx, sim, cnt = (x.cpu().numpy()[pick] for x in lists)
+        t = time.perf_counter()
+        wi, wv, wc = sized_recommend(w, d, bank.a, bank.b, ptr, item, pref, idx, sim, cnt, *data, qrows[pick],
+                                     args.how_many)
+        c["oracle_s"] = time.perf_counter() - t
+        gi, gv, gc = (x.cpu().numpy()[pick] for x in res)
+        c["parity_users"] = int(pick.shape[0])
+        c["parity"] = bool((gc == wc).all() and (gi == wi).all() and gv.tobytes() == wv.tobytes())
+        rec["recommend"][label] = c
     bank.close()
     ctx.close()
 
