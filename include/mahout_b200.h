@@ -598,7 +598,9 @@ int mb200_cosine_last_fallback_rows(mb200_ctx* ctx, int64_t* rows);
 /* ---- the whole item-similarity phase, on one GPU or on all GPUs of the box ------------------------------- */
 /* One process drives n_gpus GPUs: one mb200_ctx and one host worker thread per GPU, peer access between all of
  * them (SURVEY.md 8b: `mb200_create(int n_gpus, ...)`).  devices may be NULL (GPUs 0 .. n_gpus-1); n_gpus == 0
- * takes every visible GPU.  This is what a JVM binds for `--numGpus`. */
+ * takes every visible GPU.  An explicit list may name a device more than once: that device gets one context per
+ * entry (no peer access is needed between them), and n_gpus is bounded by MB200_MAX_BLOCKS, not by the visible
+ * GPUs.  This is what a JVM binds for `--numGpus`. */
 typedef struct mb200_multi mb200_multi;
 int mb200_create_multi(int32_t n_gpus, const int32_t* devices, mb200_multi** out);
 int mb200_multi_destroy(mb200_multi* m);
@@ -638,6 +640,42 @@ typedef struct mb200_job_stats {
 int mb200_job_item_similarity(mb200_multi* m, const int64_t* row, const int64_t* key, const float* inc, int64_t n,
                               int64_t num_items, const mb200_job_params* p, int64_t* out_idx, double* out_sim,
                               int32_t* out_cnt, mb200_job_stats* stats);
+
+/* ---- CosineCM with a CountMinSketchConfig on all GPUs of m: one sized-bank replica per GPU --------------------- */
+/* mb200_sized_multi_create builds one full mb200_sized_bank on every GPU of m, all GPUs in parallel, from the same
+ * HOST arrays (mb200_sized_bank_create's meaning).  Each replica costs what one sized bank costs: counters
+ * (cells + 2) * 8 B, sums of squares rows * 8 B, quanta nnz * 8 B, hash residues nnz * max(depth) * 8 B, and 36 B per
+ * user of shapes and offsets.  The calls below take and return HOST arrays in the caller's order and split the work
+ * by user: query position t goes to GPU t mod G; estimates go by user, the j-th distinct user row (ascending) to GPU
+ * j mod G with every pair of that user.  Results are bit-identical to the single-context calls for any G (floats,
+ * NaN slots, counts, unused slots -1 / 0).  NULL arrays, q or m < 0, n outside [1, 1024], how_many outside [1, 1024],
+ * a NaN min_similarity or a malformed item CSR fail with MB200_ERR_BAD_ARG before any GPU work; a device-found error
+ * fails the call with the first failing GPU's code and "GPU d: <message>" (mb200_multi_last_error).  The handle stays
+ * usable after a failed call.  One call at a time per mb200_multi: every call holds m's lock. */
+typedef struct mb200_sized_multi mb200_sized_multi;
+int mb200_sized_multi_create(mb200_multi* m, int64_t users, const int32_t* width, const int32_t* depth,
+                             const int64_t* a, const int64_t* b, int32_t frac_bits, const int64_t* user_ptr,
+                             const int64_t* item, const float* pref, mb200_sized_multi** out);
+int mb200_sized_multi_destroy(mb200_sized_multi* sm);
+/* mb200_sized_neighborhood's contract: out_idx / out_sim [q][n], out_cnt [q] */
+int mb200_sized_multi_neighborhood(mb200_sized_multi* sm, const int64_t* query_rows, int64_t q, int32_t n,
+                                   double min_similarity, int64_t* out_idx, double* out_sim, int32_t* out_cnt);
+/* recommend(user, how_many) for the m user rows: each GPU computes its users' neighbourhoods (n, min_similarity)
+ * and runs mb200_sized_recommend over them; the lists never leave that GPU.  The data model as there: item_ptr
+ * [users + 1], item_col [nnz], item_ids [num_items] strictly ascending.  out_item / out_value [m][how_many],
+ * out_cnt [m]. */
+int mb200_sized_multi_recommend(mb200_sized_multi* sm, const int64_t* users, int64_t m, int32_t n,
+                                double min_similarity, const int64_t* item_ptr, const int32_t* item_col, int64_t nnz,
+                                const int64_t* item_ids, int64_t num_items, int32_t how_many, int include_known,
+                                int64_t* out_item, float* out_value, int32_t* out_cnt);
+/* doEstimatePreference for the q pairs (user[t], item_id[t]) over each user's neighbourhood (n, min_similarity),
+ * each distinct user's neighbourhood computed once: mb200_sized_estimate_prefs's values, float32 out [q] */
+int mb200_sized_multi_estimate_prefs(mb200_sized_multi* sm, const int64_t* user, const int64_t* item_id, int64_t q,
+                                     int32_t n, double min_similarity, float* out);
+/* the last call on sm (create included): work[g] = queries (pairs for estimates, users for create) given to GPU g,
+ * seconds[g] = host wall clock of GPU g's worker, wall_s = the call's wall clock.  work and seconds have
+ * mb200_multi_gpus entries; any pointer may be NULL. */
+int mb200_sized_multi_last_stats(mb200_sized_multi* sm, int64_t* work, double* seconds, double* wall_s);
 
 #ifdef __cplusplus
 }

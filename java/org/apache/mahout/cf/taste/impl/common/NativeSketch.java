@@ -184,6 +184,35 @@ public final class NativeSketch {
                                            long[] itemPtr, int[] itemCol, long[] itemIds, long[] users, int howMany,
                                            boolean includeKnown, long[] outItem, float[] outValue, int[] outCnt);
 
+  /**
+   * mb200_sized_multi_create / mb200_sized_multi_destroy: createSizedBank's inputs, one replica of the sized bank on
+   * every GPU of a createMulti handle (--numGpus), built in parallel.  The calls below split their users between the
+   * GPUs (query position t to GPU t mod G; estimates by distinct user) and return what the single-GPU calls return,
+   * bit for bit, in the caller's order.  Destroy the sized handle before its multi handle.
+   */
+  public static native long createSizedMulti(long multi, int[] width, int[] depth, long[] a, long[] b, int fracBits,
+                                             long[] userPtr, long[] item, float[] pref);
+  public static native void destroySizedMulti(long sizedMulti);
+
+  /** mb200_sized_multi_neighborhood: sizedNeighborhood over all GPUs; outIdx / outSim [queries][n], outCnt [queries]. */
+  public static native void sizedMultiNeighborhood(long sizedMulti, long[] queryRows, int n, double minSimilarity,
+                                                   long[] outIdx, double[] outSim, int[] outCnt);
+
+  /**
+   * mb200_sized_multi_recommend: each user's sizedNeighborhood(n, minSimilarity), then sizedRecommend over it on the
+   * GPU that computed it (the lists never leave that GPU).  outItem / outValue [users][howMany], outCnt [users].
+   */
+  public static native void sizedMultiRecommend(long sizedMulti, long[] users, int n, double minSimilarity,
+                                                long[] itemPtr, int[] itemCol, long[] itemIds, int howMany,
+                                                boolean includeKnown, long[] outItem, float[] outValue, int[] outCnt);
+
+  /**
+   * mb200_sized_multi_estimate_prefs: doEstimatePreference for the (user row, itemID) pairs user[t], itemId[t] over
+   * each user's sizedNeighborhood(n, minSimilarity), each distinct user's computed once; out[t] NaN = no estimate.
+   */
+  public static native void sizedMultiEstimatePrefs(long sizedMulti, long[] user, long[] itemId, int n,
+                                                    double minSimilarity, float[] out);
+
   /** mb200_host_alloc / mb200_host_free wrapped as a direct ByteBuffer. */
   public static native ByteBuffer allocPinned(long bytes);
   public static native void freePinned(ByteBuffer buffer);

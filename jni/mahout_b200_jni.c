@@ -499,3 +499,107 @@ JNIEXPORT void JNICALL JNI_FN(sizedRecommend)(JNIEnv* env, jclass c, jlong bank,
   (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
   CHECK(rc, NULL);
 }
+
+/* ---- the sized bank on all GPUs of the process (csrc/sized_multi.cu) ------------------------------------------- */
+JNIEXPORT jlong JNICALL JNI_FN(createSizedMulti)(JNIEnv* env, jclass c, jlong multi, jintArray width, jintArray depth,
+                                                 jlongArray a, jlongArray b, jint fracBits, jlongArray userPtr,
+                                                 jlongArray item, jfloatArray pref) {
+  mb200_multi* m = (mb200_multi*)(intptr_t)multi;
+  mb200_sized_multi* sm = NULL;
+  const jsize users = (*env)->GetArrayLength(env, width);
+  jint* pw = (*env)->GetIntArrayElements(env, width, NULL);
+  jint* pd = (*env)->GetIntArrayElements(env, depth, NULL);
+  jlong* pa = (*env)->GetLongArrayElements(env, a, NULL);
+  jlong* pb = (*env)->GetLongArrayElements(env, b, NULL);
+  jlong* pp = (*env)->GetLongArrayElements(env, userPtr, NULL);
+  jlong* pi = (*env)->GetLongArrayElements(env, item, NULL);
+  jfloat* pv = (*env)->GetFloatArrayElements(env, pref, NULL);
+  int rc = (*env)->GetArrayLength(env, depth) != users || (*env)->GetArrayLength(env, userPtr) != users + 1 ||
+                   (*env)->GetArrayLength(env, pref) != (*env)->GetArrayLength(env, item) ||
+                   (users > 0 && pp[users] != (*env)->GetArrayLength(env, item))
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_multi_create(m, users, (const int32_t*)pw, (const int32_t*)pd, (const int64_t*)pa,
+                                          (const int64_t*)pb, fracBits, (const int64_t*)pp, (const int64_t*)pi,
+                                          (const float*)pv, &sm);
+  (*env)->ReleaseIntArrayElements(env, width, pw, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, depth, pd, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, a, pa, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, b, pb, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, userPtr, pp, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, item, pi, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, pref, pv, JNI_ABORT);
+  if (rc != MB200_OK) throw_multi(env, rc, m);
+  return (jlong)(intptr_t)sm;
+}
+
+JNIEXPORT void JNICALL JNI_FN(destroySizedMulti)(JNIEnv* env, jclass c, jlong sizedMulti) {
+  mb200_sized_multi_destroy((mb200_sized_multi*)(intptr_t)sizedMulti);
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedMultiNeighborhood)(JNIEnv* env, jclass c, jlong sizedMulti, jlongArray queryRows,
+                                                      jint n, jdouble minSimilarity, jlongArray outIdx,
+                                                      jdoubleArray outSim, jintArray outCnt) {
+  const jsize q = (*env)->GetArrayLength(env, queryRows);
+  jlong* pq = (*env)->GetLongArrayElements(env, queryRows, NULL);
+  jlong* oi = (*env)->GetLongArrayElements(env, outIdx, NULL);
+  jdouble* os = (*env)->GetDoubleArrayElements(env, outSim, NULL);
+  jint* oc = (*env)->GetIntArrayElements(env, outCnt, NULL);
+  int rc = (*env)->GetArrayLength(env, outCnt) != q || (int64_t)(*env)->GetArrayLength(env, outIdx) != (int64_t)q * n ||
+                   (*env)->GetArrayLength(env, outSim) != (*env)->GetArrayLength(env, outIdx)
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_multi_neighborhood((mb200_sized_multi*)(intptr_t)sizedMulti, (const int64_t*)pq, q, n,
+                                                minSimilarity, (int64_t*)oi, os, (int32_t*)oc);
+  (*env)->ReleaseLongArrayElements(env, queryRows, pq, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outIdx, oi, 0);
+  (*env)->ReleaseDoubleArrayElements(env, outSim, os, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
+  if (rc != MB200_OK) throw_multi(env, rc, NULL);  /* the calling thread's message: "GPU d: ..." */
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedMultiRecommend)(JNIEnv* env, jclass c, jlong sizedMulti, jlongArray users, jint n,
+                                                   jdouble minSimilarity, jlongArray itemPtr, jintArray itemCol,
+                                                   jlongArray itemIds, jint howMany, jboolean includeKnown,
+                                                   jlongArray outItem, jfloatArray outValue, jintArray outCnt) {
+  jlong* pu = (*env)->GetLongArrayElements(env, users, NULL);
+  jlong* pp = (*env)->GetLongArrayElements(env, itemPtr, NULL);
+  jint* pl = (*env)->GetIntArrayElements(env, itemCol, NULL);
+  jlong* pd = (*env)->GetLongArrayElements(env, itemIds, NULL);
+  jlong* oi = (*env)->GetLongArrayElements(env, outItem, NULL);
+  jfloat* ov = (*env)->GetFloatArrayElements(env, outValue, NULL);
+  jint* oc = (*env)->GetIntArrayElements(env, outCnt, NULL);
+  const jsize m = (*env)->GetArrayLength(env, users);
+  int rc = (*env)->GetArrayLength(env, outCnt) != m ||
+                   (int64_t)(*env)->GetArrayLength(env, outItem) != (int64_t)m * howMany ||
+                   (*env)->GetArrayLength(env, outValue) != (*env)->GetArrayLength(env, outItem)
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_multi_recommend((mb200_sized_multi*)(intptr_t)sizedMulti, (const int64_t*)pu, m, n,
+                                             minSimilarity, (const int64_t*)pp, (const int32_t*)pl,
+                                             (*env)->GetArrayLength(env, itemCol), (const int64_t*)pd,
+                                             (*env)->GetArrayLength(env, itemIds), howMany, includeKnown, (int64_t*)oi,
+                                             (float*)ov, (int32_t*)oc);
+  (*env)->ReleaseLongArrayElements(env, users, pu, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemPtr, pp, JNI_ABORT);
+  (*env)->ReleaseIntArrayElements(env, itemCol, pl, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemIds, pd, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, outItem, oi, 0);
+  (*env)->ReleaseFloatArrayElements(env, outValue, ov, 0);
+  (*env)->ReleaseIntArrayElements(env, outCnt, oc, 0);
+  if (rc != MB200_OK) throw_multi(env, rc, NULL);
+}
+
+JNIEXPORT void JNICALL JNI_FN(sizedMultiEstimatePrefs)(JNIEnv* env, jclass c, jlong sizedMulti, jlongArray user,
+                                                       jlongArray itemId, jint n, jdouble minSimilarity,
+                                                       jfloatArray out) {
+  const jsize q = (*env)->GetArrayLength(env, user);
+  jlong* pu = (*env)->GetLongArrayElements(env, user, NULL);
+  jlong* pt = (*env)->GetLongArrayElements(env, itemId, NULL);
+  jfloat* po = (*env)->GetFloatArrayElements(env, out, NULL);
+  int rc = (*env)->GetArrayLength(env, itemId) != q || (*env)->GetArrayLength(env, out) != q
+               ? MB200_ERR_BAD_ARG
+               : mb200_sized_multi_estimate_prefs((mb200_sized_multi*)(intptr_t)sizedMulti, (const int64_t*)pu,
+                                                  (const int64_t*)pt, q, n, minSimilarity, (float*)po);
+  (*env)->ReleaseLongArrayElements(env, user, pu, JNI_ABORT);
+  (*env)->ReleaseLongArrayElements(env, itemId, pt, JNI_ABORT);
+  (*env)->ReleaseFloatArrayElements(env, out, po, 0);
+  if (rc != MB200_OK) throw_multi(env, rc, NULL);
+}

@@ -229,6 +229,12 @@ _PROTOS = {
     "mb200_multi_ctx": (C.c_int, [vp, i32, C.POINTER(vp)]),
     "mb200_multi_last_error": (C.c_char_p, [vp]),
     "mb200_job_item_similarity": (C.c_int, [vp, vp, vp, vp, i64, i64, C.POINTER(JobParams), vp, vp, vp, C.POINTER(JobStats)]),
+    "mb200_sized_multi_create": (C.c_int, [vp, i64, vp, vp, vp, vp, i32, vp, vp, vp, C.POINTER(vp)]),
+    "mb200_sized_multi_destroy": (C.c_int, [vp]),
+    "mb200_sized_multi_neighborhood": (C.c_int, [vp, vp, i64, i32, f64, vp, vp, vp]),
+    "mb200_sized_multi_recommend": (C.c_int, [vp, vp, i64, i32, f64, vp, vp, i64, vp, i64, i32, C.c_int, vp, vp, vp]),
+    "mb200_sized_multi_estimate_prefs": (C.c_int, [vp, vp, vp, i64, i32, f64, vp]),
+    "mb200_sized_multi_last_stats": (C.c_int, [vp, vp, vp, C.POINTER(f64)]),
     # bench / test support (mahout_b200/csrc/synth.h)
     "mb200_synth_events": (C.c_int, [vp, C.c_uint64, i64, i64, i64, vp, i64, vp, vp, vp, vp]),
     "mb200_bench_red64": (C.c_int, [vp, i64, i64, C.POINTER(f64), C.POINTER(f64)]),

@@ -81,29 +81,39 @@ class CosineCM:
         cm.update(items, prefs)
         return cm
 
+    def sized_model(self):
+        """the inputs of a sized bank, host arrays: every user row's (width, depth) from `config`, shaped as `new
+        DoubleCountMinSketch(delta, epsilon, hfb)` shapes it (cm_dims of the stored parameters, never best_dims),
+        and the prefs as CSR by user row -- (width [U] int32, depth [U] int32, user_ptr [U+1], item, pref float32)"""
+        if self.config is None:
+            raise ValueError("no CountMinSketchConfig was given")
+        dims = {}
+        w = np.empty(self.user_ids.shape[0], np.int32)
+        d = np.empty(self.user_ids.shape[0], np.int32)
+        for r, u in enumerate(self.user_ids.tolist()):
+            key = (self.config.getDelta(u), self.config.getEpsilon(u))
+            if key not in dims:
+                try:
+                    dims[key] = sk.cm_dims(*key)
+                except sk.N.CMException as e:    # CosineCM.java:45-47 wraps it in a TasteException
+                    raise RuntimeError(f"CountMinSketch error:{e}") from e
+            w[r], d[r] = dims[key]
+        ptr = np.zeros(self.user_ids.shape[0] + 1, np.int64)
+        np.cumsum(np.bincount(np.searchsorted(self.user_ids, self._u_sorted), minlength=self.user_ids.shape[0]),
+                  out=ptr[1:])
+        return w, d, ptr, self._i_sorted, self._p_sorted.astype(np.float32)
+
     def sized_bank(self) -> sk.SizedBank:
-        """every user's sketch at its own (delta, epsilon) from `config`, shaped as `new DoubleCountMinSketch(delta,
-        epsilon, hfb)` shapes it (cm_dims of the stored parameters, never best_dims); built on first use"""
+        """every user's sketch at its own (delta, epsilon) from `config` (sized_model); built on first use"""
         if self._sized is None:
-            if self.config is None:
-                raise ValueError("no CountMinSketchConfig was given")
-            dims = {}
-            w = np.empty(self.user_ids.shape[0], np.int32)
-            d = np.empty(self.user_ids.shape[0], np.int32)
-            for r, u in enumerate(self.user_ids.tolist()):
-                key = (self.config.getDelta(u), self.config.getEpsilon(u))
-                if key not in dims:
-                    try:
-                        dims[key] = sk.cm_dims(*key)
-                    except sk.N.CMException as e:    # CosineCM.java:45-47 wraps it in a TasteException
-                        raise RuntimeError(f"CountMinSketch error:{e}") from e
-                w[r], d[r] = dims[key]
-            ptr = np.zeros(self.user_ids.shape[0] + 1, np.int64)
-            np.cumsum(np.bincount(np.searchsorted(self.user_ids, self._u_sorted), minlength=self.user_ids.shape[0]),
-                      out=ptr[1:])
-            self._sized = sk.SizedBank(w, d, self._hfb, ptr, self._i_sorted, self._p_sorted.astype(np.float32),
-                                       self._frac_bits, self.bank.ctx)
+            w, d, ptr, item, pref = self.sized_model()
+            self._sized = sk.SizedBank(w, d, self._hfb, ptr, item, pref, self._frac_bits, self.bank.ctx)
         return self._sized
+
+    def multi_sized_bank(self, multi):
+        """sized_bank() replicated on every GPU of a MultiGpu (mahout_b200.multi.MultiSizedBank)"""
+        w, d, ptr, item, pref = self.sized_model()
+        return multi.sized_bank(w, d, self._hfb, ptr, item, pref, self._frac_bits)
 
     def userSimilaritiesPerUserConfig(self, ids1, ids2) -> np.ndarray:
         """CosineCM.userSimilarity exactly as written (:84-96) for the pairs (ids1[t], ids2[t]): user 1's prefs

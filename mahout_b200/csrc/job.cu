@@ -19,19 +19,10 @@
 // Host threads meet at barriers between the steps that read another GPU's memory.
 #include <string.h>
 
-#include <chrono>
 #include <condition_variable>
 #include <thread>
 
-#include "common.cuh"
-
-struct mb200_multi {
-  int n = 0;
-  std::vector<int> devices;
-  std::vector<mb200_ctx*> ctx;
-  std::string err;
-  std::mutex mu;
-};
+#include "multi.cuh"
 
 namespace {
 
@@ -52,10 +43,6 @@ struct HostBarrier {
     }
   }
 };
-
-double now_s() {
-  return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count();
-}
 
 struct Shared {
   mb200_multi* m;
@@ -112,7 +99,7 @@ void worker(Shared& sh, int g) {
   cudaSetDevice(ctx->device);
   const int64_t s0 = sh.n * g / G, s1 = sh.n * (g + 1) / G, ns = s1 - s0;
   void *d_row = nullptr, *d_key = nullptr, *d_inc = nullptr;
-  const double t0 = now_s();
+  const double t0 = multi_now_s();
   // ---- slice + count
   if (ns > 0) {
     JOB_CUDA(cudaMalloc(&d_row, (size_t)ns * 8));
@@ -148,8 +135,8 @@ void worker(Shared& sh, int g) {
     JOB_TRY(mb200_sync(ctx));
   }
   sh.bar.wait();
-  if (g == 0) sh.t_route = now_s() - t0;
-  const double t1 = now_s();
+  if (g == 0) sh.t_route = multi_now_s() - t0;
+  const double t1 = multi_now_s();
   // ---- build the shard bank
   mb200_bank* bank = nullptr;
   if (!sh.failed()) {
@@ -175,8 +162,8 @@ void worker(Shared& sh, int g) {
     cudaFree(sh.r_inc[g]);
   }
   mb200_release_workspace(ctx);  // the grouping workspaces: 20 B per event
-  if (g == 0) sh.t_build = now_s() - t1;
-  const double t2 = now_s();
+  if (g == 0) sh.t_build = multi_now_s() - t1;
+  const double t2 = multi_now_s();
   const int k = P.k;
   const int64_t E = sh.E_loc;
   void *o_idx = nullptr, *o_sim = nullptr, *o_cnt = nullptr;
@@ -328,13 +315,7 @@ void worker(Shared& sh, int g) {
   if (bank) mb200_bank_destroy(bank);
   mb200_release_workspace(ctx);
   sh.bar.wait();
-  if (g == 0) sh.t_cosine = now_s() - t2;
-}
-
-int multi_fail(mb200_multi* m, int code, const std::string& msg) {
-  if (m) m->err = msg;
-  mb200_set_global_error(msg.c_str());
-  return code;
+  if (g == 0) sh.t_cosine = multi_now_s() - t2;
 }
 
 }  // namespace
@@ -350,8 +331,12 @@ int mb200_create_multi(int32_t n_gpus, const int32_t* devices, mb200_multi** out
     return mb200_fail(nullptr, MB200_ERR_NO_DEVICE, "mb200_create_multi: no CUDA device (%s); this library has no CPU fallback",
                       e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
   if (n_gpus == 0) n_gpus = have;  // all GPUs of the box
-  if (n_gpus < 0 || n_gpus > have || n_gpus > MB200_MAX_BLOCKS)
+  // an explicit list may name a device more than once (several contexts on it); without one, GPUs 0 .. n_gpus-1
+  if (n_gpus < 0 || (!devices && n_gpus > have) || n_gpus > MB200_MAX_BLOCKS)
     return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_create_multi: %d GPUs asked for, %d visible", n_gpus, have);
+  for (int g = 0; devices && g < n_gpus; g++)
+    if (devices[g] < 0 || devices[g] >= have)
+      return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_create_multi: device %d out of range [0, %d)", devices[g], have);
   mb200_multi* m = new mb200_multi();
   m->n = n_gpus;
   for (int g = 0; g < n_gpus; g++) m->devices.push_back(devices ? devices[g] : g);
@@ -369,7 +354,7 @@ int mb200_create_multi(int32_t n_gpus, const int32_t* devices, mb200_multi** out
   for (int a = 0; a < n_gpus; a++) {
     cudaSetDevice(m->devices[a]);
     for (int b = 0; b < n_gpus; b++) {
-      if (a == b) continue;
+      if (m->devices[a] == m->devices[b]) continue;  // a device listed twice reaches its own memory
       int can = 0;
       cudaDeviceCanAccessPeer(&can, m->devices[a], m->devices[b]);
       if (!can) {

@@ -4,6 +4,9 @@ Mirror of what a JVM does through JNI for `--numGpus`: `MultiGpu(n)` is `mb200_c
 is `mb200_job_item_similarity` = phase 1 of ItemSimilarityJob.run (ItemSimilarityJob.java:146-162).  The
 one-process-per-GPU path over torch.distributed (similarity.sharded_item_similarity) computes the same thing for
 callers that already run one rank per GPU.
+
+`sized_bank` is CosineCM with a CountMinSketchConfig on every GPU of the handle (csrc/sized_multi.cu): one
+replica of the sized bank per GPU, query users split t mod G, results bit-identical to `SizedBank`'s.
 """
 from __future__ import annotations
 
@@ -12,7 +15,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
-from .sketch import _DTYPES, _PRECISIONS
+from .sketch import _DTYPES, _PRECISIONS, HashFunctionBuilder, IdentityHashBuilder
 
 
 class MultiGpu:
@@ -28,6 +31,7 @@ class MultiGpu:
         n = C.c_int32()
         N.lib().mb200_multi_gpus(h, C.byref(n))
         self.n_gpus = n.value
+        self.devices = dv.tolist() if dv is not None else list(range(self.n_gpus))
 
     def close(self):
         if getattr(self, "_h", None) is not None:
@@ -86,3 +90,119 @@ class MultiGpu:
             cnt.ctypes.data_as(C.c_void_p), C.byref(st)))
         del keep
         return idx, sim, cnt, {f: getattr(st, f) for f, _ in N.JobStats._fields_}
+
+    def sized_bank(self, width, depth, hfBuilder, user_ptr, item, pref, frac_bits: int = 1) -> "MultiSizedBank":
+        """SizedBank's inputs (host arrays): one replica of the sized bank on every GPU of this handle"""
+        return MultiSizedBank(self, width, depth, hfBuilder, user_ptr, item, pref, frac_bits)
+
+    def contexts(self):
+        """the raw mb200_ctx handles of the GPUs, in order (launch counts, stats)"""
+        out = []
+        for g in range(self.n_gpus):
+            h = C.c_void_p()
+            N.lib().mb200_multi_ctx(self._h, g, C.byref(h))
+            out.append(h)
+        return out
+
+
+def _host(a, dtype):
+    if hasattr(a, "cpu"):
+        a = a.cpu().numpy()
+    return np.ascontiguousarray(np.atleast_1d(np.asarray(a)), dtype)
+
+
+def _p(a):
+    return a.ctypes.data_as(C.c_void_p)
+
+
+class MultiSizedBank:
+    """CosineCM's per-user-sized sketches replicated on every GPU of a MultiGpu (mb200_sized_multi_*).  Each call
+    splits its users between the GPUs -- query position t to GPU t mod G; estimates by distinct user -- and returns
+    numpy arrays in the caller's order, bit-identical to the same SizedBank calls on one GPU."""
+
+    def __init__(self, multi: MultiGpu, width, depth, hfBuilder, user_ptr, item, pref, frac_bits: int = 1):
+        self.multi = multi
+        if not isinstance(hfBuilder, (HashFunctionBuilder, IdentityHashBuilder)):
+            hfBuilder = HashFunctionBuilder(int(hfBuilder))
+        self.width = _host(width, np.int32)
+        self.depth = _host(depth, np.int32)
+        if self.width.shape != self.depth.shape:
+            raise ValueError("width and depth must be 1-d arrays of one entry per user")
+        dmax = int(self.depth.max()) if self.depth.size else 1
+        if not (0 < dmax <= N.MAX_DEPTH):
+            raise ValueError(f"depth must be in (0, {N.MAX_DEPTH}] (got {dmax})")
+        self.a, self.b = hfBuilder.params(dmax)
+        ptr, it, pr = _host(user_ptr, np.int64), _host(item, np.int64), _host(pref, np.float32)
+        if ptr.shape[0] != self.width.shape[0] + 1 or it.shape != pr.shape:
+            raise ValueError("user_ptr must have users + 1 entries; item and pref the same length")
+        self.U, self.frac_bits = int(self.width.shape[0]), int(frac_bits)
+        h = C.c_void_p()
+        self._h = None
+        multi._check(N.lib().mb200_sized_multi_create(multi._h, self.U, _p(self.width), _p(self.depth), _p(self.a),
+                                                      _p(self.b), self.frac_bits, _p(ptr), _p(it), _p(pr), C.byref(h)))
+        self._h = h
+
+    @property
+    def handle(self):
+        if self._h is None:
+            raise ValueError("bank is closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and getattr(self.multi, "_h", None) is not None:
+            try:
+                N.lib().mb200_sized_multi_destroy(self._h)
+            except Exception:   # interpreter shutdown
+                pass
+        self._h = None
+
+    __del__ = close
+
+    def neighborhood(self, query_rows, n: int, min_similarity: float = -np.inf):
+        """SizedBank.neighborhood over all GPUs: (idx [q, n] int64, sim [q, n] float64, cnt [q] int32)"""
+        q = _host(query_rows, np.int64)
+        n = int(n)
+        idx = np.empty((q.shape[0], max(n, 0)), np.int64)
+        sim = np.empty((q.shape[0], max(n, 0)), np.float64)
+        cnt = np.empty(q.shape[0], np.int32)
+        self.multi._check(N.lib().mb200_sized_multi_neighborhood(self.handle, _p(q), q.shape[0], n,
+                                                                 float(min_similarity), _p(idx), _p(sim), _p(cnt)))
+        return idx, sim, cnt
+
+    def recommend_users(self, users, n: int, min_similarity: float, item_ptr, item_col, item_ids, how_many: int,
+                        include_known: bool = False):
+        """each user's neighbourhood(n, min_similarity), then SizedBank.recommend over it, on the GPU that computed
+        it: (items [m, how_many] int64, values [m, how_many] float32, counts [m] int32), unused slots -1 / 0"""
+        us = _host(users, np.int64)
+        ip, ic, ii = _host(item_ptr, np.int64), _host(item_col, np.int32), _host(item_ids, np.int64)
+        if ip.shape[0] != self.U + 1:
+            raise ValueError("item_ptr must be [U + 1] for the bank's U rows")
+        m, h = us.shape[0], int(how_many)
+        items = np.empty((m, max(h, 0)), np.int64)
+        vals = np.empty((m, max(h, 0)), np.float32)
+        cnt = np.empty(m, np.int32)
+        self.multi._check(N.lib().mb200_sized_multi_recommend(
+            self.handle, _p(us), m, int(n), float(min_similarity), _p(ip), _p(ic), ic.shape[0], _p(ii), ii.shape[0], h,
+            int(bool(include_known)), _p(items), _p(vals), _p(cnt)))
+        return items, vals, cnt
+
+    def estimate_prefs(self, user, item_id, n: int, min_similarity: float = -np.inf):
+        """doEstimatePreference for the pairs (user[t], item_id[t]) over each user's neighbourhood(n,
+        min_similarity); float32 [q], NaN where there is no estimate"""
+        u, it = _host(user, np.int64), _host(item_id, np.int64)
+        if u.shape != it.shape:
+            raise ValueError("user and item_id must have the same length")
+        out = np.empty(u.shape[0], np.float32)
+        self.multi._check(N.lib().mb200_sized_multi_estimate_prefs(self.handle, _p(u), _p(it), u.shape[0], int(n),
+                                                                   float(min_similarity), _p(out)))
+        return out
+
+    def stats(self) -> dict:
+        """the last call: {"work": queries (pairs for estimates) per GPU, "seconds": each GPU's worker wall clock,
+        "wall_s": the call's wall clock}"""
+        G = self.multi.n_gpus
+        work = np.zeros(G, np.int64)
+        secs = np.zeros(G, np.float64)
+        wall = C.c_double()
+        self.multi._check(N.lib().mb200_sized_multi_last_stats(self.handle, _p(work), _p(secs), C.byref(wall)))
+        return {"work": work.tolist(), "seconds": secs.tolist(), "wall_s": wall.value}
