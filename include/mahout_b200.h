@@ -111,8 +111,8 @@ int mb200_launch_count(mb200_ctx* ctx, int64_t* launches);
 typedef struct mb200_stats {
   int32_t device, num_sms;
   int64_t launches;            /* kernels launched since creation */
-  int64_t workspace_bytes;     /* grow-only device workspaces of the cosine stage */
-  int64_t staging_bytes;       /* device staging of host-memory arguments and events */
+  int64_t workspace_bytes;     /* grow-only device workspaces: the cosine stage's and every other call's scratch */
+  int64_t staging_bytes;       /* grow-only device staging of host-memory arguments, results and K1 events */
   int64_t last_fallback_rows;  /* rows of the last cosine call that took the exact full-row path */
   int32_t cosine_job_active;
   char device_name[64];

@@ -922,68 +922,6 @@ __global__ void __launch_bounds__(SR_THREADS, 1) k_sized_recommend(const SrArgs 
 // ---------------------------------------------------------------------------------------------------------------
 // host helpers
 // ---------------------------------------------------------------------------------------------------------------
-// grow-only slots 80.. of ctx->ws_group hold this file's staging and scratch
-constexpr size_t SLOT_SW = 80, SLOT_IN = 81;
-
-struct SzStage {
-  mb200_ctx* ctx;
-  int mem;
-  size_t next = SLOT_IN;
-  std::vector<std::pair<void*, std::pair<void*, size_t>>> outs;
-  SzStage(mb200_ctx* c, int m) : ctx(c), mem(m) {}
-  template <typename T>
-  int in(const T* user, size_t n, const T** dev) {
-    next++;
-    if (mem == MB200_MEM_DEVICE || !user) {
-      *dev = user;
-      return MB200_OK;
-    }
-    void* p = nullptr;
-    MB_CHECK(mb200_group_ws(ctx, next, n * sizeof(T), &p));
-    if (n) MB_CUDA(ctx, cudaMemcpyAsync(p, user, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-    ctx->stat_h2d += (int64_t)(n * sizeof(T));
-    *dev = (const T*)p;
-    return MB200_OK;
-  }
-  template <typename T>
-  int out(T* user, size_t n, T** dev) {
-    next++;
-    if (mem == MB200_MEM_DEVICE) {
-      *dev = user;
-      return MB200_OK;
-    }
-    void* p = nullptr;
-    MB_CHECK(mb200_group_ws(ctx, next, n * sizeof(T), &p));
-    outs.push_back({p, {(void*)user, n * sizeof(T)}});
-    *dev = (T*)p;
-    return MB200_OK;
-  }
-  int scratch(size_t bytes, void** p) { return mb200_group_ws(ctx, ++next, bytes, p); }
-  int finish() {
-    for (auto& o : outs) {
-      if (o.second.second)
-        MB_CUDA(ctx, cudaMemcpyAsync(o.second.first, o.first, o.second.second, cudaMemcpyDeviceToHost, ctx->stream));
-      ctx->stat_d2h += (int64_t)o.second.second;
-    }
-    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return MB200_OK;
-  }
-};
-
-int status_words(mb200_ctx* ctx, unsigned long long** sw) {
-  void* p = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, SLOT_SW, SW_WORDS * sizeof(unsigned long long), &p));
-  MB_CUDA(ctx, cudaMemsetAsync(p, 0, SW_WORDS * sizeof(unsigned long long), ctx->stream));
-  *sw = (unsigned long long*)p;
-  return MB200_OK;
-}
-
-int read_words(mb200_ctx* ctx, const unsigned long long* sw, unsigned long long* h) {
-  MB_CUDA(ctx, cudaMemcpyAsync(h, sw, SW_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return MB200_OK;
-}
-
 SizedDev dev_view(const mb200_sized_bank* bk) {
   SizedDev v;
   v.W = bk->w;
@@ -1043,14 +981,14 @@ int create_impl(mb200_ctx* ctx, int64_t U, const int32_t* width, const int32_t* 
   MB_CUDA(ctx, cudaMemcpyAsync(bk->w, width, (size_t)U * 4, cudaMemcpyDefault, ctx->stream));
   MB_CUDA(ctx, cudaMemcpyAsync(bk->d, depth, (size_t)U * 4, cudaMemcpyDefault, ctx->stream));
   MB_CUDA(ctx, cudaMemcpyAsync(bk->ptr, user_ptr, ((size_t)U + 1) * 8, cudaMemcpyDefault, ctx->stream));
-  unsigned long long* sw = nullptr;
-  MB_CHECK(status_words(ctx, &sw));
+  StatusWords sw(ctx, SW_WORDS);
+  MB_CHECK(sw.zero(WS_STATUS));
   k_sized_validate<<<(unsigned)std::min<int64_t>(ceil_div64(U + 1, 256), 4096), 256, 0, ctx->stream>>>(
-      bk->w, bk->d, bk->ptr, U, sw);
+      bk->w, bk->d, bk->ptr, U, sw.dev);
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
   unsigned long long h[SW_WORDS];
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   if (h[SW_BAD])
     return mb200_fail(ctx, MB200_ERR_BAD_ARG,
                       "mb200_sized_bank_create: %llu width(s) < 1, depth(s) outside [1, %d] or user_ptr entries not "
@@ -1110,23 +1048,23 @@ int create_impl(mb200_ctx* ctx, int64_t U, const int32_t* width, const int32_t* 
   MB_CUDA(ctx, cudaMemsetAsync(bk->counters, 0, (size_t)bk->cells * 8, ctx->stream));
   // the prefs only pass through workspace slots on their way into quanta / hash residues
   void *ditem = nullptr, *dpref = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, SLOT_IN, (size_t)(nnz ? nnz : 1) * 8, &ditem));
-  MB_CHECK(mb200_group_ws(ctx, SLOT_IN + 1, (size_t)(nnz ? nnz : 1) * 4, &dpref));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_ITEM, (size_t)(nnz ? nnz : 1) * 8, &ditem));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_PREF, (size_t)(nnz ? nnz : 1) * 4, &dpref));
   if (nnz) {
     MB_CUDA(ctx, cudaMemcpyAsync(ditem, item, (size_t)nnz * 8, cudaMemcpyDefault, ctx->stream));
     MB_CUDA(ctx, cudaMemcpyAsync(dpref, pref, (size_t)nnz * 4, cudaMemcpyDefault, ctx->stream));
   }
-  MB_CHECK(status_words(ctx, &sw));
+  MB_CHECK(sw.zero(WS_STATUS));
   if (U > 0) {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
     k_sized_build<<<(unsigned)U, SZ_THREADS, 0, ctx->stream>>>(bk->w, bk->d, bk->off, bk->rowoff, bk->ptr,
                                                                (const long long*)ditem, (const float*)dpref, nnz,
                                                                bk->dmax, hash_of(bk), ldexp(1.0, frac_bits),
-                                                               bk->counters, bk->sumsq, bk->quanta, bk->hres, sw);
+                                                               bk->counters, bk->sumsq, bk->quanta, bk->hres, sw.dev);
   }
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   if (h[SW_INEXACT])
     return mb200_fail(ctx, MB200_ERR_INEXACT,
                       "%llu increment(s) are not multiples of 2^-%d (or not finite): the bank cannot hold them "
@@ -1207,7 +1145,7 @@ int mb200_sized_pair_cosine(mb200_sized_bank* bk, const int64_t* u1, const int64
   if (n == 0) return MB200_OK;
   if (!u1 || !u2 || !out) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_pair_cosine: NULL array argument");
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  SzStage st(ctx, mem);
+  ArgStage st(ctx, mem);
   const long long *d1, *d2;
   double* dout;
   MB_CHECK(st.in((const long long*)u1, (size_t)n, &d1));
@@ -1217,19 +1155,19 @@ int mb200_sized_pair_cosine(mb200_sized_bank* bk, const int64_t* u1, const int64
   int64_t grid = std::min<int64_t>(n, (int64_t)ctx->num_sms * 2);
   grid = std::max<int64_t>(1, std::min<int64_t>(grid, (int64_t)(SZ_DENSE / ((size_t)slice * 8))));
   void* slices = nullptr;
-  MB_CHECK(st.scratch((size_t)grid * slice * 8, &slices));
-  unsigned long long* sw = nullptr;
-  MB_CHECK(status_words(ctx, &sw));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_SLICE, (size_t)grid * slice * 8, &slices));
+  StatusWords sw(ctx, SW_WORDS);
+  MB_CHECK(sw.zero(WS_STATUS));
   {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
     k_sized_pair<<<(unsigned)grid, SZ_THREADS, 0, ctx->stream>>>(dev_view(bk), d1, d2, n, (long long*)slices, slice,
-                                                                  dout, sw);
+                                                                  dout, sw.dev);
   }
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[SW_WORDS];
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   if (h[SW_BAD])
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_pair_cosine: %llu user row(s) outside [0, %lld)", h[SW_BAD],
                       (long long)bk->U);
@@ -1255,7 +1193,7 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
   if (!query_rows || !out_idx || !out_sim || !out_cnt)
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_neighborhood: NULL array argument");
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  SzStage st(ctx, mem);
+  ArgStage st(ctx, mem);
   const long long* dq;
   long long* didx;
   double* dsim;
@@ -1264,13 +1202,14 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
   MB_CHECK(st.out((long long*)out_idx, (size_t)q * n, &didx));
   MB_CHECK(st.out(out_sim, (size_t)q * n, &dsim));
   MB_CHECK(st.out((int*)out_cnt, (size_t)q, &dcnt));
-  unsigned long long* sw = nullptr;
-  MB_CHECK(status_words(ctx, &sw));
-  k_sized_check_rows<<<(unsigned)std::min<int64_t>(ceil_div64(q, 256), 4096), 256, 0, ctx->stream>>>(dq, q, bk->U, sw);
+  StatusWords sw(ctx, SW_WORDS);
+  MB_CHECK(sw.zero(WS_STATUS));
+  k_sized_check_rows<<<(unsigned)std::min<int64_t>(ceil_div64(q, 256), 4096), 256, 0, ctx->stream>>>(dq, q, bk->U,
+                                                                                                       sw.dev);
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
   unsigned long long h[SW_WORDS];
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   if (h[SW_BAD])
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_neighborhood: %llu query row(s) outside [0, %lld)", h[SW_BAD],
                       (long long)bk->U);
@@ -1306,9 +1245,9 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
   const int grid = ctx->num_sms * 2;
   const size_t smem = (size_t)SZ_TQ * 32 * 8 + qsmem_used;
   void *wsims = nullptr, *wslice = nullptr, *wcls = nullptr, *witems = nullptr;
-  MB_CHECK(st.scratch((size_t)qb * std::max<int64_t>(U, 1) * 8, &wsims));
-  MB_CHECK(st.scratch(global_classes ? (size_t)grid * slice_cells * 8 : 8, &wslice));
-  MB_CHECK(st.scratch((size_t)std::max(C, 1) * 4 * 4, &wcls));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_SIMS, (size_t)qb * std::max<int64_t>(U, 1) * 8, &wsims));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_SLICE, global_classes ? (size_t)grid * slice_cells * 8 : 8, &wslice));
+  MB_CHECK(ws_slot(ctx, WS_SIZED_CLASSES, (size_t)std::max(C, 1) * 4 * 4, &wcls));
   std::vector<int> hcls((size_t)std::max(C, 1) * 4);
   for (int c = 0; c < C; c++) {
     hcls[c] = bk->cw[c];
@@ -1329,10 +1268,10 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
           items.push_back({c, (int)m0, (int)std::min<int64_t>(cmem[c], bk->cptr[c + 1] - m0), (int)t0});
     // the staging slot of the items is refilled per batch: the previous batch must be done with it
     MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    MB_CHECK(mb200_group_ws(ctx, SLOT_IN + 20, std::max<size_t>(items.size(), 1) * sizeof(SzItem), &witems));
+    MB_CHECK(ws_slot(ctx, WS_SIZED_ITEMS, std::max<size_t>(items.size(), 1) * sizeof(SzItem), &witems));
     MB_CUDA(ctx, cudaMemcpyAsync(witems, items.data(), items.size() * sizeof(SzItem), cudaMemcpyHostToDevice,
                                  ctx->stream));
-    MB_CUDA(ctx, cudaMemsetAsync(sw + SW_NEXT, 0, 8, ctx->stream));
+    MB_CUDA(ctx, cudaMemsetAsync(sw.dev + SW_NEXT, 0, 8, ctx->stream));
     ScoreArgs a;
     a.b = dev_view(bk);
     a.members = bk->members;
@@ -1347,7 +1286,7 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
     a.sims = (double*)wsims;
     a.gslice = (long long*)wslice;
     a.slice_cells = slice_cells;
-    a.sw = sw;
+    a.sw = sw.dev;
     {
       ProfScope prof(ctx, MB200_K_RECOMMEND);
       k_sized_score<<<grid, SZ_THREADS, smem, ctx->stream>>>(a);
@@ -1365,7 +1304,7 @@ int mb200_sized_neighborhood(mb200_sized_bank* bk, const int64_t* query_rows, in
     n_items_total += (int64_t)items.size();
   }
   MB_CHECK(st.finish());
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   mb200_sized_plan& pl = ctx->last_sized_plan;
   pl.queries = q;
   pl.classes = C;
@@ -1403,7 +1342,7 @@ int mb200_sized_estimate_prefs(mb200_sized_bank* bk, const int64_t* nb_idx, cons
   if (!user || !item_id || !out || (nb_rows > 0 && (!nb_idx || !nb_sim || !nb_cnt)))
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_sized_estimate_prefs: NULL array argument");
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  SzStage st(ctx, mem);
+  ArgStage st(ctx, mem);
   const long long *d_idx, *d_user, *d_row, *d_item;
   const double* d_sim;
   const int* d_cnt;
@@ -1416,20 +1355,20 @@ int mb200_sized_estimate_prefs(mb200_sized_bank* bk, const int64_t* nb_idx, cons
   MB_CHECK(st.in((const long long*)nb_row, nb_row ? (size_t)q : 0, &d_row));
   MB_CHECK(st.in((const long long*)item_id, (size_t)q, &d_item));
   MB_CHECK(st.out(out, (size_t)q, &d_out));
-  unsigned long long* sw = nullptr;
-  MB_CHECK(status_words(ctx, &sw));
+  StatusWords sw(ctx, SW_WORDS);
+  MB_CHECK(sw.zero(WS_STATUS));
   const int dmax = bk->dmax > 0 ? bk->dmax : 1;
   {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
     k_sized_estimate<<<(unsigned)ceil_div64(q, EST_THREADS), EST_THREADS, (size_t)dmax * EST_THREADS * 8, ctx->stream>>>(
         dev_view(bk), hash_of(bk), bk->dmax, ldexp(1.0, -bk->frac_bits), d_idx, d_sim, d_cnt, nb_rows, nb_ld, d_user,
-        d_row, d_item, q, d_out, sw);
+        d_row, d_item, q, d_out, sw.dev);
   }
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[SW_WORDS];
-  MB_CHECK(read_words(ctx, sw, h));
+  MB_CHECK(sw.read(h));
   if (h[SW_BAD])
     return mb200_fail(ctx, MB200_ERR_BAD_ARG,
                       "mb200_sized_estimate_prefs: %llu user row(s), neighbourhood row(s), counts or neighbour "
@@ -1486,7 +1425,7 @@ int mb200_sized_recommend(mb200_sized_bank* bk, const int64_t* nb_idx, const dou
   const size_t smem = fixed + (size_t)stages * stage_bytes;
   const int grid = (int)std::min<int64_t>(m, ctx->num_sms);
 
-  SzStage st(ctx, mem);
+  ArgStage st(ctx, mem);
   SrArgs a;
   a.W = bk->w;
   a.D = bk->d;
@@ -1518,19 +1457,19 @@ int mb200_sized_recommend(mb200_sized_bank* bk, const int64_t* nb_idx, const dou
   MB_CHECK(st.out((long long*)out_item, (size_t)m * how_many, &a.out_item));
   MB_CHECK(st.out(out_value, (size_t)m * how_many, &a.out_value));
   MB_CHECK(st.out((int*)out_cnt, (size_t)m, &a.out_cnt));
-  void *wb = nullptr, *wc = nullptr, *wk = nullptr, *wv = nullptr, *wp = nullptr;
+  void *wb = nullptr, *wc = nullptr, *wk = nullptr, *wv = nullptr;
   const size_t per = (size_t)(num_items > 0 ? num_items : 1);
-  MB_CHECK(st.scratch(bitmap_smem ? 4 : (size_t)grid * words * 4, &wb));
-  MB_CHECK(st.scratch((size_t)grid * per * 4, &wc));
-  MB_CHECK(st.scratch((size_t)grid * per * 8, &wk));
-  MB_CHECK(st.scratch((size_t)grid * per * 4, &wv));
-  MB_CHECK(st.scratch(RP_WORDS * sizeof(unsigned long long), &wp));
-  MB_CUDA(ctx, cudaMemsetAsync(wp, 0, RP_WORDS * sizeof(unsigned long long), ctx->stream));
+  MB_CHECK(ws_slot(ctx, WS_REC_BITMAP, bitmap_smem ? 4 : (size_t)grid * words * 4, &wb));
+  MB_CHECK(ws_slot(ctx, WS_REC_CAND, (size_t)grid * per * 4, &wc));
+  MB_CHECK(ws_slot(ctx, WS_REC_KEY, (size_t)grid * per * 8, &wk));
+  MB_CHECK(ws_slot(ctx, WS_REC_VAL, (size_t)grid * per * 4, &wv));
+  StatusWords plan(ctx, RP_WORDS);
+  MB_CHECK(plan.zero(WS_STATUS));
   a.ws_bitmap = (unsigned*)wb;
   a.ws_cand = (int*)wc;
   a.ws_key = (unsigned long long*)wk;
   a.ws_val = (float*)wv;
-  a.plan = (unsigned long long*)wp;
+  a.plan = plan.dev;
   MB_CUDA(ctx, cudaFuncSetAttribute(k_sized_recommend, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
@@ -1540,8 +1479,7 @@ int mb200_sized_recommend(mb200_sized_bank* bk, const int64_t* nb_idx, const dou
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[RP_WORDS];
-  MB_CUDA(ctx, cudaMemcpyAsync(h, wp, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  MB_CHECK(plan.read(h));
   mb200_sized_recommend_plan& pl = ctx->last_sized_recommend_plan;
   pl.users = m;
   pl.chunks = (int64_t)h[RP_CHUNKS];

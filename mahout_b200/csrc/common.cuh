@@ -29,6 +29,41 @@ struct ProfSpan {
   cudaEvent_t beg, end;
 };
 
+// Named grow-only device workspaces of the context (ws_slot).  Two buffers live in the same call have different
+// names; buffers of the same role in calls that never run together share one.
+enum WsSlot {
+  WS_GROUP_SMALL,     // group.cu: histogram, segment offsets, cursors and ticket of one sub-batch
+  WS_GROUP_KQ2,       // group.cu: (key, quanta) records in entity order
+  WS_GROUP_KQ1,       // group.cu: (key, quanta) records after the coarse level
+  WS_GROUP_ENT1,      // group.cu: entities after the coarse level
+  WS_GROUP_WINDOWS,   // group.cu: first record of each K1 window
+  WS_GROUP_TILES,     // group.cu: tile descriptors of the second scatter level
+  WS_GROUP_TICKET,    // group.cu: work ticket of mb200_bank_update_grouped
+  WS_ROUTE,           // route.cu: per-shard counts and cursors
+  WS_WIDEN_ENTITY,    // sketch.cu: entity column of widened u8 events
+  WS_WIDEN_KEY,       // sketch.cu: key column of widened u8 events
+  WS_WIDEN_INC,       // sketch.cu: increment column of widened u8 events
+  WS_KEYTAB,          // sketch.cu: the K1 key table, all zero between calls
+  WS_K1_STATS,        // sketch.cu: MB200_TRACE counters of K1
+  WS_STATUS,          // recommend.cu, cmsized.cu: plan and status words of a call (StatusWords)
+  WS_REC_BITMAP,      // recommend.cu, cmsized.cu: per-CTA candidate bitmaps of k_recommend / k_sized_recommend
+  WS_REC_CAND,        // recommend.cu, cmsized.cu: per-CTA candidate lists
+  WS_REC_KEY,         // recommend.cu, cmsized.cu: per-CTA top-N keys
+  WS_REC_VAL,         // recommend.cu, cmsized.cu: per-CTA estimates
+  WS_IB_RANK_KEY,     // recommend.cu: (itemID, row) sort keys of the item-based rank table
+  WS_IB_RANK_ROW,     // recommend.cu: rank -> row
+  WS_IB_RANK_OF,      // recommend.cu: row -> rank
+  WS_IB_DENSE,        // recommend.cu: item-based dense slices, kept zero by k_itembased
+  WS_IB_LOCKS,        // recommend.cu: locks of the dense slices
+  WS_SIZED_ITEM,      // cmsized.cu: item column of the prefs while a sized bank is built
+  WS_SIZED_PREF,      // cmsized.cu: pref column of the prefs while a sized bank is built
+  WS_SIZED_SIMS,      // cmsized.cu: similarities of a query batch
+  WS_SIZED_SLICE,     // cmsized.cu: per-CTA global sketch slices (pair cosine, neighbourhood)
+  WS_SIZED_CLASSES,   // cmsized.cu: shape-class table of a neighbourhood call
+  WS_SIZED_ITEMS,     // cmsized.cu: work items of a neighbourhood batch
+  WS_SLOT_COUNT
+};
+
 struct mb200_ctx {
   int device = 0;
   int num_sms = 0;
@@ -52,14 +87,14 @@ struct mb200_ctx {
   // grow-only device workspaces of the cosine stage (slot i = i-th request of a call); cudaMalloc /
   // cudaFree of a few hundred MB per call would otherwise cost more than the kernels
   std::vector<std::pair<void*, size_t>> ws;
-  // grow-only workspaces of the grouped K1 path (group.cu) and of the event router (route.cu)
-  std::vector<std::pair<void*, size_t>> ws_group;
+  // named grow-only workspaces (WsSlot)
+  std::pair<void*, size_t> ws_slots[WS_SLOT_COUNT] = {};
   int64_t group_min_events = 1 << 16;  // MB200_OPT_GROUP_MIN_EVENTS
   int group_prefetch = 0;              // MB200_OPT_GROUP_PREFETCH
   int single_kernel = 1;               // MB200_OPT_SINGLE_KERNEL
   int64_t max_fallback_rows = -1;      // MB200_OPT_MAX_FALLBACK_ROWS
-  // grow-only device staging of host-memory arguments (see io_slot in sketch.cu)
-  std::pair<void*, size_t> io[3] = {{nullptr, 0}, {nullptr, 0}, {nullptr, 0}};
+  // grow-only device staging of host-memory arguments, in request order within a call (ArgStage)
+  std::vector<std::pair<void*, size_t>> io;
   // pull-gather: per-block arrival flags written by the copy stream, read by K3 (+ 1 abort word)
   uint32_t* gather_flags = nullptr;
   uint32_t* gather_abort = nullptr;
@@ -74,7 +109,7 @@ struct mb200_ctx {
   mb200_itembased_plan last_itembased_plan = {};  // mb200_itembased_last_plan
   mb200_sized_plan last_sized_plan = {};          // mb200_sized_last_plan
   mb200_sized_recommend_plan last_sized_recommend_plan = {};  // mb200_sized_recommend_last_plan
-  int64_t itembased_dense_items = -1, itembased_dense_slices = -1;  // layout of the zeroed dense slices (slot 62)
+  int64_t itembased_dense_items = -1, itembased_dense_slices = -1;  // layout of the zeroed dense slices (WS_IB_DENSE)
 };
 
 // borrows workspace slots from the context in request order; nothing is freed on return
@@ -98,9 +133,10 @@ struct mb200_bank {
 };
 
 int mb200_fail(mb200_ctx* ctx, int code, const char* fmt, ...);
+// the named workspace `slot`, (re)allocated when smaller than `bytes`; *fresh tells that it just was
+int ws_slot(mb200_ctx* ctx, WsSlot slot, size_t bytes, void** out, bool* fresh = nullptr);
 // group.cu: bank-mode K1 through device-side grouping (called with ctx->mu held)
 bool mb200_group_applicable(const mb200_bank* bk, int64_t n);
-int mb200_group_ws(mb200_ctx* ctx, size_t slot, size_t bytes, void** out);  // grow-only slot of ctx->ws_group
 template <typename T>
 int mb200_group_update(mb200_bank* bk, const long long* entity, const long long* key, const T* inc, int64_t n);
 extern "C" void mb200_job_release(struct mb200_cosine_job* job);  // cosine.cu (internal)
@@ -126,6 +162,63 @@ struct ProfScope {
   int idx = -1;
   ProfScope(mb200_ctx* c, int kernel_id);
   ~ProfScope();
+};
+
+// A call's array arguments.  Under MB200_MEM_DEVICE, and for a NULL input, the caller's pointer passes through;
+// otherwise in() copies the host array into ctx->io and out() lends a buffer there that finish() copies back.
+// ctx->io is taken in request order, so no staged call may run while another is in progress.  The caller's host
+// buffers are only borrowed for the call: finish() synchronises when anything was staged, and the destructor does
+// when inputs were staged and finish() did not run.
+struct ArgStage {
+  mb200_ctx* ctx;
+  int mem;
+  ArgStage(mb200_ctx* c, int m) : ctx(c), mem(m) {}
+  ~ArgStage();
+  template <typename T>
+  int in(const T* user, size_t n, const T** dev) {
+    *dev = user;
+    if (mem == MB200_MEM_DEVICE || !user) return MB200_OK;
+    void* p = nullptr;
+    MB_CHECK(buffer(n * sizeof(T), &p));
+    if (n) MB_CUDA(ctx, cudaMemcpyAsync(p, user, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
+    ctx->stat_h2d += (int64_t)(n * sizeof(T));
+    inputs = true;
+    *dev = (const T*)p;
+    return MB200_OK;
+  }
+  template <typename T>
+  int out(T* user, size_t n, T** dev) {
+    *dev = user;
+    if (mem == MB200_MEM_DEVICE) return MB200_OK;
+    void* p = nullptr;
+    MB_CHECK(buffer(n * sizeof(T), &p));
+    outs.push_back({p, user, n * sizeof(T)});
+    *dev = (T*)p;
+    return MB200_OK;
+  }
+  int finish();
+
+ private:
+  struct Out {
+    void* dev;
+    void* user;
+    size_t bytes;
+  };
+  size_t next = 0;
+  bool inputs = false;  // staged inputs not yet synchronised
+  std::vector<Out> outs;
+  int buffer(size_t bytes, void** out);
+};
+
+// `n` status / plan words in a named workspace: zero() clears them on the stream before the launch, read() copies
+// them to the host with one synchronise
+struct StatusWords {
+  mb200_ctx* ctx;
+  size_t n;
+  unsigned long long* dev = nullptr;
+  StatusWords(mb200_ctx* c, size_t words) : ctx(c), n(words) {}
+  int zero(WsSlot slot);
+  int read(unsigned long long* h);
 };
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

@@ -755,25 +755,6 @@ __global__ void k_check_row_ptr(const long long* __restrict__ row_ptr, long long
   if (bad) atomicAdd(&flags[FLAG_BAD_ENTITY], 1ull);
 }
 
-int ws_get(mb200_ctx* ctx, size_t slot, size_t bytes, void** out) {
-  while (slot >= ctx->ws_group.size()) ctx->ws_group.emplace_back(nullptr, 0);
-  auto& s = ctx->ws_group[slot];
-  if (s.second < bytes || !s.first) {
-    if (s.first) cudaFree(s.first);
-    s.first = nullptr;
-    s.second = 0;
-    const size_t want = bytes ? bytes : 1;
-    cudaError_t e = cudaMalloc(&s.first, want);
-    if (e != cudaSuccess) {
-      s.first = nullptr;
-      return mb200_fail(ctx, MB200_ERR_OOM, "cannot allocate %zu bytes of grouping workspace: %s", want, cudaGetErrorString(e));
-    }
-    s.second = want;
-  }
-  *out = s.first;
-  return MB200_OK;
-}
-
 template <typename Src, typename IdxT>
 int launch_grouped(mb200_bank* bk, const Src& src, const IdxT* seg, const IdxT* end, unsigned* ticket,
                    const unsigned* wide_seen, long long max_records) {
@@ -791,7 +772,7 @@ int launch_grouped(mb200_bank* bk, const Src& src, const IdxT* seg, const IdxT* 
   {
     void* wf;
     const long long max_win = max_records / U_WINDOW + 2;
-    MB_CHECK(ws_get(ctx, 9, (size_t)max_win * 4, &wf));
+    MB_CHECK(ws_slot(ctx, WS_GROUP_WINDOWS, (size_t)max_win * 4, &wf));
     ga.win_first = (const unsigned*)wf;
     const int g = (int)(max_win / 256 + 1 < 1024 ? max_win / 256 + 1 : 1024);
     k_window_desc<IdxT><<<g, 256, 0, ctx->stream>>>(seg, bk->E, (unsigned*)wf);
@@ -824,8 +805,6 @@ int launch_grouped(mb200_bank* bk, const Src& src, const IdxT* seg, const IdxT* 
 
 }  // namespace
 
-int mb200_group_ws(mb200_ctx* ctx, size_t slot, size_t bytes, void** out) { return ws_get(ctx, slot, bytes, out); }
-
 // ---- host orchestration (called with the context's mutex held) ------------------------------------------
 bool mb200_group_applicable(const mb200_bank* bk, int64_t n) {
   // worth it once the events outnumber the fixed cost of the extra passes; the two partition levels cover
@@ -850,9 +829,9 @@ int mb200_group_update(mb200_bank* bk, const long long* entity, const long long*
     unsigned *hist, *seg, *cur2, *cur1, *base1, *tile_ptr, *ticket, *ent1;
     uint2 *kq1, *kq2;
     void* p;
-    // slot 0: all the small arrays in one allocation
+    // the small arrays in one allocation
     const size_t words = (size_t)(E + 1) * 3 + (size_t)(G_NB + 1) * 3 + 8;
-    MB_CHECK(ws_get(ctx, 0, words * 4, &p));
+    MB_CHECK(ws_slot(ctx, WS_GROUP_SMALL, words * 4, &p));
     hist = (unsigned*)p;
     seg = hist + (E + 1);
     cur2 = seg + (E + 1);
@@ -860,14 +839,14 @@ int mb200_group_update(mb200_bank* bk, const long long* entity, const long long*
     base1 = cur1 + (G_NB + 1);
     tile_ptr = base1 + (G_NB + 1);
     ticket = tile_ptr + (G_NB + 1);
-    MB_CHECK(ws_get(ctx, 1, (size_t)m * 8, &p));
+    MB_CHECK(ws_slot(ctx, WS_GROUP_KQ2, (size_t)m * 8, &p));
     kq2 = (uint2*)p;
     kq1 = nullptr;
     ent1 = nullptr;
     if (two_level) {
-      MB_CHECK(ws_get(ctx, 2, (size_t)m * 8, &p));
+      MB_CHECK(ws_slot(ctx, WS_GROUP_KQ1, (size_t)m * 8, &p));
       kq1 = (uint2*)p;
-      MB_CHECK(ws_get(ctx, 3, (size_t)m * 4, &p));
+      MB_CHECK(ws_slot(ctx, WS_GROUP_ENT1, (size_t)m * 4, &p));
       ent1 = (unsigned*)p;
     }
     {
@@ -928,7 +907,7 @@ int mb200_group_update(mb200_bank* bk, const long long* entity, const long long*
       {
         void* dp;
         const long long max_tiles = m / G_TILE + nb1 + 2;
-        MB_CHECK(ws_get(ctx, 10, (size_t)max_tiles * sizeof(uint4), &dp));
+        MB_CHECK(ws_slot(ctx, WS_GROUP_TILES, (size_t)max_tiles * sizeof(uint4), &dp));
         a2.desc = (const uint4*)dp;
         const int g = (int)(max_tiles / 256 + 1 < 2048 ? max_tiles / 256 + 1 : 2048);
         k_tile_desc<<<g, 256, 0, ctx->stream>>>(tile_ptr, base1, cur1, nb1, (uint4*)dp);
@@ -967,25 +946,17 @@ extern "C" int mb200_bank_update_grouped(mb200_bank* bk, const int64_t* row_ptr,
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_update_grouped: mem must be MB200_MEM_HOST or MB200_MEM_DEVICE");
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
   const long long E = bk->E;
-  const long long* d_ptr = (const long long*)row_ptr;
-  const long long* d_key = (const long long*)key;
-  const float* d_inc = inc;
   void* p;
-  MB_CHECK(ws_get(ctx, 4, 64, &p));
+  MB_CHECK(ws_slot(ctx, WS_GROUP_TICKET, 64, &p));
   unsigned* ticket = (unsigned*)p;
-  if (mem == MB200_MEM_HOST) {
-    if (row_ptr[0] != 0 || row_ptr[E] != n)
-      return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_update_grouped: row_ptr[0] must be 0 and row_ptr[entities] must be n");
-    MB_CHECK(ws_get(ctx, 5, (size_t)(E + 1) * 8, &p));
-    MB_CUDA(ctx, cudaMemcpyAsync(p, row_ptr, (size_t)(E + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
-    d_ptr = (const long long*)p;
-    MB_CHECK(ws_get(ctx, 6, (size_t)(n > 0 ? n : 1) * 8, &p));
-    MB_CUDA(ctx, cudaMemcpyAsync(p, key, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-    d_key = (const long long*)p;
-    MB_CHECK(ws_get(ctx, 7, (size_t)(n > 0 ? n : 1) * 4, &p));
-    MB_CUDA(ctx, cudaMemcpyAsync(p, inc, (size_t)n * 4, cudaMemcpyHostToDevice, ctx->stream));
-    d_inc = (const float*)p;
-  }
+  if (mem == MB200_MEM_HOST && (row_ptr[0] != 0 || row_ptr[E] != n))
+    return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_update_grouped: row_ptr[0] must be 0 and row_ptr[entities] must be n");
+  ArgStage st(ctx, mem);
+  const long long *d_ptr, *d_key;
+  const float* d_inc;
+  MB_CHECK(st.in((const long long*)row_ptr, (size_t)E + 1, &d_ptr));
+  MB_CHECK(st.in((const long long*)key, (size_t)n, &d_key));
+  MB_CHECK(st.in(inc, (size_t)n, &d_inc));
   MB_CUDA(ctx, cudaMemsetAsync(ticket, 0, 32, ctx->stream));
   k_check_row_ptr<<<(unsigned)ceil_div64(E + 1, 256), 256, 0, ctx->stream>>>(d_ptr, E, n, bk->flags);
   ctx->launches++;
@@ -1001,6 +972,5 @@ extern "C" int mb200_bank_update_grouped(mb200_bank* bk, const int64_t* row_ptr,
     MB_CHECK((launch_grouped<WideSrc<float>, long long>(bk, src, d_ptr, d_ptr + 1, ticket, nullptr, n)));
   }
   bk->events_total += (double)n;
-  if (mem == MB200_MEM_HOST) MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return MB200_OK;
+  return st.finish();
 }

@@ -800,68 +800,6 @@ __global__ void k_rank_scatter(const int* __restrict__ row_at, long long n, int*
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-// host-memory arguments are staged through grow-only slots of the context (mb200_group_ws; slots 40.. are this file's)
-namespace {
-struct Staged {
-  mb200_ctx* ctx;
-  int mem;
-  int next_slot = 40;
-  std::vector<std::pair<void*, std::pair<void*, size_t>>> outs;  // (device, (user, bytes))
-  Staged(mb200_ctx* c, int m) : ctx(c), mem(m) {}
-  template <typename T>
-  int in(const T* user, size_t n, const T** dev) {
-    if (mem == MB200_MEM_DEVICE || !user) {
-      *dev = user;
-      next_slot++;
-      return MB200_OK;
-    }
-    void* p = nullptr;
-    MB_CHECK(mb200_group_ws(ctx, next_slot++, n * sizeof(T), &p));
-    if (n) MB_CUDA(ctx, cudaMemcpyAsync(p, user, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
-    ctx->stat_h2d += (int64_t)(n * sizeof(T));
-    *dev = (const T*)p;
-    return MB200_OK;
-  }
-  template <typename T>
-  int out(T* user, size_t n, T** dev) {
-    if (mem == MB200_MEM_DEVICE) {
-      *dev = user;
-      next_slot++;
-      return MB200_OK;
-    }
-    void* p = nullptr;
-    MB_CHECK(mb200_group_ws(ctx, next_slot++, n * sizeof(T), &p));
-    outs.push_back({p, {(void*)user, n * sizeof(T)}});
-    *dev = (T*)p;
-    return MB200_OK;
-  }
-  int finish() {
-    for (auto& o : outs) {
-      if (o.second.second)
-        MB_CUDA(ctx, cudaMemcpyAsync(o.second.first, o.first, o.second.second, cudaMemcpyDeviceToHost, ctx->stream));
-      ctx->stat_d2h += (int64_t)o.second.second;
-    }
-    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return MB200_OK;
-  }
-};
-
-// the plan / error words live in a slot of their own; read back after the launch
-int plan_words(mb200_ctx* ctx, unsigned long long** plan) {
-  void* p = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, 39, PL_WORDS * sizeof(unsigned long long), &p));
-  MB_CUDA(ctx, cudaMemsetAsync(p, 0, PL_WORDS * sizeof(unsigned long long), ctx->stream));
-  *plan = (unsigned long long*)p;
-  return MB200_OK;
-}
-
-int read_plan(mb200_ctx* ctx, const unsigned long long* plan, unsigned long long* h) {
-  MB_CUDA(ctx, cudaMemcpyAsync(h, plan, PL_WORDS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  return MB200_OK;
-}
-}  // namespace
-
 extern "C" {
 
 int mb200_bank_estimate_prefs(mb200_bank* bk, const int64_t* nb_idx, const double* nb_sim, const int32_t* nb_cnt,
@@ -877,7 +815,7 @@ int mb200_bank_estimate_prefs(mb200_bank* bk, const int64_t* nb_idx, const doubl
   if (!user || !item_id || !out || (nb_rows > 0 && (!nb_idx || !nb_sim || !nb_cnt)))
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_estimate_prefs: NULL array argument");
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  Staged st(ctx, mem);
+  ArgStage st(ctx, mem);
   const long long *d_idx, *d_user, *d_row, *d_item;
   const double* d_sim;
   const int* d_cnt;
@@ -890,19 +828,19 @@ int mb200_bank_estimate_prefs(mb200_bank* bk, const int64_t* nb_idx, const doubl
   MB_CHECK(st.in((const long long*)nb_row, nb_row ? (size_t)q : 0, &d_row));
   MB_CHECK(st.in((const long long*)item_id, (size_t)q, &d_item));
   MB_CHECK(st.out(out, (size_t)q, &d_out));
-  unsigned long long* plan = nullptr;
-  MB_CHECK(plan_words(ctx, &plan));
+  StatusWords plan(ctx, PL_WORDS);
+  MB_CHECK(plan.zero(WS_STATUS));
   {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
     k_estimate_prefs<<<(unsigned)ceil_div64(q, EST_THREADS), EST_THREADS, (size_t)bk->d * EST_THREADS * 4, ctx->stream>>>(
         bk->counters, bk->hf, bk->E, ldexp(1.0, -bk->frac_bits), d_idx, d_sim, d_cnt, nb_rows, nb_ld, d_user, d_row,
-        d_item, q, d_out, plan);
+        d_item, q, d_out, plan.dev);
   }
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[PL_WORDS];
-  MB_CHECK(read_plan(ctx, plan, h));
+  MB_CHECK(plan.read(h));
   if (h[PL_BAD])
     return mb200_fail(ctx, MB200_ERR_BAD_ARG,
                       "mb200_bank_estimate_prefs: %llu user row(s), neighbourhood row(s), counts or neighbour index(es) "
@@ -958,7 +896,7 @@ int mb200_bank_recommend(mb200_bank* bk, const int64_t* nb_idx, const double* nb
   const size_t smem = fixed + (size_t)stages * row_bytes;
   const int grid = (int)(m < ctx->num_sms ? m : ctx->num_sms);
 
-  Staged st(ctx, mem);
+  ArgStage st(ctx, mem);
   RecArgs a;
   a.counters = bk->counters;
   a.hf = bk->hf;
@@ -987,15 +925,17 @@ int mb200_bank_recommend(mb200_bank* bk, const int64_t* nb_idx, const double* nb
   MB_CHECK(st.out((int*)out_cnt, (size_t)m, &a.out_cnt));
   void *wb = nullptr, *wc = nullptr, *wk = nullptr, *wv = nullptr;
   const size_t per = (size_t)(num_items > 0 ? num_items : 1);
-  MB_CHECK(mb200_group_ws(ctx, 36, bitmap_smem ? 4 : (size_t)grid * words * 4, &wb));
-  MB_CHECK(mb200_group_ws(ctx, 37, (size_t)grid * per * 4, &wc));
-  MB_CHECK(mb200_group_ws(ctx, 38, (size_t)grid * per * 8, &wk));
-  MB_CHECK(mb200_group_ws(ctx, 35, (size_t)grid * per * 4, &wv));
+  MB_CHECK(ws_slot(ctx, WS_REC_BITMAP, bitmap_smem ? 4 : (size_t)grid * words * 4, &wb));
+  MB_CHECK(ws_slot(ctx, WS_REC_CAND, (size_t)grid * per * 4, &wc));
+  MB_CHECK(ws_slot(ctx, WS_REC_KEY, (size_t)grid * per * 8, &wk));
+  MB_CHECK(ws_slot(ctx, WS_REC_VAL, (size_t)grid * per * 4, &wv));
   a.ws_bitmap = (unsigned*)wb;
   a.ws_cand = (int*)wc;
   a.ws_key = (unsigned long long*)wk;
   a.ws_val = (float*)wv;
-  MB_CHECK(plan_words(ctx, &a.plan));
+  StatusWords plan(ctx, PL_WORDS);
+  MB_CHECK(plan.zero(WS_STATUS));
+  a.plan = plan.dev;
   MB_CUDA(ctx, cudaFuncSetAttribute(k_recommend, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
@@ -1005,7 +945,7 @@ int mb200_bank_recommend(mb200_bank* bk, const int64_t* nb_idx, const double* nb
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[PL_WORDS];
-  MB_CHECK(read_plan(ctx, a.plan, h));
+  MB_CHECK(plan.read(h));
   mb200_recommend_plan& pl = ctx->last_recommend_plan;
   pl.stream_users = (int64_t)h[PL_STREAM];
   pl.gather_users = (int64_t)h[PL_GATHER];
@@ -1061,7 +1001,7 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
   const long long n = x.num_items;
   const long long words = (n + 31) / 32;
 
-  Staged st(ctx, x.mem);
+  ArgStage st(ctx, x.mem);
   IbArgs a;
   a.num_items = n;
   a.ld = x.sim_ld;
@@ -1088,15 +1028,15 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
   // the itemID rank table: (itemID, row) sorted on the device, rank -> row and row -> rank
   long long npad = 1;
   while (npad < n) npad <<= 1;
-  void *wk = nullptr, *wr = nullptr, *wo = nullptr, *wp = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, 60, (size_t)npad * 8, &wk));
-  MB_CHECK(mb200_group_ws(ctx, 61, (size_t)npad * 4, &wr));
-  MB_CHECK(mb200_group_ws(ctx, 63, (size_t)(n > 0 ? n : 1) * 4, &wo));
-  MB_CHECK(mb200_group_ws(ctx, 64, IP_WORDS * sizeof(unsigned long long), &wp));
+  void *wk = nullptr, *wr = nullptr, *wo = nullptr;
+  MB_CHECK(ws_slot(ctx, WS_IB_RANK_KEY, (size_t)npad * 8, &wk));
+  MB_CHECK(ws_slot(ctx, WS_IB_RANK_ROW, (size_t)npad * 4, &wr));
+  MB_CHECK(ws_slot(ctx, WS_IB_RANK_OF, (size_t)(n > 0 ? n : 1) * 4, &wo));
+  StatusWords plan(ctx, IP_WORDS);
+  MB_CHECK(plan.zero(WS_STATUS));
   a.row_at = (const int*)wr;
   a.rank_of = (const int*)wo;
-  a.plan = (unsigned long long*)wp;
-  MB_CUDA(ctx, cudaMemsetAsync(wp, 0, IP_WORDS * sizeof(unsigned long long), ctx->stream));
+  a.plan = plan.dev;
   if (n > 0) {
     ProfScope prof(ctx, MB200_K_RECOMMEND);
     unsigned long long* key = (unsigned long long*)wk;
@@ -1127,18 +1067,18 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
   const size_t slice_bytes = (size_t)(n > 0 ? n : 1) * (8 + 8 + 4 + 4 + 8);
   long long slices = (long long)(IB_DENSE_MAX_BYTES / slice_bytes);
   slices = slices < 1 ? 1 : (slices > grid ? grid : slices);
-  // slot 62 holds the slices; num / den / cnt are kept zero by the kernel, so they are cleared only when the slot or
-  // its layout changes
+  // num / den / cnt of the slices are kept zero by the kernel, so they are cleared only when the slot is (re)allocated
+  // or its layout changes
   const size_t dense_bytes = (size_t)slices * slice_bytes;
-  const size_t had = ctx->ws_group.size() > 62 ? ctx->ws_group[62].second : 0;
   void *wd = nullptr, *wl = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, 62, dense_bytes, &wd));
-  if (ctx->ws_group[62].second != had || ctx->itembased_dense_items != n || ctx->itembased_dense_slices != slices) {
+  bool fresh = false;
+  MB_CHECK(ws_slot(ctx, WS_IB_DENSE, dense_bytes, &wd, &fresh));
+  if (fresh || ctx->itembased_dense_items != n || ctx->itembased_dense_slices != slices) {
     MB_CUDA(ctx, cudaMemsetAsync(wd, 0, dense_bytes, ctx->stream));
     ctx->itembased_dense_items = n;
     ctx->itembased_dense_slices = slices;
   }
-  MB_CHECK(mb200_group_ws(ctx, 65, (size_t)slices * 4, &wl));
+  MB_CHECK(ws_slot(ctx, WS_IB_LOCKS, (size_t)slices * 4, &wl));
   MB_CUDA(ctx, cudaMemsetAsync(wl, 0, (size_t)slices * 4, ctx->stream));
   const size_t per = (size_t)slices * (n > 0 ? n : 1);
   a.d_num = (double*)wd;
@@ -1156,8 +1096,7 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
   MB_CUDA(ctx, cudaGetLastError());
   MB_CHECK(st.finish());
   unsigned long long h[IP_WORDS];
-  MB_CUDA(ctx, cudaMemcpyAsync(h, a.plan, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  MB_CHECK(plan.read(h));
   mb200_itembased_plan& pl = ctx->last_itembased_plan;
   pl.users = x.m;
   pl.smem_users = (int64_t)h[IP_SMEM];

@@ -140,26 +140,6 @@ __global__ void __launch_bounds__(R_THREADS, 2) k_route_scatter(const RouteArgs 
   }
 }
 
-int route_ws(mb200_ctx* ctx, size_t slot, size_t bytes, void** out) {
-  while (slot >= ctx->ws_group.size()) ctx->ws_group.emplace_back(nullptr, 0);
-  auto& s = ctx->ws_group[slot];
-  if (s.second < bytes || !s.first) {
-    if (s.first) cudaFree(s.first);
-    s.first = nullptr;
-    s.second = 0;
-    cudaError_t e = cudaMalloc(&s.first, bytes ? bytes : 1);
-    if (e != cudaSuccess) {
-      s.first = nullptr;
-      return mb200_fail(ctx, MB200_ERR_OOM, "cannot allocate %zu bytes of routing workspace: %s", bytes, cudaGetErrorString(e));
-    }
-    s.second = bytes ? bytes : 1;
-  }
-  *out = s.first;
-  return MB200_OK;
-}
-
-constexpr size_t ROUTE_SLOT = 8;  // ws_group slots 0..7 belong to group.cu
-
 void pow2_of(int G, int& gmask, int& gshift) {
   gmask = -1;
   gshift = 0;
@@ -181,7 +161,7 @@ int mb200_route_count(mb200_ctx* ctx, const int64_t* row, int64_t n, int32_t sha
                       (long long)n, shards, MB200_MAX_BLOCKS);
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
   void* p;
-  MB_CHECK(route_ws(ctx, ROUTE_SLOT, 2 * MB200_MAX_BLOCKS * sizeof(unsigned long long), &p));
+  MB_CHECK(ws_slot(ctx, WS_ROUTE, 2 * MB200_MAX_BLOCKS * sizeof(unsigned long long), &p));
   unsigned long long* d_counts = (unsigned long long*)p;
   MB_CUDA(ctx, cudaMemsetAsync(d_counts, 0, MB200_MAX_BLOCKS * sizeof(unsigned long long), ctx->stream));
   if (n > 0) {
@@ -212,7 +192,7 @@ int mb200_route_scatter(mb200_ctx* ctx, const int64_t* row, const int64_t* key, 
   if (n == 0) return MB200_OK;
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
   void* p;
-  MB_CHECK(route_ws(ctx, ROUTE_SLOT, 2 * MB200_MAX_BLOCKS * sizeof(unsigned long long), &p));
+  MB_CHECK(ws_slot(ctx, WS_ROUTE, 2 * MB200_MAX_BLOCKS * sizeof(unsigned long long), &p));
   unsigned long long* d_cursor = (unsigned long long*)p + MB200_MAX_BLOCKS;
   unsigned long long h[MB200_MAX_BLOCKS];
   RouteArgs a;

@@ -20,9 +20,10 @@ int mb200_fail(mb200_ctx* ctx, int code, const char* fmt, ...) {
   return code;
 }
 
-int Workspace::get(size_t bytes, void** out) {
-  while (next >= ctx->ws.size()) ctx->ws.emplace_back(nullptr, 0);
-  auto& slot = ctx->ws[next++];
+// Grow-only device buffer: reallocated only when smaller than `bytes`, never freed on return.  cudaMalloc / cudaFree
+// synchronise the device and were measured at 1 ms .. 1 s each on a process holding tens of GB.
+static int grow(mb200_ctx* ctx, std::pair<void*, size_t>& slot, size_t bytes, void** out, bool* fresh = nullptr) {
+  if (fresh) *fresh = false;
   if (slot.second < bytes || !slot.first) {
     if (slot.first) cudaFree(slot.first);
     slot.first = nullptr;
@@ -34,8 +35,55 @@ int Workspace::get(size_t bytes, void** out) {
       return mb200_fail(ctx, MB200_ERR_OOM, "cannot allocate %zu bytes of workspace: %s", want, cudaGetErrorString(e));
     }
     slot.second = want;
+    if (fresh) *fresh = true;
   }
   *out = slot.first;
+  return MB200_OK;
+}
+
+// the next buffer of a request-order pool (a cosine job may start its requests past the pool's end)
+static int grow_next(mb200_ctx* ctx, std::vector<std::pair<void*, size_t>>& pool, size_t& next, size_t bytes,
+                     void** out) {
+  while (next >= pool.size()) pool.emplace_back(nullptr, 0);
+  return grow(ctx, pool[next++], bytes, out);
+}
+
+int Workspace::get(size_t bytes, void** out) { return grow_next(ctx, ctx->ws, next, bytes, out); }
+
+int ws_slot(mb200_ctx* ctx, WsSlot slot, size_t bytes, void** out, bool* fresh) {
+  return grow(ctx, ctx->ws_slots[slot], bytes, out, fresh);
+}
+
+int ArgStage::buffer(size_t bytes, void** out) { return grow_next(ctx, ctx->io, next, bytes, out); }
+
+int ArgStage::finish() {
+  if (!inputs && outs.empty()) return MB200_OK;
+  for (auto& o : outs) {
+    if (o.bytes) MB_CUDA(ctx, cudaMemcpyAsync(o.user, o.dev, o.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    ctx->stat_d2h += (int64_t)o.bytes;
+  }
+  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  inputs = false;
+  outs.clear();
+  return MB200_OK;
+}
+
+ArgStage::~ArgStage() {
+  // pageable inputs are already copied when cudaMemcpyAsync returns; pinned ones are read asynchronously
+  if (inputs) cudaStreamSynchronize(ctx->stream);
+}
+
+int StatusWords::zero(WsSlot slot) {
+  void* p = nullptr;
+  MB_CHECK(ws_slot(ctx, slot, n * sizeof(unsigned long long), &p));
+  MB_CUDA(ctx, cudaMemsetAsync(p, 0, n * sizeof(unsigned long long), ctx->stream));
+  dev = (unsigned long long*)p;
+  return MB200_OK;
+}
+
+int StatusWords::read(unsigned long long* h) {
+  MB_CUDA(ctx, cudaMemcpyAsync(h, dev, n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+  MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return MB200_OK;
 }
 
@@ -127,7 +175,7 @@ int mb200_destroy(mb200_ctx* ctx) {
     if (w.first) cudaFree(w.first);
   for (auto& w : ctx->io)
     if (w.first) cudaFree(w.first);
-  for (auto& w : ctx->ws_group)
+  for (auto& w : ctx->ws_slots)
     if (w.first) cudaFree(w.first);
   if (ctx->gather_flags) cudaFree(ctx->gather_flags);
   if (ctx->gather_ev) cudaEventDestroy(ctx->gather_ev);
@@ -156,6 +204,7 @@ int mb200_get_stats(mb200_ctx* ctx, mb200_stats* out) {
   out->num_sms = ctx->num_sms;
   out->launches = ctx->launches;
   for (auto& w : ctx->ws) out->workspace_bytes += (int64_t)w.second;
+  for (auto& w : ctx->ws_slots) out->workspace_bytes += (int64_t)w.second;
   for (auto& w : ctx->io) out->staging_bytes += (int64_t)w.second;
   out->staging_bytes += 2 * (int64_t)ctx->stage_bytes;
   out->last_fallback_rows = ctx->last_fallback_rows;
@@ -183,13 +232,13 @@ int mb200_release_workspace(mb200_ctx* ctx) {
   for (auto& w : ctx->ws)
     if (w.first) cudaFree(w.first);
   ctx->ws.clear();
-  for (auto& w : ctx->ws_group)
-    if (w.first) cudaFree(w.first);
-  ctx->ws_group.clear();
-  for (auto& w : ctx->io) {
+  for (auto& w : ctx->ws_slots) {
     if (w.first) cudaFree(w.first);
     w = {nullptr, 0};
   }
+  for (auto& w : ctx->io)
+    if (w.first) cudaFree(w.first);
+  ctx->io.clear();
   return MB200_OK;
 }
 

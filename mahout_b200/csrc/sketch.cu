@@ -635,7 +635,6 @@ __global__ void __launch_bounds__(256) k_widen_events(const uint32_t* __restrict
 // The flush costs a scan of the table plus d reductions per distinct key, so the table pays off on large calls only;
 // the host-memory path stages 2^23-event chunks, which stay on the direct path.  DESIGN.md §3 has the crossover.
 static constexpr int64_t KT_MIN_EVENTS = 1LL << 26;
-static constexpr size_t KT_SLOT = 20, KT_STATS_SLOT = 21;  // ws_group slots
 
 static int64_t keytab_min_events() {
   if (const char* ev = getenv("MB200_K1_KEYTABLE_MIN_EVENTS"))  // tuning / test override: 0 = always, huge = never
@@ -645,10 +644,10 @@ static int64_t keytab_min_events() {
 
 // the table is zeroed when it is allocated and every call leaves it zeroed (k_keytab_flush)
 static int keytab(mb200_ctx* ctx, long long** out) {
-  const size_t had = ctx->ws_group.size() > KT_SLOT ? ctx->ws_group[KT_SLOT].second : 0;
   void* p = nullptr;
-  MB_CHECK(mb200_group_ws(ctx, KT_SLOT, (size_t)KT_ROWS * sizeof(long long), &p));
-  if (ctx->ws_group[KT_SLOT].second != had) MB_CUDA(ctx, cudaMemsetAsync(p, 0, (size_t)KT_ROWS * sizeof(long long), ctx->stream));
+  bool fresh = false;
+  MB_CHECK(ws_slot(ctx, WS_KEYTAB, (size_t)KT_ROWS * sizeof(long long), &p, &fresh));
+  if (fresh) MB_CUDA(ctx, cudaMemsetAsync(p, 0, (size_t)KT_ROWS * sizeof(long long), ctx->stream));
   *out = (long long*)p;
   return MB200_OK;
 }
@@ -662,9 +661,9 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
       if (!entity) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_update_u8: entity is NULL but the bank has %lld entities", (long long)bk->E);
       if (bk->frac_bits > 24) return mb200_fail(ctx, MB200_ERR_UNSUPPORTED, "mb200_bank_update_u8: bank mode needs frac_bits <= 24");
       void *we, *wk, *wi;
-      MB_CHECK(mb200_group_ws(ctx, 16, (size_t)n * 8, &we));
-      MB_CHECK(mb200_group_ws(ctx, 17, (size_t)n * 8, &wk));
-      MB_CHECK(mb200_group_ws(ctx, 18, (size_t)n * 4, &wi));
+      MB_CHECK(ws_slot(ctx, WS_WIDEN_ENTITY, (size_t)n * 8, &we));
+      MB_CHECK(ws_slot(ctx, WS_WIDEN_KEY, (size_t)n * 8, &wk));
+      MB_CHECK(ws_slot(ctx, WS_WIDEN_INC, (size_t)n * 4, &wi));
       long long want = ceil_div64(n, 256);
       const int grid = (int)(want < (long long)ctx->num_sms * 16 ? want : (long long)ctx->num_sms * 16);
       k_widen_events<<<grid, 256, 0, ctx->stream>>>((const uint32_t*)entity, (const uint32_t*)key, (const unsigned char*)inc, n,
@@ -702,14 +701,10 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
     const bool table = !agg && n >= keytab_min_events();
     const bool trace = getenv("MB200_TRACE") != nullptr;
     long long* ktab = nullptr;
-    unsigned long long* stats = nullptr;
+    StatusWords sw(ctx, KS_WORDS);
     if (table) MB_CHECK(keytab(ctx, &ktab));
-    if (trace) {
-      void* s = nullptr;
-      MB_CHECK(mb200_group_ws(ctx, KT_STATS_SLOT, KS_WORDS * sizeof(unsigned long long), &s));
-      MB_CUDA(ctx, cudaMemsetAsync(s, 0, KS_WORDS * sizeof(unsigned long long), ctx->stream));
-      stats = (unsigned long long*)s;
-    }
+    if (trace) MB_CHECK(sw.zero(WS_K1_STATS));
+    unsigned long long* stats = sw.dev;
 #define LAUNCH_V2_C(VEC, D, AGG, KT, COUNT)                                                                  \
   do {                                                                                                       \
     MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single_v2<T, VEC, D, K, AGG, KT, COUNT>,                      \
@@ -748,8 +743,7 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
     if (trace) {
       MB_CUDA(ctx, cudaGetLastError());
       unsigned long long h[KS_WORDS];
-      MB_CUDA(ctx, cudaMemcpyAsync(h, stats, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-      MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      MB_CHECK(sw.read(h));
       // L2 reductions of the call: one per table miss, d per direct event, cached key and flushed table key
       const double reds = (double)h[KS_TABLE] + (double)bk->d * (double)(h[KS_DIRECT] + h[KS_CACHE] + h[KS_FLUSHED]);
       fprintf(stderr,
@@ -867,81 +861,6 @@ static int bank_update_impl(mb200_bank* bk, const KIn* entity, const KIn* key, c
   return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_update: mem must be MB200_MEM_HOST or MB200_MEM_DEVICE");
 }
 
-// Device staging of host-memory arguments: grow-only slots on the context (slot = position of the
-// argument in the call).  cudaMalloc / cudaFree per call were measured at 1 ms .. 1 s each on a
-// process holding tens of GB (they synchronise the device), which dominated mb200_bank_read.
-static int io_slot(mb200_ctx* ctx, int slot, size_t bytes, void** out) {
-  auto& s = ctx->io[slot];
-  if (s.second < bytes || !s.first) {
-    if (s.first) MB_CUDA(ctx, cudaFree(s.first));
-    s.first = nullptr;
-    s.second = 0;
-    const size_t want = bytes ? bytes : 1;
-    cudaError_t e = cudaMalloc(&s.first, want);
-    if (e != cudaSuccess) {
-      s.first = nullptr;
-      return mb200_fail(ctx, MB200_ERR_OOM, "cannot allocate %zu bytes of staging memory: %s", want, cudaGetErrorString(e));
-    }
-    s.second = want;
-  }
-  *out = s.first;
-  return MB200_OK;
-}
-
-// copy `bytes` of results to the caller (host) or leave them where the kernel wrote them
-struct OutBuf {
-  mb200_ctx* ctx;
-  void* user;
-  void* dev = nullptr;
-  size_t bytes;
-  int mem, slot;
-  bool staged = false;
-  OutBuf(mb200_ctx* c, void* u, size_t b, int m, int s) : ctx(c), user(u), bytes(b), mem(m), slot(s) {}
-  int acquire() {
-    if (mem == MB200_MEM_DEVICE) {
-      dev = user;
-      return MB200_OK;
-    }
-    MB_CHECK(io_slot(ctx, slot, bytes, &dev));
-    staged = true;
-    return MB200_OK;
-  }
-  int release() {
-    if (!staged) return MB200_OK;
-    ctx->stat_d2h += (int64_t)bytes;
-    MB_CUDA(ctx, cudaMemcpyAsync(user, dev, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    MB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return MB200_OK;
-  }
-};
-
-struct InBuf {
-  mb200_ctx* ctx;
-  const void* user;
-  void* dev = nullptr;
-  size_t bytes;
-  int mem, slot;
-  bool staged = false;
-  InBuf(mb200_ctx* c, const void* u, size_t b, int m, int s) : ctx(c), user(u), bytes(b), mem(m), slot(s) {}
-  int acquire() {
-    if (!user) return MB200_OK;
-    if (mem == MB200_MEM_DEVICE) {
-      dev = const_cast<void*>(user);
-      return MB200_OK;
-    }
-    MB_CHECK(io_slot(ctx, slot, bytes, &dev));
-    staged = true;
-    ctx->stat_h2d += (int64_t)bytes;
-    MB_CUDA(ctx, cudaMemcpyAsync(dev, user, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    return MB200_OK;
-  }
-  ~InBuf() {
-    // the caller's buffer is only borrowed for the call (pageable copies are already staged by the
-    // runtime when cudaMemcpyAsync returns; pinned ones are read asynchronously)
-    if (staged) cudaStreamSynchronize(ctx->stream);
-  }
-};
-
 extern "C" {
 
 int mb200_hash_keys(mb200_ctx* ctx, int64_t a, int64_t b, int32_t w, const int64_t* keys, int64_t n,
@@ -952,16 +871,17 @@ int mb200_hash_keys(mb200_ctx* ctx, int64_t a, int64_t b, int32_t w, const int64
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_hash_keys: bad arguments (w=%d n=%lld)", w, (long long)n);
   if (n == 0) return MB200_OK;
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  InBuf in(ctx, keys, (size_t)n * 8, mem, 0);
-  OutBuf ob(ctx, out, (size_t)n * 4, mem, 2);
-  MB_CHECK(in.acquire());
-  MB_CHECK(ob.acquire());
+  ArgStage st(ctx, mem);
+  const long long* d_keys;
+  int* d_out;
+  MB_CHECK(st.in((const long long*)keys, (size_t)n, &d_keys));
+  MB_CHECK(st.out((int*)out, (size_t)n, &d_out));
   uint32_t wmask = (w > 1 && (w & (w - 1)) == 0) ? (uint32_t)(w - 1) : 0u;
   k_hash_keys<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(
-      cmh_residue(a), cmh_residue(b), (uint32_t)w, wmask, (const long long*)in.dev, n, (int*)ob.dev);
+      cmh_residue(a), cmh_residue(b), (uint32_t)w, wmask, d_keys, n, d_out);
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
-  return ob.release();
+  return st.finish();
 }
 
 int mb200_bank_create_params(mb200_ctx* ctx, int64_t entities, int32_t depth, int32_t width,
@@ -1180,14 +1100,15 @@ int mb200_bank_read(mb200_bank* bk, int64_t e0, int64_t e1, double* out, int mem
   for (int64_t e = e0; e < e1; e += step) {
     int64_t m = (e1 - e) < step ? (e1 - e) : step;
     int64_t cells = m * cells_per;
-    OutBuf ob(ctx, out + (e - e0) * cells_per, (size_t)cells * 8, mem, 2);
-    MB_CHECK(ob.acquire());
+    ArgStage st(ctx, mem);
+    double* d_out;
+    MB_CHECK(st.out(out + (e - e0) * cells_per, (size_t)cells, &d_out));
     long long want = ceil_div64(cells, 256);
     int grid = (int)(want < (long long)ctx->num_sms * 32 ? want : (long long)ctx->num_sms * 32);
-    k_read<<<grid, 256, 0, ctx->stream>>>(bk->counters + e * cells_per, cells, inv_q, (double*)ob.dev, bk->flags);
+    k_read<<<grid, 256, 0, ctx->stream>>>(bk->counters + e * cells_per, cells, inv_q, d_out, bk->flags);
     ctx->launches++;
     MB_CUDA(ctx, cudaGetLastError());
-    MB_CHECK(ob.release());
+    MB_CHECK(st.finish());
   }
   return check_flags(bk);
 }
@@ -1216,14 +1137,15 @@ int mb200_bank_read_i32(mb200_bank* bk, int64_t e0, int64_t e1, int32_t* out, in
   for (int64_t e = e0; e < e1; e += step) {
     int64_t m = (e1 - e) < step ? (e1 - e) : step;
     int64_t cells = m * cells_per;
-    OutBuf ob(ctx, out + (e - e0) * cells_per, (size_t)cells * 4, mem, 2);
-    MB_CHECK(ob.acquire());
+    ArgStage st(ctx, mem);
+    int* d_out;
+    MB_CHECK(st.out((int*)out + (e - e0) * cells_per, (size_t)cells, &d_out));
     long long want = ceil_div64(cells, 256);
     int grid = (int)(want < (long long)ctx->num_sms * 32 ? want : (long long)ctx->num_sms * 32);
-    k_read_i32<<<grid, 256, 0, ctx->stream>>>(bk->counters + e * cells_per, cells, (int*)ob.dev, bk->flags);
+    k_read_i32<<<grid, 256, 0, ctx->stream>>>(bk->counters + e * cells_per, cells, d_out, bk->flags);
     ctx->launches++;
     MB_CUDA(ctx, cudaGetLastError());
-    MB_CHECK(ob.release());
+    MB_CHECK(st.finish());
   }
   return check_flags(bk);
 }
@@ -1237,17 +1159,17 @@ int mb200_bank_query(mb200_bank* bk, const int64_t* entity, const int64_t* key, 
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_query: bad arguments");
   if (n == 0) return MB200_OK;
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  InBuf ie(ctx, entity, (size_t)n * 8, mem, 0), ik(ctx, key, (size_t)n * 8, mem, 1);
-  OutBuf ob(ctx, out, (size_t)n * 8, mem, 2);
-  MB_CHECK(ie.acquire());
-  MB_CHECK(ik.acquire());
-  MB_CHECK(ob.acquire());
+  ArgStage st(ctx, mem);
+  const long long *d_entity, *d_key;
+  double* d_out;
+  MB_CHECK(st.in((const long long*)entity, (size_t)n, &d_entity));
+  MB_CHECK(st.in((const long long*)key, (size_t)n, &d_key));
+  MB_CHECK(st.out(out, (size_t)n, &d_out));
   k_query<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(
-      bk->counters, bk->hf, bk->E, ldexp(1.0, -bk->frac_bits), (const long long*)ie.dev,
-      (const long long*)ik.dev, n, (double*)ob.dev, bk->flags);
+      bk->counters, bk->hf, bk->E, ldexp(1.0, -bk->frac_bits), d_entity, d_key, n, d_out, bk->flags);
   ctx->launches++;
   MB_CUDA(ctx, cudaGetLastError());
-  MB_CHECK(ob.release());
+  MB_CHECK(st.finish());
   return check_flags(bk);
 }
 
@@ -1266,22 +1188,22 @@ int mb200_bank_cross_cosine(mb200_bank* bka, const int64_t* ea, mb200_bank* bkb,
     return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_bank_cross_cosine: bad arguments");
   if (n == 0) return MB200_OK;
   MB_CUDA(ctx, cudaSetDevice(ctx->device));
-  InBuf ia(ctx, ea, (size_t)n * 8, mem, 0), ib(ctx, eb, (size_t)n * 8, mem, 1);
-  OutBuf ob(ctx, out, (size_t)n * 8, mem, 2);
-  MB_CHECK(ia.acquire());
-  MB_CHECK(ib.acquire());
-  MB_CHECK(ob.acquire());
+  ArgStage st(ctx, mem);
+  const long long *d_a, *d_b;
+  double* d_out;
+  MB_CHECK(st.in((const long long*)ea, (size_t)n, &d_a));
+  MB_CHECK(st.in((const long long*)eb, (size_t)n, &d_b));
+  MB_CHECK(st.out(out, (size_t)n, &d_out));
   const int64_t max_grid = 1 << 30;
   for (int64_t off = 0; off < n; off += max_grid) {
     int64_t m = (n - off) < max_grid ? (n - off) : max_grid;
     k_pair_cosine<<<(unsigned)m, 256, 0, ctx->stream>>>(
         bka->counters, bkb->counters, bka->d, bka->W, bka->E, bkb->E, ldexp(1.0, -bka->frac_bits),
-        ldexp(1.0, -bkb->frac_bits), (const long long*)ia.dev + off, (const long long*)ib.dev + off,
-        (double*)ob.dev + off, bka->flags);
+        ldexp(1.0, -bkb->frac_bits), d_a + off, d_b + off, d_out + off, bka->flags);
     ctx->launches++;
     MB_CUDA(ctx, cudaGetLastError());
   }
-  MB_CHECK(ob.release());
+  MB_CHECK(st.finish());
   MB_CHECK(check_flags(bka));
   return bka == bkb ? MB200_OK : check_flags(bkb);
 }
