@@ -74,13 +74,6 @@ int mb200_sync(mb200_ctx* ctx);
                                         the device first (default 65536; 0 = always; INT64_MAX = never) */
 #define MB200_OPT_GROUP_PREFETCH 2   /* the partition passes of that grouping pull their next tile into L2 with
                                         cp.async.bulk.prefetch (default 0: measured neutral on B200, profiles/r2_k1_bank.md) */
-#define MB200_OPT_SINGLE_KERNEL 3    /* single-sketch K1: 0 = first form (2 x 512 threads, 4096 direct-mapped slots),
-                                        1 = one 1024-thread CTA per SM with a 2-way cache of 14336 keys (default; measured
-                                        152 vs 103 G events/s on config 2); on calls of at least 2^26 events its
-                                        misses with keys in [0, 2^24) are summed per key in a 128 MiB table on the
-                                        context (one L2 reduction each) and scattered once per distinct key at the
-                                        end of the call (DESIGN.md §3 K1), 2 = the same with warp-level aggregation of
-                                        equal keys through MATCH.ANY (measured 45 G events/s: kept for the record) */
 #define MB200_OPT_MAX_FALLBACK_ROWS 4 /* RESCORED / CERTIFIED: fail with MB200_ERR_UNSUPPORTED instead of sending more
                                         than this many rows through the exact full-row path (default -1: no limit) */
 int mb200_set_option(mb200_ctx* ctx, int option, int64_t value);

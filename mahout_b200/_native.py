@@ -19,7 +19,7 @@ MEM_HOST, MEM_DEVICE = 0, 1
 DTYPE_F16, DTYPE_BF16 = 0, 1
 PRECISION_TENSOR, PRECISION_RESCORED, PRECISION_CERTIFIED = 0, 1, 2
 K_UPDATE, K_NORMALIZE, K_COSINE, K_RESCORE, K_PARSE, K_PREPARE, K_GROUP, K_ROUTE, K_RECOMMEND = 0, 1, 2, 3, 4, 5, 6, 7, 8
-OPT_GROUP_MIN_EVENTS, OPT_GROUP_PREFETCH, OPT_SINGLE_KERNEL, OPT_MAX_FALLBACK_ROWS = 1, 2, 3, 4
+OPT_GROUP_MIN_EVENTS, OPT_GROUP_PREFETCH, OPT_MAX_FALLBACK_ROWS = 1, 2, 4
 MAX_DEPTH = 32
 
 

@@ -91,7 +91,6 @@ struct mb200_ctx {
   std::pair<void*, size_t> ws_slots[WS_SLOT_COUNT] = {};
   int64_t group_min_events = 1 << 16;  // MB200_OPT_GROUP_MIN_EVENTS
   int group_prefetch = 0;              // MB200_OPT_GROUP_PREFETCH
-  int single_kernel = 1;               // MB200_OPT_SINGLE_KERNEL
   int64_t max_fallback_rows = -1;      // MB200_OPT_MAX_FALLBACK_ROWS
   // grow-only device staging of host-memory arguments, in request order within a call (ArgStage)
   std::vector<std::pair<void*, size_t>> io;

@@ -22,7 +22,6 @@ struct UpdateArgs {
   double qscale;  // 2^frac_bits
   unsigned long long* flags;
   HashFamily hf;
-  int slots_log2;  // hot-key cache (single-sketch kernel)
 };
 
 template <typename T>

@@ -257,10 +257,6 @@ int mb200_set_option(mb200_ctx* ctx, int option, int64_t value) {
       if (value < 0) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_set_option: GROUP_MIN_EVENTS must be >= 0");
       ctx->group_min_events = value;
       return MB200_OK;
-    case MB200_OPT_SINGLE_KERNEL:
-      if (value < 0 || value > 2) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_set_option: SINGLE_KERNEL must be 0, 1 or 2");
-      ctx->single_kernel = (int)value;
-      return MB200_OK;
     case MB200_OPT_MAX_FALLBACK_ROWS:
       ctx->max_fallback_rows = value;
       return MB200_OK;

@@ -122,127 +122,22 @@ __global__ void __launch_bounds__(256) k_update_bank(const UpdateArgs<T, K> p) {
 }
 
 // ------------------------------------------------------------------------------------------
-// K1 (single-sketch mode, E == 1): Zipf-skewed keys hammer a handful of counters, and L2
-// serialises same-address atomics.  Each CTA keeps a shared-memory cache keyed by the KEY
-// (one lookup covers all d rows): slot = {tag, 64-bit sum as lo/hi 32-bit words}.  The first
-// key to claim a slot owns it for the CTA's lifetime (hot keys show up first); owned keys
-// cost one LDS + one ATOMS.ADD.32 (+ a rare carry add), everything else takes the direct
-// d x RED.ADD.64 path.  At the end each slot is flushed with d global atomics.
+// K1 (single-sketch mode, E == 1): Zipf-skewed keys hammer a handful of counters, and L2 serialises same-address
+// reductions.  ONE CTA of 1024 threads per SM owns a 2-way set-associative shared-memory cache of SETS x 2 keys
+// (32-bit tags; slot = {tag, 64-bit sum as lo/hi 32-bit words}), keyed by the KEY, so one lookup covers all d rows.
+// The first key to claim a way owns it for the CTA's lifetime (hot keys show up first); owned keys cost one LDS + one
+// ATOMS.ADD.32 (+ a rare carry add).  Keys outside [0, 2^32 - 1) and keys whose set is full are misses: they take the
+// direct d x RED.ADD.64 path, or the key table on large calls (below).  At the end each slot is flushed with d global
+// reductions.
 // ------------------------------------------------------------------------------------------
-#define CACHE_KEY_XOR 0x8000000000000000ull  /* tag 0 == empty; key Long.MIN_VALUE is never cached */
-
-// returns true when the event was absorbed by the CTA's cache
-__device__ __forceinline__ bool cache_absorb(unsigned long long* tag, unsigned int* lo, int* hi, int slots_log2,
-                                             long long key, long long q) {
-  const unsigned long long t = (unsigned long long)key ^ CACHE_KEY_XOR;
-  const unsigned int slot =
-      (unsigned int)(((unsigned long long)key * 0x9E3779B97F4A7C15ull) >> (64 - slots_log2));
-  bool owned = false;
-  if (t != 0) {
-    unsigned long long cur = *reinterpret_cast<volatile unsigned long long*>(&tag[slot]);
-    if (cur == t) {
-      owned = true;
-    } else if (cur == 0) {
-      cur = atomicCAS(&tag[slot], 0ull, t);
-      owned = (cur == 0 || cur == t);
-    }
-  }
-  if (owned) {
-    const unsigned int qlo = (unsigned int)(unsigned long long)q;
-    const int qhi = (int)(q >> 32);
-    const unsigned int old = atomicAdd(&lo[slot], qlo);
-    const int h = qhi + ((unsigned int)(old + qlo) < qlo ? 1 : 0);
-    if (h != 0) atomicAdd(&hi[slot], h);
-  }
-  return owned;
-}
+static constexpr int V2_THREADS = 1024;
+static constexpr int V2_SETS = 7168;            // 2 ways each; 24 bytes per set
+static constexpr unsigned V2_EMPTY = 0xFFFFFFFFu;
 
 // Events the cache does not own are not scattered by the lane that met them -- with ~1/3 of the lanes
 // missing, every warp would run the d hashes + d REDs at 1/3 occupancy.  They are queued per warp in
 // shared memory and drained 32 at a time, every lane busy.
 static constexpr int MISS_Q = 64;  // entries per warp (a trip adds at most 32)
-
-template <typename T, bool VEC, int D, typename K = long long>
-__global__ void __launch_bounds__(512, 2) k_update_single(const UpdateArgs<T, K> p) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int S = 1 << p.slots_log2;
-  unsigned long long* tag = reinterpret_cast<unsigned long long*>(smem_raw);
-  unsigned int* lo = reinterpret_cast<unsigned int*>(tag + S);
-  int* hi = reinterpret_cast<int*>(lo + S);
-  long long* mq_key = reinterpret_cast<long long*>(hi + S) + (threadIdx.x >> 5) * (2 * MISS_Q);
-  long long* mq_val = mq_key + MISS_Q;
-  for (int s = threadIdx.x; s < S; s += blockDim.x) {
-    tag[s] = 0;
-    lo[s] = 0;
-    hi[s] = 0;
-  }
-  __syncthreads();
-
-  const int lane = threadIdx.x & 31;
-  int qn = 0;  // entries in this warp's miss queue (warp-uniform)
-  unsigned int bad = 0;
-  unsigned long long maxabs = 0;
-  const long long n4 = p.n & ~3LL;
-  const long long stride = (long long)gridDim.x * blockDim.x * 4;
-  // whole warps iterate together: the trip count is made warp-uniform
-  const long long first = ((long long)blockIdx.x * blockDim.x + (threadIdx.x & ~31)) * 4;
-  for (long long wbase = first; wbase < n4; wbase += stride) {
-    const long long base = wbase + (long long)lane * 4;
-    const bool live = base < n4;
-    Quad<T> ev;
-    if (live) load_quad<T, false, VEC, K>(p, base, ev);
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-      bool miss = false;
-      long long q = 0;
-      if (live) {
-        q = inc_to_quanta(ev.inc[j], p.qscale, bad, maxabs);
-        if (q != 0) miss = !cache_absorb(tag, lo, hi, p.slots_log2, ev.key[j], q);
-      }
-      const unsigned m = __ballot_sync(0xffffffffu, miss);
-      if (miss) {
-        const int at = qn + __popc(m & ((1u << lane) - 1u));
-        mq_key[at] = ev.key[j];
-        mq_val[at] = q;
-      }
-      qn += __popc(m);
-      __syncwarp();
-      if (qn >= 32) {
-        qn -= 32;
-        scatter_event<D>(p.counters, p.hf, mq_key[qn + lane], mq_val[qn + lane]);
-        __syncwarp();
-      }
-    }
-  }
-  if (lane < qn) scatter_event<D>(p.counters, p.hf, mq_key[lane], mq_val[lane]);
-  if (blockIdx.x == 0 && threadIdx.x < (unsigned)(p.n - n4)) {
-    long long t = n4 + threadIdx.x;
-    long long q = inc_to_quanta(p.inc[t], p.qscale, bad, maxabs);
-    if (q != 0) scatter_event<D>(p.counters, p.hf, p.key[t], q);
-  }
-  __syncthreads();
-  // flush: one key -> d global atomics
-  for (int s = threadIdx.x; s < S; s += blockDim.x) {
-    unsigned long long t = tag[s];
-    if (t == 0) continue;
-    long long sum = (long long)(((unsigned long long)(unsigned int)hi[s] << 32) | lo[s]);
-    if (sum != 0) scatter_event<D>(p.counters, p.hf, (long long)(t ^ CACHE_KEY_XOR), sum);
-  }
-  publish_flags(p.flags, bad, 0u, maxabs);
-}
-
-// ------------------------------------------------------------------------------------------
-// K1 (single-sketch mode), second form.  The first form is bound by the L2 reduction path (measured: 0.91 of the
-// RED.ADD.64 rate the chip sustains into a 32 MiB array) with 1.5 reductions per event, and three quarters of its
-// shared-memory atomic wavefronts are same-address replays of the Zipf head.  Here:
-//   * ONE CTA of 1024 threads per SM owns a 2-way set-associative cache of SETS x 2 keys (14336 slots instead of
-//     2 x 4096 direct-mapped ones, 32-bit tags): more of the head is absorbed, fewer reductions reach L2;
-//   * AGG: lanes of a warp that carry the same key are combined first (MATCH.ANY + REDUX.SUM): one shared-memory
-//     atomic -- or one queued miss -- per distinct key per warp instead of one per event.
-// ------------------------------------------------------------------------------------------
-static constexpr int V2_THREADS = 1024;
-static constexpr int V2_SETS = 7168;            // 2 ways each; 24 bytes per set
-static constexpr unsigned V2_EMPTY = 0xFFFFFFFFu;
 
 struct CacheV2 {
   uint2* tags;       // [SETS] two 32-bit tags per set
@@ -251,7 +146,7 @@ struct CacheV2 {
 };
 
 // returns true when (key, q) was added to the CTA's cache; key < 2^32 - 1
-__device__ __forceinline__ bool cache_absorb_v2(const CacheV2& c, unsigned int t, long long q) {
+__device__ __forceinline__ bool cache_add(const CacheV2& c, unsigned int t, long long q) {
   const unsigned int set = __umulhi(t * 0x9E3779B1u, (unsigned)V2_SETS);
   unsigned int* tg = reinterpret_cast<unsigned int*>(c.tags + set);
   const unsigned long long both = *reinterpret_cast<volatile unsigned long long*>(c.tags + set);
@@ -333,7 +228,7 @@ __device__ __forceinline__ void publish_count(unsigned long long* stats, int wor
 }
 
 // COUNT: keep the trace counters (MB200_TRACE only: the counting costs issue slots)
-template <typename T, bool VEC, int D, typename K, bool AGG, bool KT, bool COUNT>
+template <typename T, bool VEC, int D, typename K, bool KT, bool COUNT>
 __global__ void __launch_bounds__(V2_THREADS, 1)
     k_update_single_v2(const UpdateArgs<T, K> p, long long* __restrict__ ktab, unsigned long long* __restrict__ stats) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -371,23 +266,10 @@ __global__ void __launch_bounds__(V2_THREADS, 1)
       if (live) q = quanta_of(ev.inc[j], p.qscale, qscale_f, bad, maxabs);
       const long long key = ev.key[j];
       const bool act = live && q != 0;
-      // cacheable: the key fits the 32-bit tag; AGG also needs 32 of the increments to fit an int
-      bool elig = act && (unsigned long long)key < 0xFFFFFFFFull;
+      // cacheable: the key fits the 32-bit tag
+      const bool elig = act && (unsigned long long)key < 0xFFFFFFFFull;
       bool miss = act && !elig;
-      if (AGG) {
-        elig = elig && q > -(1 << 26) && q < (1 << 26);
-        miss = act && !elig;
-        const unsigned peers = __match_any_sync(0xffffffffu, elig ? (unsigned)key : V2_EMPTY);
-        const int qs = __reduce_add_sync(peers, elig ? (int)q : 0);
-        if (elig) {
-          if (lane == __ffs(peers) - 1) {
-            q = qs;
-            miss = qs != 0 && !cache_absorb_v2(c, (unsigned)key, qs);
-          }
-        }
-      } else if (elig) {
-        miss = !cache_absorb_v2(c, (unsigned)key, q);
-      }
+      if (elig) miss = !cache_add(c, (unsigned)key, q);
       const unsigned m = __ballot_sync(0xffffffffu, miss);
       if (miss) {
         const int at = qn + __popc(m & ((1u << lane) - 1u));
@@ -683,7 +565,6 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
   p.qscale = ldexp(1.0, bk->frac_bits);
   p.flags = bk->flags;
   p.hf = bk->hf;
-  p.slots_log2 = 12;
   const bool vec = sizeof(K) == 4 ? ((((uintptr_t)key | (uintptr_t)entity) & 15) == 0 && ((uintptr_t)inc & 3) == 0)
                                   : ((((uintptr_t)key | (uintptr_t)inc | (uintptr_t)entity) & 15) == 0);
   const bool d4 = bk->d == 4;
@@ -691,45 +572,40 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
     if (bk->E > 1 && entity && mb200_group_applicable(bk, n)) return mb200_group_update<T>(bk, entity, key, inc, n);
   }
   ProfScope prof(ctx, MB200_K_UPDATE);
-  if (bk->E == 1 && ctx->single_kernel != 0) {
-    // single-sketch mode, second form: one 1024-thread CTA per SM, 2-way cache, optional warp aggregation; the
-    // default form (1) sends the cache's misses of a large call through the key table
+  if (bk->E == 1) {
+    // single-sketch mode (the entity column, if any, is not needed): one 1024-thread CTA per SM; the cache's misses of
+    // a large call go through the key table
     const size_t smem = (size_t)V2_SETS * 24 + (size_t)(V2_THREADS / 32) * 2 * MISS_Q * sizeof(long long);
     long long want = ceil_div64(n, (int64_t)V2_THREADS * 4);
     int grid = (int)(want < (long long)ctx->num_sms ? want : (long long)ctx->num_sms);
-    const bool agg = ctx->single_kernel == 2;
-    const bool table = !agg && n >= keytab_min_events();
+    const bool table = n >= keytab_min_events();
     const bool trace = getenv("MB200_TRACE") != nullptr;
     long long* ktab = nullptr;
     StatusWords sw(ctx, KS_WORDS);
     if (table) MB_CHECK(keytab(ctx, &ktab));
     if (trace) MB_CHECK(sw.zero(WS_K1_STATS));
     unsigned long long* stats = sw.dev;
-#define LAUNCH_V2_C(VEC, D, AGG, KT, COUNT)                                                                  \
-  do {                                                                                                       \
-    MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single_v2<T, VEC, D, K, AGG, KT, COUNT>,                      \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));              \
-    k_update_single_v2<T, VEC, D, K, AGG, KT, COUNT><<<grid, V2_THREADS, smem, ctx->stream>>>(p, ktab, stats); \
+#define LAUNCH_V2_C(VEC, D, KT, COUNT)                                                                    \
+  do {                                                                                                    \
+    MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single_v2<T, VEC, D, K, KT, COUNT>,                        \
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
+    k_update_single_v2<T, VEC, D, K, KT, COUNT><<<grid, V2_THREADS, smem, ctx->stream>>>(p, ktab, stats); \
   } while (0)
-#define LAUNCH_V2(VEC, D, AGG, KT)                \
-  do {                                            \
-    if (trace) LAUNCH_V2_C(VEC, D, AGG, KT, true); \
-    else LAUNCH_V2_C(VEC, D, AGG, KT, false);      \
+#define LAUNCH_V2(VEC, D, KT)                 \
+  do {                                        \
+    if (trace) LAUNCH_V2_C(VEC, D, KT, true); \
+    else LAUNCH_V2_C(VEC, D, KT, false);      \
   } while (0)
     if (d4) {
-      if (table && vec) LAUNCH_V2(true, 4, false, true);
-      else if (table) LAUNCH_V2(false, 4, false, true);
-      else if (vec && agg) LAUNCH_V2(true, 4, true, false);
-      else if (vec) LAUNCH_V2(true, 4, false, false);
-      else if (agg) LAUNCH_V2(false, 4, true, false);
-      else LAUNCH_V2(false, 4, false, false);
+      if (table && vec) LAUNCH_V2(true, 4, true);
+      else if (table) LAUNCH_V2(false, 4, true);
+      else if (vec) LAUNCH_V2(true, 4, false);
+      else LAUNCH_V2(false, 4, false);
     } else {
-      if (table && vec) LAUNCH_V2(true, 0, false, true);
-      else if (table) LAUNCH_V2(false, 0, false, true);
-      else if (vec && agg) LAUNCH_V2(true, 0, true, false);
-      else if (vec) LAUNCH_V2(true, 0, false, false);
-      else if (agg) LAUNCH_V2(false, 0, true, false);
-      else LAUNCH_V2(false, 0, false, false);
+      if (table && vec) LAUNCH_V2(true, 0, true);
+      else if (table) LAUNCH_V2(false, 0, true);
+      else if (vec) LAUNCH_V2(true, 0, false);
+      else LAUNCH_V2(false, 0, false);
     }
 #undef LAUNCH_V2
 #undef LAUNCH_V2_C
@@ -752,23 +628,6 @@ static int launch_update(mb200_bank* bk, const K* entity, const K* key, const T*
               table ? "table" : "direct", (long long)n, h[KS_TABLE], h[KS_DIRECT], h[KS_CACHE], h[KS_FLUSHED],
               reds / (double)n);
     }
-  } else if (bk->E == 1) {
-    // single-sketch mode: the entity column (if any) is not needed
-    const int threads = 512;
-    const size_t smem = (size_t)(1 << p.slots_log2) * 16 + (size_t)(threads / 32) * 2 * MISS_Q * sizeof(long long);
-    long long want = ceil_div64(n, (int64_t)threads * 4);
-    int grid = (int)(want < (long long)ctx->num_sms * 2 ? want : (long long)ctx->num_sms * 2);
-#define LAUNCH_SINGLE(VEC, D)                                                                       \
-  do {                                                                                              \
-    MB_CUDA(ctx, cudaFuncSetAttribute(k_update_single<T, VEC, D, K>,                                \
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));     \
-    k_update_single<T, VEC, D, K><<<grid, threads, smem, ctx->stream>>>(p);                         \
-  } while (0)
-    if (vec && d4) LAUNCH_SINGLE(true, 4);
-    else if (vec) LAUNCH_SINGLE(true, 0);
-    else if (d4) LAUNCH_SINGLE(false, 4);
-    else LAUNCH_SINGLE(false, 0);
-#undef LAUNCH_SINGLE
   } else {
     const int threads = 256;
     long long want = ceil_div64(n, (int64_t)threads * 4);

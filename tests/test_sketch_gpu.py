@@ -530,13 +530,12 @@ def test_bank_dump_and_load_round_trip(mb, ctx, tmp_path):
     back.close()
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2])
-def test_single_sketch_kernel_forms_bit_exact(mb, ctx, variant):
-    """MB200_OPT_SINGLE_KERNEL: the three forms of the single-sketch K1 (direct-mapped cache; 2-way cache in one
-    1024-thread CTA; the same with warp aggregation) give the oracle's counters on a Zipf stream with keys outside
-    the 32-bit tag range, negative increments and the n % 4 tail."""
-    from mahout_b200 import _native as N
-    rng = np.random.Generator(np.random.PCG64(70 + variant))
+def test_single_sketch_update_bit_exact(mb, ctx):
+    """The single-sketch K1 (2-way shared-memory cache in one 1024-thread CTA per SM) gives the oracle's counters on
+    a Zipf stream with keys outside the 32-bit tag range, keys equal to 2^32 - 1, negative increments and the n % 4
+    tail, from host and from device memory."""
+    import torch
+    rng = np.random.Generator(np.random.PCG64(71))
     n, d, w = 400003, 4, 1 << 16
     key = np.minimum(rng.zipf(1.1, n), 10 ** 7).astype(np.int64)
     key[::50] = rng.integers(-2 ** 62, 2 ** 62, key[::50].shape[0])
@@ -545,17 +544,33 @@ def test_single_sketch_kernel_forms_bit_exact(mb, ctx, variant):
     a, b = orc.hash_params(42, d)
     want = np.zeros((1, d, w))
     orc.bank_update(want, d, w, a, b, None, key, inc)
-    ctx.set_option(N.OPT_SINGLE_KERNEL, variant)
+    for dev in (False, True):
+        bank = mb.SketchBank(1, w, d, 42, 1, ctx)
+        if dev:
+            bank.update(None, torch.from_numpy(key).cuda(), torch.from_numpy(inc).cuda())
+        else:
+            bank.update(None, key, inc)
+        bank.check()
+        assert bank.read().tobytes() == want.tobytes(), dev
+        bank.close()
+
+
+def test_set_option_rejects_unknown_options(mb):
+    """Option 3 (the removed single-sketch kernel selector) is unknown: mb200_set_option fails with
+    MB200_ERR_BAD_ARG.  Options 1 (GROUP_MIN_EVENTS), 2 (GROUP_PREFETCH) and 4 (MAX_FALLBACK_ROWS) still take
+    values."""
+    from mahout_b200 import _native as N
+    c = mb.Context(0)
     try:
-        import torch
-        for dev in (False, True):
-            bank = mb.SketchBank(1, w, d, 42, 1, ctx)
-            if dev:
-                bank.update(None, torch.from_numpy(key).cuda(), torch.from_numpy(inc).cuda())
-            else:
-                bank.update(None, key, inc)
-            bank.check()
-            assert bank.read().tobytes() == want.tobytes(), (variant, dev)
-            bank.close()
+        for val in (0, 1, 2):
+            assert N.lib().mb200_set_option(c.handle, 3, val) == N.ERR_BAD_ARG
+            assert "unknown option" in N.last_error(c.handle)
+            with pytest.raises(ValueError, match="unknown option"):
+                c.set_option(3, val)
+        c.set_option(N.OPT_GROUP_MIN_EVENTS, 0)
+        c.set_option(N.OPT_GROUP_MIN_EVENTS, 1 << 16)
+        c.set_option(N.OPT_GROUP_PREFETCH, 0)
+        c.set_option(N.OPT_MAX_FALLBACK_ROWS, 64)
+        c.set_option(N.OPT_MAX_FALLBACK_ROWS, -1)
     finally:
-        ctx.set_option(N.OPT_SINGLE_KERNEL, 1)
+        c.close()

@@ -16,20 +16,17 @@ what = sys.argv[1] if len(sys.argv) > 1 else "all"
 ctx = mb.Context(0)
 rng = np.random.Generator(np.random.PCG64(1))
 
-# ---- K1 single sketch: all three forms
+# ---- K1 single sketch
 n, d, w = 30011, 4, 4096
 key = np.minimum(rng.zipf(1.1, n), 10 ** 6).astype(np.int64)
 inc = (rng.integers(1, 11, n) * 0.5).astype(np.float32)
 a, b = orc.hash_params(42, d)
 want = np.zeros((1, d, w))
 orc.bank_update(want, d, w, a, b, None, key, inc)
-for form in (0, 1, 2):
-    ctx.set_option(N.OPT_SINGLE_KERNEL, form)
-    bank = mb.SketchBank(1, w, d, 42, 1, ctx)
-    bank.update(None, key, inc)
-    assert bank.read().tobytes() == want.tobytes(), form
-    bank.close()
-ctx.set_option(N.OPT_SINGLE_KERNEL, 1)
+bank = mb.SketchBank(1, w, d, 42, 1, ctx)
+bank.update(None, key, inc)
+assert bank.read().tobytes() == want.tobytes()
+bank.close()
 bank = mb.SketchBank(1, w, d, 42, 1, ctx)
 bank.update_u8(None, key.astype(np.uint32), (inc * 2).astype(np.uint8))
 assert bank.read().tobytes() == want.tobytes()
