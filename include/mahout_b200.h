@@ -326,7 +326,8 @@ int mb200_sized_recommend_last_plan(mb200_ctx* ctx, mb200_sized_recommend_plan* 
  *   (value desc, itemID asc), the first how_many kept.
  * Every array is in the memory space `mem`.  Out-of-range list entries or counts, a malformed user_ptr, pref_row
  * entries out of range or not strictly ascending within a user, and user rows out of range are found on the device
- * and fail the call with MB200_ERR_BAD_ARG. */
+ * and fail the call with MB200_ERR_BAD_ARG.  mb200_itembased_multi_recommend (below) returns the same bytes from all
+ * GPUs of an mb200_multi, each user row computed on one of them. */
 typedef struct mb200_itembased_args {
   /* the similarity matrix: row j = item j's top-k list exactly as mb200_bank_cosine_topk writes it */
   const int64_t* sim_idx;  /* [num_items][sim_ld] item rows */
@@ -669,6 +670,35 @@ int mb200_sized_multi_estimate_prefs(mb200_sized_multi* sm, const int64_t* user,
  * seconds[g] = host wall clock of GPU g's worker, wall_s = the call's wall clock.  work and seconds have
  * mb200_multi_gpus entries; any pointer may be NULL. */
 int mb200_sized_multi_last_stats(mb200_sized_multi* sm, int64_t* work, double* seconds, double* wall_s);
+
+/* ---- item-based recommendation on all GPUs of m: one replica of the lists and user vectors per GPU ------------ */
+/* mb200_itembased_multi_create copies the item top-k lists (sim_idx / sim_val [num_items][sim_ld], sim_cnt
+ * [num_items]), the user CSR (user_ptr [num_users + 1], pref_row / pref_val [nnz]) and item_ids [num_items], all HOST
+ * arrays with mb200_itembased_args' meaning, to every GPU of m once, all GPUs in parallel: num_items * (16 * sim_ld +
+ * 12) + 8 * nnz + 8 * (num_users + 1) bytes per GPU.  The replicas live until destroy.
+ * mb200_itembased_multi_recommend serves the m user rows `users` (HOST) with mb200_recommend_item_based's
+ * semantics: query position t goes to GPU t mod G, each GPU uploads only its share of the users and the allowed mask
+ * (optional HOST [ceil(num_items / 32)] words, NULL = all items), and out_item / out_value [m][how_many], out_cnt [m]
+ * (HOST) are exactly what mb200_recommend_item_based on one context returns for the same arguments -- values,
+ * itemIDs, counts and the -1 / 0 fill of unused slots, byte for byte, for any G, either accumulator path, with and
+ * without boolean_data and allowed.  Repeated calls of the same or a smaller shape allocate no device memory.
+ * NULL arrays, m < 0, how_many outside [1, 1024], max_prefs_per_user < 1 and bad shapes fail with
+ * MB200_ERR_BAD_ARG before any GPU work; an error found on a device (a user row out of range, a malformed CSR or
+ * list) fails the call with the first failing GPU's code and "GPU d: <message>" (mb200_multi_last_error).  The
+ * handle stays usable after a failed call.  One call at a time per mb200_multi: every call holds m's lock.
+ * mb200_itembased_multi_last_stats: the last call on h (create included): work[g] = users given to GPU g (every
+ * user for create), seconds[g] = host wall clock of GPU g's worker, wall_s = the call's wall clock; GPU g's plan is
+ * mb200_itembased_last_plan of mb200_multi_ctx(m, g).  Any pointer may be NULL. */
+typedef struct mb200_itembased_multi mb200_itembased_multi;
+int mb200_itembased_multi_create(mb200_multi* m, const int64_t* sim_idx, const double* sim_val, const int32_t* sim_cnt,
+                                 int64_t num_items, int32_t sim_ld, const int64_t* user_ptr, const int32_t* pref_row,
+                                 const float* pref_val, int64_t num_users, int64_t nnz, const int64_t* item_ids,
+                                 mb200_itembased_multi** out);
+int mb200_itembased_multi_recommend(mb200_itembased_multi* h, const int64_t* users, int64_t m, int32_t how_many,
+                                    int32_t max_prefs_per_user, int32_t boolean_data, const uint32_t* allowed,
+                                    int64_t* out_item, float* out_value, int32_t* out_cnt);
+int mb200_itembased_multi_last_stats(mb200_itembased_multi* h, int64_t* work, double* seconds, double* wall_s);
+int mb200_itembased_multi_destroy(mb200_itembased_multi* h);
 
 #ifdef __cplusplus
 }

@@ -235,6 +235,10 @@ _PROTOS = {
     "mb200_sized_multi_recommend": (C.c_int, [vp, vp, i64, i32, f64, vp, vp, i64, vp, i64, i32, C.c_int, vp, vp, vp]),
     "mb200_sized_multi_estimate_prefs": (C.c_int, [vp, vp, vp, i64, i32, f64, vp]),
     "mb200_sized_multi_last_stats": (C.c_int, [vp, vp, vp, C.POINTER(f64)]),
+    "mb200_itembased_multi_create": (C.c_int, [vp, vp, vp, vp, i64, i32, vp, vp, vp, i64, i64, vp, C.POINTER(vp)]),
+    "mb200_itembased_multi_recommend": (C.c_int, [vp, vp, i64, i32, i32, i32, vp, vp, vp, vp]),
+    "mb200_itembased_multi_last_stats": (C.c_int, [vp, vp, vp, C.POINTER(f64)]),
+    "mb200_itembased_multi_destroy": (C.c_int, [vp]),
     # bench / test support (mahout_b200/csrc/synth.h)
     "mb200_synth_events": (C.c_int, [vp, C.c_uint64, i64, i64, i64, vp, i64, vp, vp, vp, vp]),
     "mb200_bench_red64": (C.c_int, [vp, i64, i64, C.POINTER(f64), C.POINTER(f64)]),

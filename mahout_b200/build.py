@@ -19,7 +19,7 @@ LIB = os.path.join(HERE, "libmahout_b200.so")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 
 SOURCES = ["runtime.cu", "sketch.cu", "group.cu", "route.cu", "synth.cu", "cosine.cu", "ingest.cu", "job.cu", "recommend.cu",
-           "cmsized.cu", "sized_multi.cu"]
+           "cmsized.cu", "sized_multi.cu", "itembased_multi.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

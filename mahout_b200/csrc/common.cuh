@@ -140,6 +140,9 @@ template <typename T>
 int mb200_group_update(mb200_bank* bk, const long long* entity, const long long* key, const T* inc, int64_t n);
 extern "C" void mb200_job_release(struct mb200_cosine_job* job);  // cosine.cu (internal)
 void mb200_set_global_error(const char* msg);
+// recommend.cu: mb200_recommend_item_based, except that with data_on_device the lists, the user CSR and the itemIDs
+// are device pointers whatever args->mem says (itembased_multi.cu's replicas); the other arrays follow args->mem
+int mb200_itembased_call(mb200_ctx* ctx, const mb200_itembased_args* args, bool data_on_device);
 
 #define MB_CUDA(ctx, expr)                                                                   \
   do {                                                                                       \

@@ -977,7 +977,9 @@ int mb200_recommend_last_plan(mb200_ctx* ctx, mb200_recommend_plan* out) {
   return MB200_OK;
 }
 
-int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args) {
+}  // extern "C"
+
+int mb200_itembased_call(mb200_ctx* ctx, const mb200_itembased_args* args, bool data_on_device) {
   if (!ctx || !args) return mb200_fail(ctx, MB200_ERR_BAD_ARG, "mb200_recommend_item_based: NULL argument");
   std::lock_guard<std::mutex> g(ctx->mu);
   const mb200_itembased_args& x = *args;
@@ -1012,13 +1014,16 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
   a.max_prefs = x.max_prefs_per_user;
   a.boolean_data = x.boolean_data != 0;
   const size_t lists = (size_t)n * x.sim_ld;
-  MB_CHECK(st.in((const long long*)x.sim_idx, lists, &a.sim_idx));
-  MB_CHECK(st.in(x.sim_val, lists, &a.sim_val));
-  MB_CHECK(st.in((const int*)x.sim_cnt, (size_t)n, &a.sim_cnt));
-  MB_CHECK(st.in((const long long*)x.user_ptr, (size_t)x.num_users + 1, &a.user_ptr));
-  MB_CHECK(st.in((const int*)x.pref_row, (size_t)x.nnz, &a.pref_row));
-  MB_CHECK(st.in(x.pref_val, (size_t)x.nnz, &a.pref_val));
-  MB_CHECK(st.in((const long long*)x.item_ids, (size_t)n, &a.item_ids));
+  // the lists, the user CSR and the itemIDs: staged with the rest, or already on the device
+  ArgStage data(ctx, data_on_device ? MB200_MEM_DEVICE : x.mem);
+  ArgStage& dst = data_on_device ? data : st;
+  MB_CHECK(dst.in((const long long*)x.sim_idx, lists, &a.sim_idx));
+  MB_CHECK(dst.in(x.sim_val, lists, &a.sim_val));
+  MB_CHECK(dst.in((const int*)x.sim_cnt, (size_t)n, &a.sim_cnt));
+  MB_CHECK(dst.in((const long long*)x.user_ptr, (size_t)x.num_users + 1, &a.user_ptr));
+  MB_CHECK(dst.in((const int*)x.pref_row, (size_t)x.nnz, &a.pref_row));
+  MB_CHECK(dst.in(x.pref_val, (size_t)x.nnz, &a.pref_val));
+  MB_CHECK(dst.in((const long long*)x.item_ids, (size_t)n, &a.item_ids));
   MB_CHECK(st.in((const unsigned*)x.allowed, x.allowed ? (size_t)words : 0, &a.allowed));
   MB_CHECK(st.in((const long long*)x.users, (size_t)x.m, &a.users));
   MB_CHECK(st.out((long long*)x.out_item, (size_t)x.m * x.how_many, &a.out_item));
@@ -1120,6 +1125,12 @@ int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args)
                       "nnz %lld, sim_ld %d)",
                       h[IP_BAD], (long long)x.num_users, (long long)n, (long long)x.nnz, x.sim_ld);
   return MB200_OK;
+}
+
+extern "C" {
+
+int mb200_recommend_item_based(mb200_ctx* ctx, const mb200_itembased_args* args) {
+  return mb200_itembased_call(ctx, args, false);
 }
 
 int mb200_itembased_last_plan(mb200_ctx* ctx, mb200_itembased_plan* out) {

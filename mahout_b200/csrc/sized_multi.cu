@@ -15,11 +15,9 @@
 // row computed on its own.  The workers share nothing, so there are no barriers: every worker runs its part to the
 // end (or to its first failure) and the call joins them.  Host-side argument errors fail with MB200_ERR_BAD_ARG
 // before any GPU work; a GPU's failure fails the call with the first failing GPU's code and "GPU d: <message>".
-#include <stdarg.h>
 #include <string.h>
 
 #include <algorithm>
-#include <thread>
 
 #include "multi.cuh"
 
@@ -27,100 +25,13 @@ struct mb200_sized_multi {
   mb200_multi* m = nullptr;
   int64_t U = 0;
   std::vector<mb200_sized_bank*> bank;  // bank[g] lives on m->ctx[g]
-  std::vector<int64_t> work;            // last call: queries (pairs for estimates, users for create) per GPU
-  std::vector<double> seconds;          // last call: host wall clock of each GPU's worker
-  double wall_s = 0;
+  MultiStats st;                        // last call: queries (pairs for estimates, users for create) per GPU
 };
 
 namespace {
 
 constexpr int NB_MAX_N = 1024;   // mb200_sized_neighborhood's n
 constexpr int REC_MAX_HOW = 1024;  // mb200_sized_recommend's how_many
-
-// one GPU's part of a call: the first failure, and the device buffers it allocated
-struct Part {
-  mb200_ctx* ctx = nullptr;
-  int rc = MB200_OK;
-  std::string msg;
-  std::vector<void*> dev;
-
-  bool ok() const { return rc == MB200_OK; }
-  void take(int code) {  // a single-context call's status
-    if (code != MB200_OK && ok()) {
-      rc = code;
-      msg = mb200_last_error(ctx);
-    }
-  }
-  void cuda(cudaError_t e, const char* what) {
-    if (e != cudaSuccess && ok()) {
-      rc = e == cudaErrorMemoryAllocation ? MB200_ERR_OOM : MB200_ERR_CUDA;
-      msg = std::string(what) + " failed: " + cudaGetErrorString(e);
-    }
-  }
-  template <typename T>
-  T* alloc(size_t n) {
-    void* p = nullptr;
-    if (!ok()) return nullptr;
-    cuda(cudaMalloc(&p, (n ? n : 1) * sizeof(T)), "cudaMalloc");
-    if (!ok()) return nullptr;
-    dev.push_back(p);
-    return (T*)p;
-  }
-  template <typename T>
-  T* upload(const T* h, size_t n) {
-    T* d = alloc<T>(n);
-    if (ok() && n) cuda(cudaMemcpyAsync(d, h, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream), "cudaMemcpyAsync H2D");
-    return d;
-  }
-  template <typename T>
-  void download(std::vector<T>& h, const T* d, size_t n) {
-    h.resize(n);
-    if (ok() && n) cuda(cudaMemcpyAsync(h.data(), d, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream), "cudaMemcpyAsync D2H");
-  }
-  void finish() {
-    if (ok()) cuda(cudaStreamSynchronize(ctx->stream), "cudaStreamSynchronize");
-  }
-  void release() {
-    for (void* p : dev) cudaFree(p);
-    dev.clear();
-  }
-};
-
-// the positions t = l * G + g of [0, q) that go to GPU g
-inline int64_t share(int64_t q, int g, int G) { return q > g ? (q - g + G - 1) / G : 0; }
-
-// runs fn(g, part) on one worker thread per GPU (GPU 0 on the caller's), records the per-GPU and wall times, and
-// returns the first failing GPU's status
-template <typename F>
-int run_parts(mb200_sized_multi* sm, F&& fn) {
-  mb200_multi* m = sm->m;
-  const int G = m->n;
-  std::vector<Part> parts(G);
-  sm->work.assign(G, 0);
-  sm->seconds.assign(G, 0.0);
-  int caller_device = 0;
-  cudaGetDevice(&caller_device);
-  const double t0 = multi_now_s();
-  auto one = [&](int g) {
-    const double s = multi_now_s();
-    Part& p = parts[g];
-    p.ctx = m->ctx[g];
-    p.cuda(cudaSetDevice(p.ctx->device), "cudaSetDevice");
-    if (p.ok()) fn(g, p);
-    if (!p.ok()) cudaStreamSynchronize(p.ctx->stream);  // nothing may still use the buffers freed below
-    p.release();
-    sm->seconds[g] = multi_now_s() - s;
-  };
-  std::vector<std::thread> th;
-  for (int g = 1; g < G; g++) th.emplace_back(one, g);
-  one(0);
-  for (auto& t : th) t.join();
-  sm->wall_s = multi_now_s() - t0;
-  cudaSetDevice(caller_device);  // GPU 0's worker ran on the caller's thread
-  for (int g = 0; g < G; g++)
-    if (!parts[g].ok()) return multi_fail(m, parts[g].rc, "GPU " + std::to_string(m->devices[g]) + ": " + parts[g].msg);
-  return MB200_OK;
-}
 
 // GPU g's share of the query rows, its neighbourhood lists on the device ([mine][n], as mb200_sized_neighborhood
 // returns them)
@@ -143,22 +54,6 @@ Lists device_lists(Part& p, mb200_sized_bank* bank, const std::vector<int64_t>& 
   return L;
 }
 
-std::vector<int64_t> gather(const int64_t* v, int64_t q, int g, int G) {
-  std::vector<int64_t> out((size_t)share(q, g, G));
-  for (size_t l = 0; l < out.size(); l++) out[l] = v[(int64_t)l * G + g];
-  return out;
-}
-
-int bad_arg(mb200_multi* m, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
-int bad_arg(mb200_multi* m, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  return multi_fail(m, MB200_ERR_BAD_ARG, buf);
-}
-
 }  // namespace
 
 extern "C" {
@@ -168,16 +63,16 @@ int mb200_sized_multi_create(mb200_multi* m, int64_t users, const int32_t* width
                              const int64_t* item, const float* pref, mb200_sized_multi** out) {
   if (!m) return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_sized_multi_create: handle is NULL");
   std::lock_guard<std::mutex> lock(m->mu);
-  if (!out) return bad_arg(m, "mb200_sized_multi_create: out is NULL");
+  if (!out) return multi_bad_arg(m, "mb200_sized_multi_create: out is NULL");
   *out = nullptr;
   if (users < 0 || !a || !b || !user_ptr || (users > 0 && (!width || !depth)))
-    return bad_arg(m, "mb200_sized_multi_create: bad shape (users=%lld) or NULL array argument", (long long)users);
+    return multi_bad_arg(m, "mb200_sized_multi_create: bad shape (users=%lld) or NULL array argument", (long long)users);
   mb200_sized_multi* sm = new mb200_sized_multi();
   sm->m = m;
   sm->U = users;
   sm->bank.assign(m->n, nullptr);
-  const int rc = run_parts(sm, [&](int g, Part& p) {
-    sm->work[g] = users;
+  const int rc = run_parts(sm->m, sm->st, [&](int g, Part& p) {
+    sm->st.work[g] = users;
     p.take(mb200_sized_bank_create(p.ctx, users, width, depth, a, b, frac_bits, user_ptr, item, pref, MB200_MEM_HOST,
                                    &sm->bank[g]));
   });
@@ -206,16 +101,16 @@ int mb200_sized_multi_neighborhood(mb200_sized_multi* sm, const int64_t* query_r
   mb200_multi* m = sm->m;
   std::lock_guard<std::mutex> lock(m->mu);
   if (n < 1 || n > NB_MAX_N)
-    return bad_arg(m, "mb200_sized_multi_neighborhood: n must be in [1, %d] (got %d)", NB_MAX_N, n);
+    return multi_bad_arg(m, "mb200_sized_multi_neighborhood: n must be in [1, %d] (got %d)", NB_MAX_N, n);
   if (q < 0 || min_similarity != min_similarity)
-    return bad_arg(m, "mb200_sized_multi_neighborhood: bad shape (q=%lld) or NaN min_similarity", (long long)q);
+    return multi_bad_arg(m, "mb200_sized_multi_neighborhood: bad shape (q=%lld) or NaN min_similarity", (long long)q);
   if (q > 0 && (!query_rows || !out_idx || !out_sim || !out_cnt))
-    return bad_arg(m, "mb200_sized_multi_neighborhood: NULL array argument");
+    return multi_bad_arg(m, "mb200_sized_multi_neighborhood: NULL array argument");
   const int G = m->n;
-  return run_parts(sm, [&](int g, Part& p) {
-    const std::vector<int64_t> rows = gather(query_rows, q, g, G);
+  return run_parts(sm->m, sm->st, [&](int g, Part& p) {
+    const std::vector<int64_t> rows = multi_gather(query_rows, q, g, G);
     const int64_t mine = (int64_t)rows.size();
-    sm->work[g] = mine;
+    sm->st.work[g] = mine;
     if (!mine) return;
     Lists L = device_lists(p, sm->bank[g], rows, n, min_similarity);
     std::vector<int64_t> hi;
@@ -242,27 +137,27 @@ int mb200_sized_multi_recommend(mb200_sized_multi* sm, const int64_t* users, int
   if (!sm) return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_sized_multi_recommend: handle is NULL");
   mb200_multi* m = sm->m;
   std::lock_guard<std::mutex> lock(m->mu);
-  if (n < 1 || n > NB_MAX_N) return bad_arg(m, "mb200_sized_multi_recommend: n must be in [1, %d] (got %d)", NB_MAX_N, n);
+  if (n < 1 || n > NB_MAX_N) return multi_bad_arg(m, "mb200_sized_multi_recommend: n must be in [1, %d] (got %d)", NB_MAX_N, n);
   if (how_many < 1 || how_many > REC_MAX_HOW)
-    return bad_arg(m, "mb200_sized_multi_recommend: how_many must be in [1, %d] (got %d)", REC_MAX_HOW, how_many);
+    return multi_bad_arg(m, "mb200_sized_multi_recommend: how_many must be in [1, %d] (got %d)", REC_MAX_HOW, how_many);
   if (m_users < 0 || nnz < 0 || num_items < 0 || num_items >= (1LL << 31) || min_similarity != min_similarity)
-    return bad_arg(m, "mb200_sized_multi_recommend: bad shape (m=%lld nnz=%lld num_items=%lld) or NaN min_similarity",
+    return multi_bad_arg(m, "mb200_sized_multi_recommend: bad shape (m=%lld nnz=%lld num_items=%lld) or NaN min_similarity",
                    (long long)m_users, (long long)nnz, (long long)num_items);
   if (m_users > 0 && (!users || !item_ptr || (nnz > 0 && !item_col) || (num_items > 0 && !item_ids) || !out_item ||
                       !out_value || !out_cnt))
-    return bad_arg(m, "mb200_sized_multi_recommend: NULL array argument");
-  if (m_users == 0) return run_parts(sm, [](int, Part&) {});  // the stats of an empty call
+    return multi_bad_arg(m, "mb200_sized_multi_recommend: NULL array argument");
+  if (m_users == 0) return run_parts(sm->m, sm->st, [](int, Part&) {});  // the stats of an empty call
   const int64_t U = sm->U;
   // the data model is host memory: its shape is checked here, as mb200_sized_recommend checks host arguments
   if (item_ptr[0] != 0 || item_ptr[U] != nnz)
-    return bad_arg(m, "mb200_sized_multi_recommend: item_ptr[0] must be 0 and item_ptr[users] = nnz (%lld)", (long long)nnz);
+    return multi_bad_arg(m, "mb200_sized_multi_recommend: item_ptr[0] must be 0 and item_ptr[users] = nnz (%lld)", (long long)nnz);
   for (int64_t t = 1; t < num_items; t++)
-    if (item_ids[t] <= item_ids[t - 1]) return bad_arg(m, "mb200_sized_multi_recommend: item_ids must be strictly ascending");
+    if (item_ids[t] <= item_ids[t - 1]) return multi_bad_arg(m, "mb200_sized_multi_recommend: item_ids must be strictly ascending");
   const int G = m->n;
-  return run_parts(sm, [&](int g, Part& p) {
-    const std::vector<int64_t> rows = gather(users, m_users, g, G);
+  return run_parts(sm->m, sm->st, [&](int g, Part& p) {
+    const std::vector<int64_t> rows = multi_gather(users, m_users, g, G);
     const int64_t mine = (int64_t)rows.size();
-    sm->work[g] = mine;
+    sm->st.work[g] = mine;
     if (!mine) return;
     Lists L = device_lists(p, sm->bank[g], rows, n, min_similarity);
     const int64_t* d_ptr = p.upload(item_ptr, (size_t)U + 1);
@@ -297,10 +192,10 @@ int mb200_sized_multi_estimate_prefs(mb200_sized_multi* sm, const int64_t* user,
   mb200_multi* m = sm->m;
   std::lock_guard<std::mutex> lock(m->mu);
   if (n < 1 || n > NB_MAX_N)
-    return bad_arg(m, "mb200_sized_multi_estimate_prefs: n must be in [1, %d] (got %d)", NB_MAX_N, n);
+    return multi_bad_arg(m, "mb200_sized_multi_estimate_prefs: n must be in [1, %d] (got %d)", NB_MAX_N, n);
   if (q < 0 || min_similarity != min_similarity)
-    return bad_arg(m, "mb200_sized_multi_estimate_prefs: bad shape (q=%lld) or NaN min_similarity", (long long)q);
-  if (q > 0 && (!user || !item_id || !out)) return bad_arg(m, "mb200_sized_multi_estimate_prefs: NULL array argument");
+    return multi_bad_arg(m, "mb200_sized_multi_estimate_prefs: bad shape (q=%lld) or NaN min_similarity", (long long)q);
+  if (q > 0 && (!user || !item_id || !out)) return multi_bad_arg(m, "mb200_sized_multi_estimate_prefs: NULL array argument");
   const int G = m->n;
   // distinct user rows, ascending: the j-th goes to GPU j mod G as row j / G of that GPU's lists
   std::vector<int64_t> uniq(user, user + q);
@@ -312,11 +207,11 @@ int mb200_sized_multi_estimate_prefs(mb200_sized_multi* sm, const int64_t* user,
     pos[j % G].push_back(t);
     nb_row[j % G].push_back(j / G);
   }
-  return run_parts(sm, [&](int g, Part& p) {
+  return run_parts(sm->m, sm->st, [&](int g, Part& p) {
     const int64_t pairs = (int64_t)pos[g].size();
-    sm->work[g] = pairs;
+    sm->st.work[g] = pairs;
     if (!pairs) return;
-    const std::vector<int64_t> rows = gather(uniq.data(), (int64_t)uniq.size(), g, G);
+    const std::vector<int64_t> rows = multi_gather(uniq.data(), (int64_t)uniq.size(), g, G);
     Lists L = device_lists(p, sm->bank[g], rows, n, min_similarity);
     std::vector<int64_t> pu((size_t)pairs), pi((size_t)pairs);
     for (int64_t l = 0; l < pairs; l++) {
@@ -341,11 +236,7 @@ int mb200_sized_multi_estimate_prefs(mb200_sized_multi* sm, const int64_t* user,
 int mb200_sized_multi_last_stats(mb200_sized_multi* sm, int64_t* work, double* seconds, double* wall_s) {
   if (!sm) return mb200_fail(nullptr, MB200_ERR_BAD_ARG, "mb200_sized_multi_last_stats: handle is NULL");
   std::lock_guard<std::mutex> lock(sm->m->mu);
-  for (size_t g = 0; g < sm->work.size(); g++) {
-    if (work) work[g] = sm->work[g];
-    if (seconds) seconds[g] = sm->seconds[g];
-  }
-  if (wall_s) *wall_s = sm->wall_s;
+  multi_last_stats(sm->st, work, seconds, wall_s);
   return MB200_OK;
 }
 

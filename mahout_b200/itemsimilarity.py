@@ -3,7 +3,7 @@
     python -m mahout_b200.itemsimilarity --input prefs.csv --output out.tsv \
         --similarityClassname SIMILARITY_COSINE | SIMILARITY_SKETCH_COSINE --maxSimilaritiesPerItem 100 \
         [--minPrefsPerUser 1] [--booleanData true] [--threshold 0.1] \
-        [--sketchWidth 4096] [--sketchDepth 4] [--sketchSeed 42] [--precision rescored|tensor]
+        [--sketchWidth 4096] [--sketchDepth 4] [--sketchSeed 42] [--precision rescored|tensor] [--numGpus N]
 
 Same flags, input format (`userID,itemID[,pref]`, split on tab or comma) and output format
 (`itemA<TAB>itemB<TAB>similarity`, itemA < itemB, ordered by (itemA, itemB)) as the reference's
@@ -13,6 +13,8 @@ arguments or failure, like AbstractJob.  SIMILARITY_COSINE is the reference's ex
 user owns a counter column); SIMILARITY_SKETCH_COSINE the count-min sketch measure of the fork.
 `--maxPrefs` is accepted for compatibility: no down-sampling takes place (the dense tensor-core
 contraction does not need it), i.e. the job behaves like the reference with --maxPrefs >= every count.
+`--numGpus N` (0 = every visible GPU) runs the preparation on the first of N GPUs of this process and phase 1 as one
+mb200_job_item_similarity call over all N, as the native driver's flag of the same name does.
 """
 from __future__ import annotations
 
@@ -57,7 +59,33 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--similarityMatrixOutput", default=None,
                     help="also write phase 1's output: SequenceFile<IntWritable,VectorWritable> rows of the "
                          "similarity matrix (what RecommenderJob / phase 2 read)")
+    ap.add_argument("--numGpus", type=int, default=None,
+                    help="run phase 1 on N GPUs of this process (0 = every visible GPU)")
     return ap
+
+
+def open_gpus(num_gpus):
+    """(MultiGpu, the Context of its first GPU) for --numGpus N, (None, None) without the flag"""
+    if num_gpus is None:
+        return None, None
+    from .multi import MultiGpu
+    multi = MultiGpu(num_gpus)
+    return multi, multi.context(0)
+
+
+def multi_item_similarity(multi, prep, args, exact: bool):
+    """phase 1 over every GPU of `multi` from prepared prefs: the host columns go to mb200_job_item_similarity; the
+    exact measure as a depth-1 bank of one column per user (hash a = 1, b = 0), as the native driver passes it.
+    Returns numpy (idx [I, k], sim [I, k], cnt [I])."""
+    row, pref = prep.row.cpu().numpy(), prep.pref.cpu().numpy()
+    if exact:
+        key, width, depth, hp = prep.ucol.cpu().numpy(), max(prep.num_users, 1), 1, ([1], [0])
+    else:
+        key, width, depth, hp = prep.user.cpu().numpy(), args.sketchWidth, args.sketchDepth, None
+    idx, s, cnt, _ = multi.item_similarity(row, key, pref, prep.num_items, k=args.maxSimilaritiesPerItem,
+                                           threshold=args.threshold, width=width, depth=depth, seed=args.sketchSeed,
+                                           frac_bits=args.fracBits, precision=args.precision, hash_params=hp)
+    return idx, s, cnt
 
 
 class ItemSimilarityJob:
@@ -73,16 +101,20 @@ class ItemSimilarityJob:
         if args.maxSimilaritiesPerItem <= 0:
             print("maxSimilarItemsPerItem must be greater then 0!", file=sys.stderr)
             return -1
+        multi = None
         try:
+            multi, ctx = open_gpus(args.numGpus)
             # PreparePreferenceMatrixJob on the GPU: the text goes to the device once, the events stay there
-            events = ingest.Events.parse_file(args.input, boolean_data=_bool(args.booleanData))
+            events = ingest.Events.parse_file(args.input, boolean_data=_bool(args.booleanData), ctx=ctx)
             prep = events.prepare(args.minPrefsPerUser)
             events.close()
             if prep.num_items == 0:
                 idx = s = cnt = ()
                 pairs = []
             else:
-                if args.similarityClassname in EXACT_MEASURES:
+                if multi is not None:
+                    idx, s, cnt = multi_item_similarity(multi, prep, args, args.similarityClassname in EXACT_MEASURES)
+                elif args.similarityClassname in EXACT_MEASURES:
                     idx, s, cnt = sim.exact_item_similarity(
                         prep.row, prep.user, prep.pref, prep.num_items, k=args.maxSimilaritiesPerItem,
                         threshold=args.threshold, frac_bits=args.fracBits, precision=args.precision,
@@ -103,6 +135,9 @@ class ItemSimilarityJob:
         except Exception as e:   # AbstractJob: failures surface as a non-zero exit code
             print(f"itemsimilarity failed: {e}", file=sys.stderr)
             return -1
+        finally:
+            if multi is not None:
+                multi.close()
         return 0
 
 

@@ -7,6 +7,10 @@ callers that already run one rank per GPU.
 
 `sized_bank` is CosineCM with a CountMinSketchConfig on every GPU of the handle (csrc/sized_multi.cu): one
 replica of the sized bank per GPU, query users split t mod G, results bit-identical to `SizedBank`'s.
+
+`item_based` is RecommenderJob's aggregate-and-recommend phase on every GPU of the handle (csrc/itembased_multi.cu):
+one replica of the item top-k lists and the user vectors per GPU, query users split t mod G, results byte-identical
+to `itembased.recommend` on one context.
 """
 from __future__ import annotations
 
@@ -15,6 +19,7 @@ import ctypes as C
 import numpy as np
 
 from . import _native as N
+from . import sketch as sk
 from .sketch import _DTYPES, _PRECISIONS, HashFunctionBuilder, IdentityHashBuilder
 
 
@@ -95,6 +100,17 @@ class MultiGpu:
         """SizedBank's inputs (host arrays): one replica of the sized bank on every GPU of this handle"""
         return MultiSizedBank(self, width, depth, hfBuilder, user_ptr, item, pref, frac_bits)
 
+    def item_based(self, lists, uv, item_id) -> "MultiItemBased":
+        """itembased.recommend's data -- the lists (idx [I, k], sim [I, k], cnt [I]) as cosine_topk or
+        item_similarity return them, a UserVectors and item_id [I], host or device memory: one replica per GPU"""
+        return MultiItemBased(self, lists, uv, item_id)
+
+    def context(self, g: int = 0) -> sk.Context:
+        """GPU g's context as a Context that the handle owns (close() on it does not destroy it)"""
+        h = C.c_void_p()
+        self._check(N.lib().mb200_multi_ctx(self._h, int(g), C.byref(h)))
+        return _BorrowedContext(h, self.devices[g], self)
+
     def contexts(self):
         """the raw mb200_ctx handles of the GPUs, in order (launch counts, stats)"""
         out = []
@@ -103,6 +119,22 @@ class MultiGpu:
             N.lib().mb200_multi_ctx(self._h, g, C.byref(h))
             out.append(h)
         return out
+
+
+class _BorrowedContext(sk.Context):
+    """one of a MultiGpu's contexts; it lives as long as the handle, and reads as closed once the handle is"""
+
+    def __init__(self, handle, device: int, owner: MultiGpu):
+        self._handle, self.device, self.stream_ptr, self._owner = handle, int(device), None, owner
+
+    @property
+    def _h(self):
+        return self._handle if getattr(self._owner, "_h", None) is not None else None
+
+    def close(self):
+        self._handle = None
+
+    __del__ = close
 
 
 def _host(a, dtype):
@@ -205,4 +237,78 @@ class MultiSizedBank:
         secs = np.zeros(G, np.float64)
         wall = C.c_double()
         self.multi._check(N.lib().mb200_sized_multi_last_stats(self.handle, _p(work), _p(secs), C.byref(wall)))
+        return {"work": work.tolist(), "seconds": secs.tolist(), "wall_s": wall.value}
+
+
+class MultiItemBased:
+    """The item top-k lists, the user vectors and the itemIDs replicated on every GPU of a MultiGpu
+    (mb200_itembased_multi_*).  recommend splits its users between the GPUs -- query position t to GPU t mod G -- and
+    returns numpy arrays in the caller's order, byte-identical to itembased.recommend on one GPU."""
+
+    def __init__(self, multi: MultiGpu, lists, uv, item_id):
+        self.multi = multi
+        self._h = None
+        idx, sim, cnt = (_host(x, t) for x, t in zip(lists, (np.int64, np.float64, np.int32)))
+        ptr, prow, pval = _host(uv.user_ptr, np.int64), _host(uv.pref_row, np.int32), _host(uv.pref_val, np.float32)
+        ids = _host(item_id, np.int64)
+        n_items = cnt.shape[0]
+        ld = idx.size // n_items if n_items else 1
+        if idx.size != n_items * ld or sim.size != idx.size or ids.shape[0] != n_items or prow.shape != pval.shape \
+                or ptr.shape[0] < 1:
+            raise ValueError("lists must be idx / sim [I, k] and cnt [I], item_id [I]; pref_row and pref_val the same "
+                             "length")
+        self.num_items, self.num_users = n_items, ptr.shape[0] - 1
+        h = C.c_void_p()
+        multi._check(N.lib().mb200_itembased_multi_create(
+            multi._h, _p(idx), _p(sim), _p(cnt), n_items, max(ld, 1), _p(ptr), _p(prow), _p(pval), self.num_users,
+            prow.shape[0], _p(ids), C.byref(h)))
+        self._h = h
+
+    @property
+    def handle(self):
+        if self._h is None:
+            raise ValueError("item-based recommender is closed")
+        return self._h
+
+    def close(self):
+        if getattr(self, "_h", None) is not None and getattr(self.multi, "_h", None) is not None:
+            try:
+                N.lib().mb200_itembased_multi_destroy(self._h)
+            except Exception:   # interpreter shutdown
+                pass
+        self._h = None
+
+    __del__ = close
+
+    def recommend(self, users=None, how_many: int = 10, max_prefs_per_user: int = 10, boolean_data: bool = False,
+                  allowed=None):
+        """itembased.recommend for the user rows `users` (None: every user row) over all GPUs.  allowed: optional
+        bit mask over item rows (itembased.allowed_mask).  Returns numpy (items [m, how_many] int64 itemIDs, values
+        [m, how_many] float32, counts [m] int32); unused slots are -1 / 0."""
+        us = np.arange(self.num_users, dtype=np.int64) if users is None else _host(users, np.int64)
+        al = None
+        if allowed is not None:
+            al = np.ascontiguousarray(allowed.cpu().numpy() if hasattr(allowed, "cpu") else allowed).reshape(-1)
+            if al.dtype.kind not in "iu" or al.dtype.itemsize != 4:
+                raise ValueError("allowed must be 32-bit words")
+            al = al.view(np.uint32)
+            if al.shape[0] != (self.num_items + 31) // 32:
+                raise ValueError(f"allowed must hold {(self.num_items + 31) // 32} words for {self.num_items} items")
+        m, n = us.shape[0], int(how_many)
+        items = np.empty((m, max(n, 0)), np.int64)
+        vals = np.empty((m, max(n, 0)), np.float32)
+        cnt = np.empty(m, np.int32)
+        self.multi._check(N.lib().mb200_itembased_multi_recommend(
+            self.handle, _p(us), m, n, int(max_prefs_per_user), int(bool(boolean_data)),
+            _p(al) if al is not None else None, _p(items), _p(vals), _p(cnt)))
+        return items, vals, cnt
+
+    def stats(self) -> dict:
+        """the last call: {"work": users per GPU (every user for create), "seconds": each GPU's worker wall clock,
+        "wall_s": the call's wall clock}"""
+        G = self.multi.n_gpus
+        work = np.zeros(G, np.int64)
+        secs = np.zeros(G, np.float64)
+        wall = C.c_double()
+        self.multi._check(N.lib().mb200_itembased_multi_last_stats(self.handle, _p(work), _p(secs), C.byref(wall)))
         return {"work": work.tolist(), "seconds": secs.tolist(), "wall_s": wall.value}

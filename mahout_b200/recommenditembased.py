@@ -5,24 +5,32 @@ and the aggregate-and-recommend phase as native calls.
         --similarityClassname SIMILARITY_COSINE | SIMILARITY_SKETCH_COSINE [--numRecommendations 10] \
         [--maxPrefsPerUser 10] [--minPrefsPerUser 1] [--maxSimilaritiesPerItem 100] [--booleanData true] \
         [--threshold 0.1] [--usersFile ids.txt] [--itemsFile ids.txt] [--outputPathForSimilarityMatrix dir/part] \
-        [--sketchWidth 4096] [--sketchDepth 4] [--sketchSeed 42] [--precision rescored|certified|tensor]
+        [--sketchWidth 4096] [--sketchDepth 4] [--sketchSeed 42] [--precision rescored|certified|tensor] \
+        [--numGpus N]
 
 Input `userID,itemID[,pref]` (tab or comma).  Output: `userID<TAB>[itemID:value,itemID:value,...]` per user with at
 least one recommendation, users in ascending userID order, values as Float.toString writes them.  --usersFile and
 --itemsFile hold one ID per line.  --maxPrefsInItemSimilarity and --randomSeed are accepted and do nothing (no
 down-sampling takes place, as in itemsimilarity).  --filterFile, --userItemFile and --sequencefileOutput are not
 supported.  Returns 0 on success, -1 on bad arguments or failure, like AbstractJob.
+
+`--numGpus N` (0 = every visible GPU) runs the job on N GPUs of this process: the preparation on the first of them,
+the similarity phase as one mb200_job_item_similarity call over all N (as itemsimilarity --numGpus), and the
+recommend phase with the lists and user vectors replicated on every GPU and the users split between them
+(multi.MultiItemBased).  The recommend phase returns the single-GPU bytes for any N; the similarity phase does so at
+--precision rescored, so there the output file is the single-GPU job's byte for byte.
 """
 from __future__ import annotations
 
 import argparse
 import sys
+import time
 
 import numpy as np
 
 from . import itembased as ib
 from . import similarity as sim
-from .itemsimilarity import EXACT_MEASURES, MEASURES, _bool
+from .itemsimilarity import EXACT_MEASURES, MEASURES, _bool, multi_item_similarity, open_gpus
 
 UNSUPPORTED = ("filterFile", "userItemFile", "sequencefileOutput")
 
@@ -51,6 +59,8 @@ def build_parser() -> argparse.ArgumentParser:
     ap.add_argument("--sketchSeed", type=int, default=42)
     ap.add_argument("--fracBits", type=int, default=1)
     ap.add_argument("--precision", default="rescored", choices=["rescored", "certified", "tensor"])
+    ap.add_argument("--numGpus", type=int, default=None,
+                    help="run the job on N GPUs of this process (0 = every visible GPU)")
     for name in UNSUPPORTED:
         ap.add_argument(f"--{name}", default=None)
     return ap
@@ -68,6 +78,9 @@ def _read_ids(path: str) -> list[int]:
 
 
 class RecommenderJob:
+    def __init__(self):
+        self.phase_s = {}   # wall clock of the phases of the last run, each ended by a device synchronise
+
     def run(self, argv) -> int:
         try:
             args = build_parser().parse_args(argv)
@@ -88,18 +101,34 @@ class RecommenderJob:
             print("recommenditembased: --maxPrefsPerUser and --maxSimilaritiesPerItem must be positive",
                   file=sys.stderr)
             return -1
+        multi = None
+        self.phase_s = {}
         try:
             import torch
             from . import ingest
+            t0 = time.perf_counter()
+
+            def phase(name):
+                nonlocal t0
+                torch.cuda.synchronize(prep.ctx.device)
+                t = time.perf_counter()
+                self.phase_s[name] = t - t0
+                t0 = t
+
+            multi, ctx = open_gpus(args.numGpus)
             boolean = _bool(args.booleanData)
             users_wanted = _read_ids(args.usersFile) if args.usersFile else None
             items_wanted = _read_ids(args.itemsFile) if args.itemsFile else None
-            events = ingest.Events.parse_file(args.input, boolean_data=boolean)
+            events = ingest.Events.parse_file(args.input, boolean_data=boolean, ctx=ctx)
             prep = events.prepare(args.minPrefsPerUser)
             events.close()
+            phase("prepare")
             lines = []
             if prep.num_items > 0:
-                if args.similarityClassname in EXACT_MEASURES:
+                exact = args.similarityClassname in EXACT_MEASURES
+                if multi is not None:
+                    lists = multi_item_similarity(multi, prep, args, exact)
+                elif exact:
                     lists = sim.exact_item_similarity(
                         prep.row, prep.user, prep.pref, prep.num_items, k=args.maxSimilaritiesPerItem,
                         threshold=args.threshold, frac_bits=args.fracBits, precision=args.precision,
@@ -109,34 +138,48 @@ class RecommenderJob:
                         prep.row, prep.user, prep.pref, prep.num_items, k=args.maxSimilaritiesPerItem,
                         threshold=args.threshold, width=args.sketchWidth, depth=args.sketchDepth,
                         seed=args.sketchSeed, frac_bits=args.fracBits, precision=args.precision, device=True)
+                phase("similarity")
                 if args.outputPathForSimilarityMatrix:
                     from . import seqfile
                     seqfile.write_similarity_matrix(args.outputPathForSimilarityMatrix,
-                                                    *(x.cpu().numpy() for x in lists), prep.index_values)
+                                                    *(x.cpu().numpy() if hasattr(x, "cpu") else x for x in lists),
+                                                    prep.index_values)
                 uv = ib.user_vectors(prep.row, prep.user, prep.pref)
                 user_ids = uv.user_ids.cpu().numpy()
                 rows = np.arange(user_ids.shape[0], dtype=np.int64)
                 if users_wanted is not None:
                     rows = rows[np.isin(user_ids, np.asarray(users_wanted, np.int64))]
-                allowed = None
-                if items_wanted is not None:
-                    allowed = torch.from_numpy(ib.allowed_mask(prep.item_id, items_wanted).view(np.int32)).to(
-                        uv.user_ptr.device)
-                item_id = torch.from_numpy(prep.item_id).to(uv.user_ptr.device)
-                items, vals, cnt = ib.recommend(lists, uv, item_id, torch.from_numpy(rows).to(uv.user_ptr.device),
-                                                how_many=args.numRecommendations,
-                                                max_prefs_per_user=args.maxPrefsPerUser, boolean_data=boolean,
-                                                allowed=allowed, ctx=prep.ctx)
-                items, vals, cnt = (x.cpu().numpy() for x in (items, vals, cnt))
+                mask = None if items_wanted is None else ib.allowed_mask(prep.item_id, items_wanted)
+                if multi is not None:
+                    rec = multi.item_based(lists, uv, prep.item_id)
+                    phase("replicate")
+                    items, vals, cnt = rec.recommend(rows, how_many=args.numRecommendations,
+                                                     max_prefs_per_user=args.maxPrefsPerUser, boolean_data=boolean,
+                                                     allowed=mask)
+                    rec.close()
+                else:
+                    dev = uv.user_ptr.device
+                    allowed = None if mask is None else torch.from_numpy(mask.view(np.int32)).to(dev)
+                    item_id = torch.from_numpy(prep.item_id).to(dev)
+                    items, vals, cnt = ib.recommend(lists, uv, item_id, torch.from_numpy(rows).to(dev),
+                                                    how_many=args.numRecommendations,
+                                                    max_prefs_per_user=args.maxPrefsPerUser, boolean_data=boolean,
+                                                    allowed=allowed, ctx=prep.ctx)
+                    items, vals, cnt = (x.cpu().numpy() for x in (items, vals, cnt))
+                phase("recommend")
                 for t, r in enumerate(rows):
                     if cnt[t]:
                         lines.append(format_line(user_ids[r], items[t, :cnt[t]], vals[t, :cnt[t]]))
             prep.close()
             with open(args.output, "w") as out:
                 out.writelines(lines)
+            self.phase_s["write"] = time.perf_counter() - t0
         except Exception as e:   # AbstractJob: failures surface as a non-zero exit code
             print(f"recommenditembased failed: {e}", file=sys.stderr)
             return -1
+        finally:
+            if multi is not None:
+                multi.close()
         return 0
 
 
